@@ -27,6 +27,11 @@ number of points.
              whole evaluation down.
   cpu_baseline / --impl reference: the reference's own C module (oracle/_ref) driven by a Python
              restatement of models.py with a fork pool over all host cores, on a bounded sample.
+
+--dump-outputs DIR writes what the last timed step of the headline leg handed back (rank 0) as
+DIR/loglik.npy and DIR/best_rows.npy (float64, every value finite: DIR/<name>_nonfinite.npy marks
+the entries that were -inf, +inf or NaN).  The workload histogram is drawn from the CPU oracle's
+p_j, so the inputs are the same for every build and two builds compare output for output.
 """
 import argparse
 import json
@@ -45,6 +50,7 @@ K_BEST = 64
 METRIC = 'loglik_point_bin_evals_per_sec'
 UNIT = 'point*bin/s'
 POINTS_PER_RANK = {'cfg3': 1000000, 'cfg4': 100000, 'cfg5': 12500000}
+DUMP_MAX_VALUES = 4 << 20  # 32 MiB of float64: a dump stays under 64 MB on every workload
 
 
 def workload_axes(name, world):
@@ -268,8 +274,8 @@ def covest_end_to_end(cores):
 
 
 def reference_histogram(name):
-    """The workload histogram for the CPU-only reference arm: drawn from the oracle's p_j (the
-    product arm draws it from the device's, the same numbers to ~1e-15)."""
+    """The workload histogram of both arms: workload.synthetic_histogram with p_j from the CPU oracle
+    instead of the device (the same numbers to ~1e-15), so that it does not depend on the build."""
     from covest_b200 import workload
     from oracle import covest_oracle as orc
     c = workload.CONFIGS[name]
@@ -278,6 +284,26 @@ def reference_histogram(name):
     rng = np.random.default_rng(c['seed'])
     h = rng.poisson(c['kmers'] * np.maximum(p, 0.0))
     return {j: int(v) for j, v in zip(range(1, c['bins'] + 1), h)}
+
+
+def save_finite(out_dir, name, a):
+    """<name>.npy holds `a` with its non-finite entries set to 0 and <name>_nonfinite.npy (float32)
+    says which they were: 0 finite, -1 -inf, 1 +inf, 2 NaN.  A point whose likelihood is 0 (a bin
+    with counts that it gives probability 0) has log-likelihood -inf, as in the reference."""
+    kind = np.where(np.isnan(a), 2, np.where(np.isinf(a), np.sign(a), 0)).astype(np.float32)
+    np.save(os.path.join(out_dir, name + '.npy'), np.where(kind == 0, a, 0.0))
+    np.save(os.path.join(out_dir, name + '_nonfinite.npy'), kind)
+
+
+def dump_outputs(out_dir, ll, rows):
+    """The log-likelihood of every point of the slice (a fixed seeded sample of them, in index
+    order, when there are more than DUMP_MAX_VALUES) and the best rows, as .npy files."""
+    os.makedirs(out_dir, exist_ok=True)
+    ll = ll.cpu().numpy()
+    if len(ll) > DUMP_MAX_VALUES:
+        ll = ll[np.sort(np.random.default_rng(0).choice(len(ll), DUMP_MAX_VALUES, replace=False))]
+    save_finite(out_dir, 'loglik', ll)
+    save_finite(out_dir, 'best_rows', rows.cpu().numpy())
 
 
 def run_reference(args, rank, world):
@@ -409,10 +435,10 @@ def run_b200(args, rank, world, local_rank):
         barrier()
         return max_over_ranks(time.perf_counter() - t0)
 
-    def measure(name, steps, warmup, with_points):
+    def measure(name, steps, warmup, with_points, dump_dir=None):
         """One workload through every arm of the device path; returns the pieces of a JSON record."""
         cfg = workload.CONFIGS[name]
-        hist = workload.synthetic_histogram(name)
+        hist = reference_histogram(name)
         model = RepeatsModel(cfg['k'], cfg['r'], hist, 0, max_error=8)
         ctx = model.device_context
         if args.path != 'auto':
@@ -431,16 +457,18 @@ def run_b200(args, rank, world, local_rank):
         dev_ll = torch.empty(count, dtype=torch.float64, device=dev)
         dev_rows = torch.empty((K_BEST, 6), dtype=torch.float64, device=dev)
         launches = [0]
+        last_rows = [None]
 
         def step_lattice():  # the headline step: the slice as its axes, everything stays in HBM
             ctx.lattice_eval(axes, first=rank, stride=world, count=count, block=block, k_best=K_BEST,
                              out_ll=dev_ll, out_rows=dev_rows, stream=stream)
             launches[0] += ctx.last_launches() + (1 if world > 1 else 0)
-            if world > 1:
-                return parallel.merge_topk(parallel.allgather_rows(dev_rows), K_BEST)
-            return dev_rows
+            last_rows[0] = parallel.merge_topk(parallel.allgather_rows(dev_rows), K_BEST) if world > 1 else dev_rows
+            return last_rows[0]
 
         total_ms, step_ms = timed_device(step_lattice, steps, warmup)
+        if dump_dir and rank == 0:
+            dump_outputs(dump_dir, dev_ll, last_rows[0])
         n_launch = launches[0] - (launches[0] // (steps + warmup)) * warmup
         value = world * count * n_bins * steps / (total_ms * 1e-3)
         best = step_lattice().cpu().numpy()
@@ -599,7 +627,8 @@ def run_b200(args, rank, world, local_rank):
         return roof, phases
 
     with ClockSampler(local_rank) as clocks:
-        main = measure(args.workload, args.steps, args.warmup, with_points=(args.workload == 'cfg3'))
+        main = measure(args.workload, args.steps, args.warmup, with_points=(args.workload == 'cfg3'),
+                       dump_dir=args.dump_outputs)
     ctx = main['ctx']
     peak_tflops = ctx.fp64_peak(0) if rank == 0 else None
     peak_dmma = ctx.fp64_peak(1) if rank == 0 else None
@@ -760,7 +789,13 @@ def main():
                     help='add the cfg5 sub-record at any number of GPUs (12.5e6 points x 2000 bins per rank)')
     ap.add_argument('--path', default='auto', choices=['auto', 'prefix', 'gemm', 'direct'],
                     help='evaluation path of the device arm (development; auto = what a user gets)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the values and best rows of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200')
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))
