@@ -150,7 +150,9 @@ CVB_API int cvb_last_kernel_ms(cvb_ctx *ctx, double *out_ms, int *out_launches);
  * 2 = factored whenever the model supports it, 3 = factored with the GEMM, 4 = factored with the
  * prefix kernel, 5 = every point term by term in the reference's order of operations (the kernel
  * that otherwise re-evaluates only points with subnormal bin probabilities; slow, a check).  The environment variable COVEST_B200_PATH=direct|factored|gemm|prefix|auto sets
- * the initial mode.  Per-bin probabilities (cvb_probs_batch) always use the per-point kernel. */
+ * the initial mode.  The factored path holds the repeats model with max_error <= 32 only: for the
+ * basic model and for max_error > 32, modes 0 and 2-4 run the per-point kernel.  Per-bin
+ * probabilities (cvb_probs_batch) always use the per-point kernel. */
 CVB_API int cvb_set_path(cvb_ctx *ctx, int mode);
 
 /* Facts about the most recent evaluation: out[0] = path used (1 per-point, 2 factored with the
