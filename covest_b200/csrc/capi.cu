@@ -78,6 +78,8 @@ struct cvb_ctx {
     unsigned long long *d_fixed = nullptr; /* two words: marked points of the most recent evaluation, work cursor */
     unsigned int *d_marked = nullptr;      /* their indices */
     size_t cap_marked = 0;
+    /* tests (COVEST_B200_POISON): byte every call first fills the double scratch it uses with, 0 = off */
+    int poison = 0;
     std::string err;
 };
 
@@ -323,6 +325,14 @@ extern "C" int cvb_ctx_create(int model_kind, int k, int r, int max_error, int n
         if (const char *wl = getenv("COVEST_B200_PROFILE_MIB"))
             if (atoll(wl) > 0)
                 c->w_limit = (size_t)atoll(wl) * (1 << 20) / sizeof(double);
+        if (const char *po = getenv("COVEST_B200_POISON")) { /* tests: nan = bytes 0xFF, finite = 0x7F (~1.4e306) */
+            c->poison = !strcmp(po, "nan") ? 0xFF : !strcmp(po, "finite") ? 0x7F : 0;
+            if (!c->poison && *po) {
+                rc = fail(nullptr, CVB_EINVAL, "COVEST_B200_POISON must be nan or finite");
+                break;
+            }
+            c->fw.poison = c->poison;
+        }
         { /* tables of the term-by-term re-evaluation (faithful.h): by bin index j - 1 */
             const int j_all = T.max_bin > 0 ? T.max_bin : 1;
             std::vector<double> cnt(j_all, -1.0), rcp(j_all);
@@ -451,6 +461,21 @@ static int launch_loglik(cvb_ctx *ctx, const CvLattice &lat, const double *const
 static int topk_device(cvb_ctx *ctx, const CvLattice &lat, const double *d_ll, const double *d_params,
                        long long n, int K, double *out_rows, cudaStream_t s);
 
+/* COVEST_B200_POISON (tests): fill `doubles` of a scratch buffer with the context's byte pattern on the
+ * call's stream, so that a kernel reading an element it did not write sees a NaN or a huge value instead
+ * of a harmless leftover.  Only buffers of doubles: an index or a count read from poison could fault. */
+static int poison_fill(cvb_ctx *ctx, void *buf, size_t doubles, cudaStream_t s)
+{
+    if (buf && doubles)
+        CU(cudaMemsetAsync(buf, ctx->poison, doubles * sizeof(double), s), "cudaMemsetAsync(poison)");
+    return CVB_OK;
+}
+
+static size_t faith_scratch_doubles(const cvb_ctx *ctx)
+{
+    return (size_t)cv_faithful_warps(ctx->n_sm) * (size_t)ctx->faith.acc_doubles;
+}
+
 /* stream ordering between the calls of one context (see cvb_ctx::order_ev) */
 static int order_enter(cvb_ctx *ctx, cudaStream_t s)
 {
@@ -518,6 +543,14 @@ static int eval_batch(cvb_ctx *ctx, int64_t n_points, const double *params, int 
     const double *dl_all = (out_ll && l_dev) ? out_ll : ctx->d_ll;
     if (out_p && !q_dev)
         CU(grow(&ctx->d_probs, &ctx->cap_probs, (size_t)chunk * nb), "cudaMalloc(probs staging)");
+    if (ctx->poison) {
+        if (int rc = poison_fill(ctx, dl_all == ctx->d_ll ? ctx->d_ll : nullptr, (size_t)chunk, s))
+            return rc;
+        if (int rc = poison_fill(ctx, out_p && !q_dev ? ctx->d_probs : nullptr, (size_t)chunk * nb, s))
+            return rc;
+        if (int rc = poison_fill(ctx, ctx->faith.scratch, faith_scratch_doubles(ctx), s))
+            return rc;
+    }
 
     bool side_copy = false;
     for (long long off = 0; off < n_points; off += chunk) {
@@ -632,6 +665,14 @@ static int topk_device(cvb_ctx *ctx, const CvLattice &lat, const double *d_ll, c
     int rc = ensure_topk(ctx, K);
     if (rc != CVB_OK)
         return rc;
+    if (ctx->poison) { /* nothing of the call has used these buffers before the selection */
+        if ((rc = poison_fill(ctx, ctx->d_cand_ll, (size_t)ctx->topk_ctas * K, s)))
+            return rc;
+        if ((rc = poison_fill(ctx, ctx->d_sel_ll, (size_t)K, s)))
+            return rc;
+        if ((rc = poison_fill(ctx, ctx->d_rows, (size_t)K * (1 + CV_MAX_PARAMS), s)))
+            return rc;
+    }
     if (n >= CVB_TOPK_SORT_MIN && cv_topk_select_fits(n, K) && !getenv("COVEST_B200_TOPK_SORT")) {
         /* large batch, few rows wanted: radix selection (topk.cu) */
         CU(grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, cv_topk_select_bytes()), "cudaMalloc(topk scratch)");
@@ -684,6 +725,9 @@ extern "C" int cvb_topk(cvb_ctx *ctx, int64_t n_points, const double *ll, const 
     const double *dl = ll, *dp = params;
     if (n_points > 0 && !is_device_ptr(ll)) {
         CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)n_points), "cudaMalloc(loglik staging)");
+        if (ctx->poison)
+            if (int rc = poison_fill(ctx, ctx->d_ll, (size_t)n_points, s))
+                return rc;
         CU(cudaMemcpyAsync(ctx->d_ll, ll, (size_t)n_points * sizeof(double), cudaMemcpyHostToDevice, s),
            "cudaMemcpyAsync(ll)");
         dl = ctx->d_ll;
@@ -767,6 +811,12 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
     if (!dl) {
         CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)(count > 0 ? count : 1)), "cudaMalloc(loglik staging)");
         dl = ctx->d_ll;
+    }
+    if (ctx->poison) {
+        if (int rc = poison_fill(ctx, l_dev ? nullptr : ctx->d_ll, (size_t)(count > 0 ? count : 1), s))
+            return rc;
+        if (int rc = poison_fill(ctx, ctx->faith.scratch, faith_scratch_doubles(ctx), s))
+            return rc;
     }
     bool need_sync = false, side_copy = false;
     /* A long slice whose values go to host memory is evaluated in parts of whole runs (and whole

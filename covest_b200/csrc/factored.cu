@@ -2699,6 +2699,10 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
         wk.w_cap = w_need + a_need;
     }
     double *A = wk.W + w_need;
+    if (wk.poison) { /* tests: what this evaluation reads of W and the partials, it must have written first */
+        CVF_CK(cudaMemsetAsync(wk.W, wk.poison, (w_need + a_need) * sizeof(double), stream));
+        CVF_CK(cudaMemsetAsync(wk.d_scratch, wk.poison, (size_t)n_sm * 32 * 3 * CVF_PB * sizeof(double), stream));
+    }
 
     /* ---- K1, then K1b + K2 or the prefix kernel, per range ---- */
     const size_t wb = cv_warp_bytes(m.n_err);

@@ -59,6 +59,7 @@ struct CvFactorWork {
     int prefix_version = 1; /* 1: cvf_prefix_kernel (cp.async rings), 2: cvf_prefix2_kernel (bulk copies, mbarrier ring) */
     int tile_interleave = 0; /* lattice plans: tiles by descending cost over all groups (0, default) or group by group (1) */
     int analytic = 0; /* 1: the plan came from the lattice axes (no sort, no host synchronisation) */
+    int poison = 0;   /* tests (COVEST_B200_POISON): byte W and d_scratch are filled with at each evaluation, 0 = off */
     CvfLatticeCache lattice;
     double gemm_fma = 0.0; /* FMAs the tiles of K2 issue (128 rows x padded copies x padded slots) */
 };

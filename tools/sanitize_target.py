@@ -1,10 +1,14 @@
 #!/usr/bin/env python
 """Small batches through every kernel of the library, for compute-sanitizer (memcheck, racecheck,
-synccheck): the per-point kernel (basic and repeats, with per-bin probabilities), the plan kernels
-(general and from lattice axes), the profile kernel, both prefix kernels, the GEMM path, the
+synccheck, initcheck): the per-point kernel (basic and repeats, with per-bin probabilities), the plan
+kernels (general and from lattice axes), the profile kernel, both prefix kernels, the GEMM path, the
 term-by-term re-evaluation, the three top-K selections and the row merge.
 
     compute-sanitizer --tool racecheck python tools/sanitize_target.py
+    compute-sanitizer --tool initcheck python tools/sanitize_target.py
+
+(initcheck reads of device memory never written; tests/test_gpu_poison.py covers the same ground
+where the tool cannot run.)
 """
 import os
 import sys
