@@ -64,8 +64,8 @@ struct cvb_ctx {
     cudaStream_t timed_stream = nullptr;
     /* the factored path of the repeats model (factored.h) */
     CvFactorWork fw;
+    CvModelDesc fdesc;         /* desc with the row tables of the batched path (cv_build_row_tables), or desc itself */
     CvfSlots slots;            /* the row layout of the profiles (factored.h) */
-    int table_lines = 0;       /* 64-slot lines of the histogram tables */
     const double *d_log_tab = nullptr;
     int path_mode = 0;         /* 0 auto, 1 per-point kernel only, 2 factored whenever supported */
     size_t w_limit = (size_t)2 << 30; /* doubles: 16 GiB of profiles per group range */
@@ -146,6 +146,28 @@ static cudaError_t upload(cvb_ctx *ctx, const std::vector<T> &v, const T **out)
         e = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
     *out = (const T *)d;
     return e;
+}
+
+/* the tables the profile kernel reads: group records, runs, slot_mult in the order of its stores */
+static cudaError_t upload_profile_tables(cvb_ctx *ctx, const CvHostTables &T, CvTables &t)
+{
+    cudaError_t e;
+    if ((e = upload(ctx, T.grp, &t.grp)) != cudaSuccess)
+        return e;
+    std::vector<double> pr(T.slot_mult.size(), 0.0); /* per 64-slot line: pair L = slots 16 (L / 8) + L % 8 and + 8 */
+    for (size_t line = 0; line + 64 <= T.slot_mult.size(); line += 64)
+        for (int L = 0; L < 32; L++) {
+            const size_t s0 = line + 16 * (L >> 3) + (L & 7);
+            pr[line + 2 * L] = T.slot_mult[s0];
+            pr[line + 2 * L + 1] = T.slot_mult[s0 + 8];
+        }
+    if ((e = upload(ctx, pr, &t.slot_mult_pair)) != cudaSuccess)
+        return e;
+    if ((e = upload(ctx, T.run_first, &t.run_first)) != cudaSuccess)
+        return e;
+    if ((e = upload(ctx, T.run_len, &t.run_len)) != cudaSuccess)
+        return e;
+    return upload(ctx, T.blk_run_begin, &t.blk_run_begin);
 }
 
 extern "C" const char *cvb_version(void) { return "covest_b200 0.2 (sm_100a)"; }
@@ -278,34 +300,36 @@ extern "C" int cvb_ctx_create(int model_kind, int k, int r, int max_error, int n
             rc = fail(nullptr, CVB_EINVAL, "histogram too long: its group tables do not fit the shared memory of an SM");
             break;
         }
-        if ((e = upload(c, T.grp, &t.grp)) != cudaSuccess) break;
+        if ((e = upload_profile_tables(c, T, t)) != cudaSuccess) break;
         if ((e = upload(c, T.slot_mult, &t.slot_mult)) != cudaSuccess) break;
-        {
-            std::vector<double> pr(T.slot_mult.size(), 0.0); /* the order of the profile kernel's stores */
-            for (size_t line = 0; line + 64 <= T.slot_mult.size(); line += 64)
-                for (int L = 0; L < 32; L++) {
-                    const size_t s0 = line + 16 * (L >> 3) + (L & 7);
-                    pr[line + 2 * L] = T.slot_mult[s0];
-                    pr[line + 2 * L + 1] = T.slot_mult[s0 + 8];
-                }
-            if ((e = upload(c, pr, &t.slot_mult_pair)) != cudaSuccess) break;
-        }
         if ((e = upload(c, T.slot_h, &t.slot_h)) != cudaSuccess) break;
         if ((e = upload(c, T.slot_bin, &t.slot_bin)) != cudaSuccess) break;
         if ((e = upload(c, T.copy_log_h, &t.copy_log_h)) != cudaSuccess) break;
         if ((e = upload(c, T.copy_log_l, &t.copy_log_l)) != cudaSuccess) break;
-        if ((e = upload(c, T.run_first, &t.run_first)) != cudaSuccess) break;
-        if ((e = upload(c, T.run_len, &t.run_len)) != cudaSuccess) break;
-        if ((e = upload(c, T.blk_run_begin, &t.blk_run_begin)) != cudaSuccess) break;
         {
             /* rows of the profiles: the lines with counts, the others summed (COVEST_B200_ROWS=full: every line) */
             const char *rows = getenv("COVEST_B200_ROWS");
+            const bool compact = !(rows && !strcmp(rows, "full"));
+            /* without a tail the batched path evaluates the lines with counts alone (cv_build_row_tables);
+             * O_thr (max_bin) and the copy logarithms stay those of the whole histogram */
+            CvHostTables RT;
+            const bool row_tables = compact && tail == 0.0 && cv_build_row_tables(T, bin_j, bin_h, RT);
+            c->fdesc = m;
+            if (row_tables) {
+                CvModelDesc &f = c->fdesc;
+                f.n_groups = RT.n_groups;
+                f.na = RT.na;
+                f.n_blocks = RT.n_blocks;
+                /* the batched path reads the slots through its row layout (CvfSlots), not these */
+                f.tab.slot_mult = f.tab.slot_h = nullptr;
+                f.tab.slot_bin = nullptr;
+                if ((e = upload_profile_tables(c, RT, f.tab)) != cudaSuccess) break;
+            }
+            const CvHostTables &FT = row_tables ? RT : T;
             std::vector<int> line_map;
             std::vector<double2> mh;
             std::vector<double> row_h;
-            cvf_build_slots(T.slot_mult, T.slot_h, !(rows && !strcmp(rows, "full")), line_map, mh, row_h,
-                            &c->slots.sum_line);
-            c->table_lines = (int)line_map.size();
+            cvf_build_slots(FT.slot_mult, FT.slot_h, compact, row_tables, line_map, mh, row_h, &c->slots.sum_line);
             c->slots.nsteps = (int)(row_h.size() / 64);
             if ((e = upload(c, line_map, &c->slots.line_map)) != cudaSuccess) break;
             if ((e = upload(c, mh, &c->slots.slot_mh)) != cudaSuccess) break;
@@ -431,7 +455,7 @@ static int launch_loglik(cvb_ctx *ctx, const CvLattice &lat, const double *const
     }
     if (try_factored) {
         ctx->fw.timed = ctx->timing;
-        CU(cvf_eval(ctx->desc, lat, lat_axes_host, d_params, n, clip, d_ll, ctx->slots,
+        CU(cvf_eval(ctx->fdesc, lat, lat_axes_host, d_params, n, clip, d_ll, ctx->slots,
                     ctx->d_log_tab, ctx->fw, ctx->n_sm,
                     ctx->smem_max, ctx->w_limit, forced ? 0.0 : ctx->min_group, ctx->min_run,
                     ctx->path_mode == 3 ? 1 : ctx->path_mode == 4 ? 2 : 0, s, &used),

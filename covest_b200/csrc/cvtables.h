@@ -194,6 +194,40 @@ static inline std::string cv_build_tables(int n_bins, const int *bin_j, const do
     return "";
 }
 
+/* The row tables of T: the tables of the keys of T's 64-slot lines that hold a count.  Keys without
+ * a count inside those lines stay, so that the groups start where they did.  Without a tail only
+ * these bins enter the log-likelihood (models.py:103-107), and the batched path evaluates them alone.
+ * Returns false when they would not leave out a line of T or need more than one block of groups.
+ * R's max_bin and copy_log are those of the subset: O_thr and the copy logarithms must come from T. */
+static inline bool cv_build_row_tables(const CvHostTables &T, const int *bin_j, const double *bin_h,
+                                       CvHostTables &R)
+{
+    const size_t lines = T.slot_h.size() / 64;
+    std::vector<int> sub_j;
+    std::vector<double> sub_h;
+    for (size_t l = 0; l < lines; l++) {
+        bool counts = false;
+        for (int i = 0; i < 64; i++)
+            counts = counts || T.slot_h[l * 64 + i] != 0.0;
+        for (int i = 0; i < 64 && counts; i++) {
+            const int b = T.slot_bin[l * 64 + i];
+            if (b >= 0) {
+                sub_j.push_back(bin_j[b]);
+                sub_h.push_back(bin_h[b]);
+            }
+        }
+    }
+    if (!cv_build_tables((int)sub_j.size(), sub_j.data(), sub_h.data(), R).empty())
+        return false; /* no count at all */
+    /* A subset of the keys never needs more lines (greedy groups cover a subset with no more groups).
+     * Row tables of one block only, a measured rule whose cause is not known: on one B200, cfg3
+     * (16 lines -> 4, one block) and cfg5 (32 -> 4, two blocks -> one) gain, while cfg4's row tables
+     * (80 lines -> 48, five blocks -> three, 7 runs of groups instead of 10) made the profile kernel
+     * slower, 0.54 ms instead of 0.40.  Multi-block row tables are left to a measurement that
+     * explains that. */
+    return R.n_blocks == 1 && R.slot_h.size() < T.slot_h.size();
+}
+
 static inline CvTables cv_tables_view(const CvHostTables &T)
 {
     CvTables v;

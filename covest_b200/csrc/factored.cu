@@ -443,7 +443,8 @@ __device__ __forceinline__ int cvf_find_warp(const int *__restrict__ start, int 
  * that row.  The lines of a row are those of the histogram tables that hold a bin with a count, in
  * their order, and -- when there are others -- one more line with the column sums of the others
  * (CvfSlots, factored.h): the bins without counts enter the result through the mass only, and the
- * mass is linear in the profiles.  K1 writes 512 contiguous bytes per (copy, line) with one warp-wide store; the prefix
+ * mass is linear in the profiles.  Without a tail the mass does not enter at all: the tables K1 runs
+ * on are then the row tables of the lines with counts, and the line of the sums holds zeros.  K1 writes 512 contiguous bytes per (copy, line) with one warp-wide store; the prefix
  * kernel fetches whole rows (a pass of 1024 slots = 8 KB contiguous) with bulk copies; K2 scatters
  * 16 rows x one line into its fragment order while loading. */
 #define CVF_STAGE_DOUBLES (CV_GB * CV_NA_MAX * CV_W)
@@ -455,7 +456,7 @@ __device__ __forceinline__ int cvf_find_warp(const int *__restrict__ start, int 
 template <int NA>
 __device__ __forceinline__ void cvf_store_profile(int lane, int blk, int o, int nsteps,
                                                   const double *__restrict__ slot_mult /* pairs */,
-                                                  const int *__restrict__ line_map, int sum_line,
+                                                  const int *__restrict__ line_map, int sum_line, bool sums,
                                                   double *__restrict__ Wg, double *stage, const double *acc)
 {
     const int r = lane >> 2, q = lane & 3;
@@ -484,18 +485,22 @@ __device__ __forceinline__ void cvf_store_profile(int lane, int blk, int o, int 
         const int line = __ldg(line_map + blk * (2 * NA) + ns); /* the same in every lane */
         if (line >= 0) {
             *reinterpret_cast<double2 *>(row0 + line * CVF_NS) = v;
-        } else {
+        } else if (sums) {
             rest.x = cv_add(rest.x, v.x);
             rest.y = cv_add(rest.y, v.y);
         }
     }
     if (sum_line >= 0) {
         /* one sum per lane: the first half of the line; block after block adds to the lane's own
-         * double, a fixed order.  The second half stays zero (K2 reads whole lines). */
+         * double, a fixed order.  The second half stays zero (K2 reads whole lines).  Without a tail
+         * (sums = false) nothing reads the sums: the line is written as zeros. */
         double *dst = Wg + ((long long)(o - 1) * nsteps + sum_line) * CVF_NS + lane;
-        double sum = cv_add(rest.x, rest.y);
-        if (blk > 0)
-            sum = cv_add(*dst, sum);
+        double sum = 0.0;
+        if (sums) {
+            sum = cv_add(rest.x, rest.y);
+            if (blk > 0)
+                sum = cv_add(*dst, sum);
+        }
         dst[0] = sum;
         dst[32] = 0.0;
     }
@@ -510,6 +515,7 @@ __device__ __forceinline__ void cvf_profile_item(int lane, const CvModelDesc &m,
     const int sp = cvf_copy_slots(m.n_err);
     const int cpt = cvf_copies_per_tile(m.n_err);
     const int kpc = sp >> 2; /* MMA slices per copy */
+    const bool sums = m.tail != 0.0; /* the mass enters the result: the line of the sums carries it */
     for (int oa = o0; oa < o0 + CVF_KC && oa <= omax4; oa += cpt) {
         cv_w_mass(lane, m, oa, cpt * sp, sp, M);
         __syncwarp();
@@ -524,7 +530,8 @@ __device__ __forceinline__ void cvf_profile_item(int lane, const CvModelDesc &m,
                 for (int i = 0; i < 4 * NA; i++)
                     acc[i] = 0.0;
                 cv_w_fused<NA>(lane, G, cc * kpc, (cc + 1) * kpc, *M.fx, acc);
-                cvf_store_profile<NA>(lane, blk, oa + cc, nsteps, m.tab.slot_mult_pair, line_map, sum_line, Wg, stage, acc);
+                cvf_store_profile<NA>(lane, blk, oa + cc, nsteps, m.tab.slot_mult_pair, line_map, sum_line, sums, Wg, stage,
+                                      acc);
             }
             __syncwarp();
         }
@@ -1090,16 +1097,16 @@ struct CvfPrefixSmem {
      *   double tbuf[planes][warps][CVF_PE][CVF_PEW]   lane partials of the last points, per warp
      *                                           (while the schedule is built: int need[CVF_PB], the
      *                                           copies of the points by batch position)
-     * planes = 2 (sum, mass) or, with a tail, 3 (sum, mass high, mass low: compensated)
+     * planes = 1 (sum) or, with a tail, 3 (sum, mass high, mass low: compensated)
      * and in global memory, per CTA (L2-resident scratch):
-     *   double red[3][warps][CVF_PB]    per (warp, point) partial */
+     *   double red[planes][warps][CVF_PB]    per (warp, point) partial */
 };
 #define CVF_SMEM_HEAD ((sizeof(CvfPrefixSmem) + 127) & ~(size_t)127)
 
 /* nw = warps of the CTA (the kernel's NW), sl = slots per thread and pass (its SL) */
 static size_t cvf_prefix_smem_bytes(bool mass, int nw, int sl)
 {
-    const size_t planes = mass ? 3 : 2;
+    const size_t planes = mass ? 3 : 1;
     return CVF_SMEM_HEAD + (size_t)CVF_PD * sl * 32 * nw * 8 +
            planes * (size_t)nw * CVF_PE * CVF_PEW * sizeof(double);
 }
@@ -1229,8 +1236,9 @@ __device__ __forceinline__ int cvf_count_below(const int *a, int n, int x, bool 
 }
 
 /* MASS: the histogram has a tail (models.py:103-104): the mass sum_j p_j enters the result through
- * 1 - mass and is summed compensated (the reference uses fsum); without a tail it only has to
- * tell whether it is below 1 (models.py:104), a plain sum.
+ * 1 - mass and is summed compensated (the reference uses fsum).  Without a tail the tail term is
+ * tail * log(1 - mass) = +-0 whenever it is formed: the mass is not formed at all, the result is the
+ * count-weighted sum of logarithms, and the slots read are those of the lines with counts.
  * FULL: the slots are a multiple of a pass (32 NW SL), no thread ever idles in a pass.
  * ONE: the bins with counts all lie in the first of a thread's SL slots (histograms whose
  * counted bins are the first quarter of every pass): the code for the other slots' logarithms is
@@ -1255,7 +1263,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                    warp * (CVF_PE * CVF_PEW); /* plane stride TBUF_ */
     /* by batch position: copies of the point; only while the schedule is built, in the place of the transpose buffers */
     int *need_s = reinterpret_cast<int *>(cvf_smem_raw + CVF_SMEM_HEAD + RING_);
-    static_assert(2 * TBUF_ * 8 >= CVF_PB * 4, "the transpose buffers hold the cut-offs of a batch");
+    static_assert(TBUF_ * 8 >= CVF_PB * 4, "the transpose buffers hold the cut-offs of a batch");
     double *red_all = scratch + (size_t)blockIdx.x * (3 * PW_ * CVF_PB);
     double *red = red_all + warp * CVF_PB; /* plane stride PW_ * CVF_PB */
     const unsigned int ring_s = cvf_pin((unsigned int)__cvta_generic_to_shared(ring));
@@ -1462,29 +1470,27 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                     /* lane group g = lane / CVF_PE takes the columns g * CVF_PE .. + CVF_PE - 1 of row e */
                     const int e = lane & (CVF_PE - 1), c0 = (lane / CVF_PE) * CVF_PE;
                     const double *rowp = tbuf + e * CVF_PEW + c0;
-                    double acc0 = rowp[0], acc1 = rowp[TBUF_], acc2 = 0.0;
-                    if (MASS)
+                    double acc0 = rowp[0], acc1 = 0.0, acc2 = 0.0;
+                    if (MASS) {
+                        acc1 = rowp[TBUF_];
                         acc2 = rowp[2 * TBUF_];
+                    }
 #pragma unroll
                     for (int c = 1; c < CVF_PE; c++) {
                         acc0 = cv_add(acc0, rowp[c]);
                         if (MASS) { /* high parts exactly (two-sum), low parts plainly */
                             cvf_two_sum_acc(acc1, acc2, rowp[TBUF_ + c]);
                             acc2 = cv_add(acc2, rowp[2 * TBUF_ + c]);
-                        } else {
-                            acc1 = cv_add(acc1, rowp[TBUF_ + c]);
                         }
                     }
 #pragma unroll
                     for (int d = CVF_PE; d <= 16; d <<= 1) {
                         acc0 = cv_add(acc0, __shfl_xor_sync(CV_FULL_MASK, acc0, d));
-                        const double oh = __shfl_xor_sync(CV_FULL_MASK, acc1, d);
                         if (MASS) {
+                            const double oh = __shfl_xor_sync(CV_FULL_MASK, acc1, d);
                             const double ol = __shfl_xor_sync(CV_FULL_MASK, acc2, d);
                             cvf_two_sum_acc(acc1, acc2, oh);
                             acc2 = cv_add(acc2, ol);
-                        } else {
-                            acc1 = cv_add(acc1, oh);
                         }
                     }
                     const int pt = __shfl_sync(CV_FULL_MASK, mypt, e);
@@ -1492,9 +1498,10 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                         double *r0 = red + pt, *r1 = r0 + PW_ * CVF_PB, *r2 = r1 + PW_ * CVF_PB;
                         if (first_pass) {
                             *r0 = acc0;
-                            *r1 = acc1;
-                            if (MASS)
+                            if (MASS) {
+                                *r1 = acc1;
                                 *r2 = acc2;
+                            }
                         } else {
                             *r0 = cv_add(*r0, acc0);
                             if (MASS) {
@@ -1502,8 +1509,6 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                                 cvf_two_sum_acc(h, l, acc1);
                                 *r1 = h;
                                 *r2 = cv_add(l, acc2);
-                            } else {
-                                *r1 = cv_add(*r1, acc1);
                             }
                         }
                     }
@@ -1594,14 +1599,11 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                         }
                         k++;
                         double ma = 0.0, mb = 0.0, mla = 0.0, mlb = 0.0; /* models.py:103: the mass */
+                        if (MASS) {
 #pragma unroll
-                        for (int i = 0; i < SL; i++) {
-                            if (MASS) {
+                            for (int i = 0; i < SL; i++) {
                                 cvf_two_sum_acc(ma, mla, pa[i]);
                                 cvf_two_sum_acc(mb, mlb, pb[i]);
-                            } else {
-                                ma = cv_add(ma, pa[i]);
-                                mb = cv_add(mb, pb[i]);
                             }
                         }
                         double sa = 0.0, sb = 0.0;
@@ -1661,10 +1663,10 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                             tb_a = tbuf_s;
                         }
                         cvf_sts64(tb_a, sa);
-                        cvf_sts64(tb_a + TBUF_ * 8, ma);
                         cvf_sts64(tb_a + CVF_PEW * 8, sb);
-                        cvf_sts64(tb_a + CVF_PEW * 8 + TBUF_ * 8, mb);
                         if (MASS) {
+                            cvf_sts64(tb_a + TBUF_ * 8, ma);
+                            cvf_sts64(tb_a + CVF_PEW * 8 + TBUF_ * 8, mb);
                             cvf_sts64(tb_a + 2 * TBUF_ * 8, mla);
                             cvf_sts64(tb_a + CVF_PEW * 8 + 2 * TBUF_ * 8, mlb);
                         }
@@ -1706,12 +1708,10 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                     need = need_next;
                     /* models.py:100-107 for the thread's slots */
                     double sum = 0.0, mh = 0.0, ml = 0.0;
+                    if (MASS) {
 #pragma unroll
-                    for (int i = 0; i < SL; i++) {
-                        if (MASS)
+                        for (int i = 0; i < SL; i++)
                             cvf_two_sum_acc(mh, ml, p[i]);
-                        else
-                            mh = cv_add(mh, p[i]);
                     }
                     if (ONE ? log_mask != 0 : log_mask == 1) { /* the usual case: the warp's first half-line holds the bins with counts */
                         double term = cv_mul(hcnt[0], cvf_safe_log<CVF_LOG_REP>(p[0], log_s)); /* utils.py:32-35 */
@@ -1729,9 +1729,10 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                             }
                     }
                     cvf_sts64(tb_a, sum);
-                    cvf_sts64(tb_a + TBUF_ * 8, mh);
-                    if (MASS)
+                    if (MASS) {
+                        cvf_sts64(tb_a + TBUF_ * 8, mh);
                         cvf_sts64(tb_a + 2 * TBUF_ * 8, ml);
+                    }
                     tb_a += CVF_PEW * 8;
                     if (lane == pending)
                         mypt = pt;
@@ -1748,18 +1749,16 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
             for (int t = tid; t < npts; t += PT_) {
                 CvPartial part;
                 part.sum = red_all[t];
-                part.mass_h = red_all[PW_ * CVF_PB + t];
+                part.mass_h = MASS ? red_all[PW_ * CVF_PB + t] : 0.0;
                 part.mass_l = MASS ? red_all[2 * PW_ * CVF_PB + t] : 0.0;
                 for (int wv = 1; wv < PW_; wv++) {
                     part.sum = cv_add(part.sum, red_all[wv * CVF_PB + t]);
                     if (MASS) {
                         cvf_two_sum_acc(part.mass_h, part.mass_l, red_all[(PW_ + wv) * CVF_PB + t]);
                         part.mass_l = cv_add(part.mass_l, red_all[(2 * PW_ + wv) * CVF_PB + t]);
-                    } else {
-                        part.mass_h = cv_add(part.mass_h, red_all[(PW_ + wv) * CVF_PB + t]);
                     }
                 }
-                out_ll[pl.idx_sorted[b0 + t]] = cv_point_finish(m, part);
+                out_ll[pl.idx_sorted[b0 + t]] = MASS ? cv_point_finish(m, part) : part.sum;
             }
             b0 += npts;
             __syncthreads();
@@ -2715,10 +2714,14 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
     const size_t k1_smem = tab + (size_t)k1_warps * wb1;
     const bool want_mass = m.tail != 0.0;
     /* warps of the prefix kernel's CTAs: one pass over the row when 768 slots or fewer do it */
-    const int kp_slots = slots_padded - (sl.sum_line >= 0 ? 32 : 0); /* the line of the sums is half a line */
+    /* The line of the sums is half a line with a tail and not read without one -- except when no line
+     * has a count: then its first half (zeros, written by K1) is read, so that every point's sum is
+     * formed by a pass (0, models.py:106) and the epilogue reads partials this launch wrote. */
+    const int kp_slots = slots_padded - (sl.sum_line >= 0 ? (want_mass || nsteps == 1 ? 32 : CVF_NS) : 0);
     /* Geometry of the prefix kernel: warps per CTA and slots per thread so that one pass covers the
      * row when 32 half-lines or fewer do it -- the fewest warps, then the fewest slots (measured on
-     * the 9 half-lines of cfg3: 3 warps x 3 slots 0.82 ms, 3 x 4 0.91 ms) */
+     * the 9 half-lines of cfg3 with a mass: 3 warps x 3 slots 0.82 ms, 3 x 4 0.91 ms; on its 8 half-lines
+     * without one: 2 x 4 0.685 ms, 3 x 3 0.745 ms) */
     const int kp_half = kp_slots / 32;
     int kp_nw = 8, kp_sl = 4;
     if (kp_half <= 24) {

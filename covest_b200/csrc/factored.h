@@ -71,9 +71,11 @@ struct CvFactorWork {
  * in the profiles: sum over such bins of p_j = sum_o b(o) * (sum over such bins of P_o[j]).  So a
  * profile row keeps the lines that hold at least one bin with a count as they are, and ONE more line
  * whose first half holds the sums of all other lines (32 partial sums per copy, one per lane of the
- * warp that stores the row; its second half is zero; every profile value is still evaluated by K1
- * and still part of the mass).  Histograms simulated or counted to a fixed max_hist
- * are mostly zero beyond a few multiples of the coverage: cfg3 keeps 4 + 1 of its 16 lines. */
+ * warp that stores the row; its second half is zero).  With a tail every profile value is evaluated
+ * by K1 and is part of the mass.  Without a tail the mass does not enter the result: K1 evaluates the
+ * row tables (cv_build_row_tables: the lines with counts only), writes the line of the sums as zeros
+ * and K2p does not read it.  Histograms simulated or counted to a fixed max_hist are mostly zero
+ * beyond a few multiples of the coverage: cfg3 keeps 4 + 1 of its 16 lines. */
 struct CvfSlots {
     int nsteps = 0;                /* lines of a row */
     int sum_line = -1;             /* the line of the sums, -1: every line has counts */
@@ -84,9 +86,11 @@ struct CvfSlots {
 };
 
 /* host: the row layout for the tables (slot_mult, slot_h), both of the same length, a multiple of
- * 64.  compact = false keeps every line (the layout before this existed; COVEST_B200_ROWS=full). */
+ * 64.  compact = false keeps every line (the layout before this existed; COVEST_B200_ROWS=full).
+ * sums = true adds the line of the sums even when every line of these tables has a count (row tables,
+ * whose histogram tables have lines without counts). */
 static inline void cvf_build_slots(const std::vector<double> &slot_mult, const std::vector<double> &slot_h,
-                                   bool compact, std::vector<int> &line_map, std::vector<double2> &mh,
+                                   bool compact, bool sums, std::vector<int> &line_map, std::vector<double2> &mh,
                                    std::vector<double> &row_h, int *sum_line)
 {
     const size_t lines = slot_h.size() / 64;
@@ -110,7 +114,7 @@ static inline void cvf_build_slots(const std::vector<double> &slot_mult, const s
         }
     }
     *sum_line = -1;
-    if ((size_t)kept < lines) {
+    if ((size_t)kept < lines || sums) {
         *sum_line = kept;
         for (int i = 0; i < 64; i++) {
             double2 v;
