@@ -70,6 +70,8 @@ def load():
     L.cvb_lattice_eval.restype = ctypes.c_int
     L.cvb_lattice_eval.argtypes = [vp, c_int32_p, c_double_p, i64, i64, i64, i64, vp, ctypes.c_int,
                                    vp, vp]
+    L.cvb_lattice_profile.restype = ctypes.c_int
+    L.cvb_lattice_profile.argtypes = [vp, c_int32_p, c_double_p, i64, i64, i64, i64, ctypes.c_uint32, vp, vp]
     L.cvb_fp64_peak.restype = ctypes.c_int
     L.cvb_fp64_peak.argtypes = [vp, ctypes.c_int, ctypes.c_int, c_double_p]
     L.cvb_set_timing.restype = ctypes.c_int
@@ -91,6 +93,6 @@ def load():
 
 
 EXPORTS = ('cvb_ctx_create', 'cvb_ctx_destroy', 'cvb_last_error', 'cvb_loglik_batch',
-           'cvb_probs_batch', 'cvb_topk', 'cvb_loglik_topk', 'cvb_lattice_eval', 'cvb_fp64_peak', 'cvb_set_timing',
+           'cvb_probs_batch', 'cvb_topk', 'cvb_loglik_topk', 'cvb_lattice_eval', 'cvb_lattice_profile', 'cvb_fp64_peak', 'cvb_set_timing',
            'cvb_last_kernel_ms', 'cvb_set_path', 'cvb_merge_rows', 'cvb_last_path_info', 'cvb_n_param', 'cvb_device_sm_count', 'cvb_version',
            'cvb_abi_version')

@@ -34,9 +34,9 @@ import numpy as np
 from scipy.optimize import minimize
 
 from . import constants, version_string
-from .data import load_histogram, parse_data, print_output, save_histogram
+from .data import interval_report, load_histogram, parse_data, print_output, save_histogram
 from . import parallel
-from .grid import initial_grid, lattice_search, optimize_grid
+from .grid import initial_grid, lattice_profile, lattice_search, optimize_grid
 from .optimizer import lockstep_minimize
 from .histogram import process_histogram
 from .models import models, select_model
@@ -280,13 +280,16 @@ class CoverageEstimator:
                 return torch.device('cuda', self.model.device_context.device)
         return None
 
-    def refine_starts(self, starts):
+    def refine_starts(self, starts, fixed=None):
         """Refine every row of `starts` (optimiser coordinates) and return the best result:
         (x, objective, success, table) with table = one row (objective, success, x...) per start.
         Start i belongs to rank i % W (parallel.split_starts); every rank refines its share -- all
         of them per launch with the lock-step optimiser, or scipy L-BFGS-B in threads -- and the
         refined optima are all-gathered, so every rank returns the same answer.  The reference's
-        counterpart is Pool.map(self._optimize, params) and the arg-min over it (covest.py:63-78)."""
+        counterpart is Pool.map(self._optimize, params) and the arg-min over it (covest.py:63-78).
+        `fixed`: a boolean mask of coordinates that keep each start's value, on top of the
+        estimator's `fix`; the lock-step optimiser then runs whatever `optimizer` says (a profile
+        likelihood holds its profiled coordinate this way)."""
         starts = np.asarray(starts, dtype=np.float64).reshape(-1, self.model.param_count)
         rank, world = parallel.world()
         mine = parallel.split_starts(starts, rank, world)
@@ -296,9 +299,11 @@ class CoverageEstimator:
         table[:, 0] = np.inf
         table[:, 1] = 0.0
         if len(mine):
-            if self.optimizer == 'lockstep':
-                fixed = [self.fix is not None and self.fix[i] is not None for i in range(n)]
-                results, launches = lockstep_minimize(self.likelihood_batch, mine, self.bounds, fixed=fixed)
+            if self.optimizer == 'lockstep' or fixed is not None:
+                held = [self.fix is not None and self.fix[i] is not None for i in range(n)]
+                if fixed is not None:
+                    held = [bool(h or f) for h, f in zip(held, fixed)]
+                results, launches = lockstep_minimize(self.likelihood_batch, mine, self.bounds, fixed=held)
             else:
                 results = self._optimize_many([list(s) for s in mine])
             for j, res in enumerate(results):
@@ -351,34 +356,7 @@ class CoverageEstimator:
             idx = np.flatnonzero(free)
             if len(idx) == 0:
                 break
-            pts = [x.copy()]
-            for i in idx:
-                for s in (1, -1):
-                    p = x.copy()
-                    p[i] += s * h[i]
-                    pts.append(p)
-            pairs = [(a, b) for ai, a in enumerate(idx) for b in idx[ai + 1:]]
-            for a, b in pairs:
-                for sa, sb in ((1, 1), (1, -1), (-1, 1), (-1, -1)):
-                    p = x.copy()
-                    p[a] += sa * h[a]
-                    p[b] += sb * h[b]
-                    pts.append(p)
-            vals = np.asarray(self.likelihood_batch(pts), dtype=np.float64)
-            fx = vals[0]
-            m = len(idx)
-            g = np.empty(m)
-            H = np.empty((m, m))
-            for t, i in enumerate(idx):
-                fp, fm = vals[1 + 2 * t], vals[2 + 2 * t]
-                g[t] = (fp - fm) / (2 * h[i])
-                H[t, t] = (fp - 2 * fx + fm) / (h[i] * h[i])
-            base = 1 + 2 * m
-            pos = {int(i): t for t, i in enumerate(idx)}
-            for q, (a, b) in enumerate(pairs):
-                fpp, fpm, fmp, fmm = vals[base + 4 * q: base + 4 * q + 4]
-                v = (fpp - fpm - fmp + fmm) / (4 * h[a] * h[b])
-                H[pos[int(a)], pos[int(b)]] = H[pos[int(b)], pos[int(a)]] = v
+            fx, g, H = self._central_differences(x, idx, h)
             if not np.all(np.isfinite(g)) or not np.all(np.isfinite(H)):
                 break
             try:
@@ -395,6 +373,269 @@ class CoverageEstimator:
                 break
         fx = float(self.likelihood_batch([x])[0])
         return x, fx
+
+    def _central_differences(self, x, idx, h):
+        """(objective, gradient, Hessian) at `x` over the coordinates `idx`, steps h[i]: the 2m^2 + 1
+        points of the central-difference stencil in one launch."""
+        pts = [x.copy()]
+        for i in idx:
+            for s in (1, -1):
+                p = x.copy()
+                p[i] += s * h[i]
+                pts.append(p)
+        pairs = [(a, b) for ai, a in enumerate(idx) for b in idx[ai + 1:]]
+        for a, b in pairs:
+            for sa, sb in ((1, 1), (1, -1), (-1, 1), (-1, -1)):
+                p = x.copy()
+                p[a] += sa * h[a]
+                p[b] += sb * h[b]
+                pts.append(p)
+        vals = np.asarray(self.likelihood_batch(pts), dtype=np.float64)
+        fx = vals[0]
+        m = len(idx)
+        g = np.empty(m)
+        H = np.empty((m, m))
+        for t, i in enumerate(idx):
+            fp, fm = vals[1 + 2 * t], vals[2 + 2 * t]
+            g[t] = (fp - fm) / (2 * h[i])
+            H[t, t] = (fp - 2 * fx + fm) / (h[i] * h[i])
+        base = 1 + 2 * m
+        pos = {int(i): t for t, i in enumerate(idx)}
+        for q, (a, b) in enumerate(pairs):
+            fpp, fpm, fmp, fmm = vals[base + 4 * q: base + 4 * q + 4]
+            v = (fpp - fpm - fmp + fmm) / (4 * h[a] * h[b])
+            H[pos[int(a)], pos[int(b)]] = H[pos[int(b)], pos[int(a)]] = v
+        return fx, g, H
+
+    # -- profile likelihoods and likelihood-ratio intervals (new) ---------------------------------
+    def _param_index(self, param):
+        return self.model.params.index(param) if isinstance(param, str) else int(param)
+
+    def _held(self):
+        n = self.model.param_count
+        return np.array([self.fix is not None and self.fix[i] is not None for i in range(n)], dtype=bool)
+
+    def _lattice_profile(self, model_axes, keep_mask):
+        """Profile rows of a lattice in model coordinates (grid.lattice_profile: on the device, sharded
+        over the ranks)."""
+        return lattice_profile(self.model, model_axes, keep_mask)
+
+    def _refine_profile(self, p, values, starts):
+        """Refine every start with coordinate p held at values[j] (and the estimator's `fix`), all
+        starts per launch: (objective, x, success) arrays."""
+        starts = np.array(starts, dtype=np.float64).reshape(len(values), self.model.param_count)
+        starts[:, p] = values
+        fixed = np.zeros(self.model.param_count, dtype=bool)
+        fixed[p] = True
+        table = self.refine_starts(starts, fixed=fixed)[3]
+        return table[:, 0].copy(), table[:, 2:].copy(), table[:, 1] > 0
+
+    def profile(self, param, values, nuisance_axes, x_hat):
+        """The profile of -loglikelihood over parameter `param` (index or name) at `values`, in
+        optimiser coordinates (error rate times err_scale, as compute_coverage_from_lattice): for
+        each value the minimum over the other free parameters.  One lattice -- the profiled axis =
+        `values`, axis j = nuisance_axes[j], or x_hat[j] where that is None; a fixed parameter takes
+        its fixed value -- whose best point per value is taken on the device (grid.lattice_profile),
+        then every finite row refined as a start with the profiled coordinate held, all starts per
+        launch (lockstep_minimize).  A refined value is never worse than its lattice row.  Returns a
+        Profile (values, fun, x, success, lattice_fun)."""
+        n = self.model.param_count
+        p = self._param_index(param)
+        values = np.asarray(values, dtype=np.float64).ravel()
+        x_hat = np.asarray(x_hat, dtype=np.float64).ravel()
+        held = self._held()
+        axes = []
+        for i in range(n):
+            if i == p:
+                axes.append(values)
+            elif held[i] or nuisance_axes[i] is None:
+                axes.append(np.array([x_hat[i]]))
+            else:
+                axes.append(np.asarray(nuisance_axes[i], dtype=np.float64).ravel())
+        model_axes = [a.copy() for a in axes]
+        for i in range(n):
+            if held[i]:
+                model_axes[i] = np.full(len(axes[i]), float(self.fix[i]))
+        model_axes[1] = model_axes[1] / self.err_scale  # as _model_rows: the lattice holds its points bit for bit
+        rows = np.asarray(self._lattice_profile(model_axes, 1 << p), dtype=np.float64)
+        self.launches += 1
+        self.evaluations += int(np.prod([len(a) for a in axes]))
+        lattice_fun = np.where(np.isnan(rows[:, 0]), np.inf, -rows[:, 0])
+        # back to optimiser coordinates: the rows hold the model-side axis values bit for bit
+        starts = np.empty((len(values), n))
+        for i in range(n):
+            for j, v in enumerate(rows[:, 1 + i]):
+                hit = np.flatnonzero(model_axes[i] == v)
+                starts[j, i] = axes[i][hit[0]] if len(hit) else v
+        starts[:, p] = values
+        fun = lattice_fun.copy()
+        x = np.full((len(values), n), np.nan)
+        success = np.zeros(len(values), dtype=bool)
+        live = np.flatnonzero(np.isfinite(lattice_fun))
+        if len(live):
+            f, xs, ok = self._refine_profile(p, values[live], starts[live])
+            better = f <= lattice_fun[live]  # the flat end game of lockstep_minimize may take a step of no gain
+            fun[live] = np.where(better, f, lattice_fun[live])
+            x[live] = np.where(better[:, None], xs, starts[live])
+            success[live] = ok
+        return Profile(values, fun, x, success, lattice_fun)
+
+    def _standard_errors(self, x, free):
+        """sqrt(diag(H^-1)) of the central-difference Hessian of the objective at x over the free
+        coordinates that are not within a stencil step of a bound (one launch, as polish); 1 % of
+        max(|x_i|, 1e-3) where that does not exist (H not positive definite, a coordinate at a bound)."""
+        lo =np.array([-np.inf if b[0] is None else b[0] for b in self.bounds], dtype=np.float64)
+        hi = np.array([np.inf if b[1] is None else b[1] for b in self.bounds], dtype=np.float64)
+        h = 1e-4 * np.maximum(np.abs(x), 1e-3)
+        se = 0.01 * np.maximum(np.abs(x), 1e-3)
+        idx = np.array([i for i in free if x[i] - h[i] >= lo[i] and x[i] + h[i] <= hi[i]], dtype=np.int64)
+        if len(idx):
+            _, _, H = self._central_differences(x.copy(), idx, h)
+            if np.all(np.isfinite(H)):
+                try:
+                    np.linalg.cholesky(H)
+                    d = np.diag(np.linalg.inv(H))
+                    ok = np.isfinite(d) & (d > 0)
+                    se[idx[ok]] = np.sqrt(d[ok])
+                except np.linalg.LinAlgError:
+                    pass
+        return se
+
+    def likelihood_intervals(self, x_hat, level=0.95, params=None):
+        """Likelihood-ratio intervals: for each free parameter (or those named in `params`) the
+        connected range around x_hat where the profile log-likelihood stays within chi2_1(level) / 2
+        of the maximum.  x_hat in optimiser coordinates (error rate times err_scale); the intervals
+        come back in model coordinates, as compute_coverage returns its estimate.
+
+          scale      standard errors from the central-difference Hessian at x_hat (_standard_errors)
+          coarse     33 profile values over x_hat +- 4 se (clipped to the bounds), nuisance axes of 12
+                     values over +- 4 se (64 for the basic model's one), one lattice each (profile);
+                     a side where the threshold is not crossed doubles its span, at most three times
+          endpoints  17 values inside each bracket of a crossing, refined from the nearer coarse
+                     optimum; the endpoint interpolates the crossing linearly there
+          flags      at_bound: a side reached a bound without crossing; open: a side crossed neither
+                     within the widest span nor at a bound (the end is the last value profiled);
+                     disjoint: a coarse profile value outside the interval is above the threshold;
+                     moved: the profile beat the log-likelihood of x_hat (x_hat is not the optimum)
+
+        Returns {name: Interval}."""
+        from scipy.stats import chi2
+        if not 0.0 < float(level) < 1.0:
+            raise ValueError('level must lie in (0, 1), not %r' % (level,))
+        n = self.model.param_count
+        x_hat = np.array([float(v) for v in x_hat], dtype=np.float64)
+        held = self._held()
+        free = [i for i in range(n) if not held[i]]
+        want = free if params is None else [self._param_index(q) for q in params]
+        for p in want:
+            if held[p]:
+                raise ValueError('%s is fixed: it has no interval' % self.model.params[p])
+        lo = np.array([-np.inf if b[0] is None else b[0] for b in self.bounds], dtype=np.float64)
+        hi = np.array([np.inf if b[1] is None else b[1] for b in self.bounds], dtype=np.float64)
+        half = float(chi2.ppf(level, 1)) / 2
+        se = self._standard_errors(x_hat, free)
+        ll_hat = -float(self.likelihood_batch([x_hat])[0])
+        out = {}
+        for p in want:
+            out[self.model.params[p]] = self._interval(p, x_hat, se, free, half, ll_hat, lo, hi, level)
+        return out
+
+    def nuisance_axes(self, p, x_hat, se, free):
+        """The lattice axes of the parameters profiled out of parameter p (profile's nuisance_axes):
+        x_hat +- 4 se over 12 values (64 for the basic model's one), clipped to the bounds."""
+        n = self.model.param_count
+        n_nuis = 64 if n == 2 else 12
+        nuisance = [None] * n
+        for j in free:
+            if j != p:
+                lo, hi = self.bounds[j]
+                lo, hi = -np.inf if lo is None else lo, np.inf if hi is None else hi
+                nuisance[j] = np.unique(np.clip(np.linspace(x_hat[j] - 4 * se[j], x_hat[j] + 4 * se[j], n_nuis),
+                                                lo, hi))
+        return nuisance
+
+    def _interval(self, p, x_hat, se, free, half, ll_hat, lo, hi, level):
+        nuisance = self.nuisance_axes(p, x_hat, se, free)
+        width = [4 * se[p], 4 * se[p]]  # below, above x_hat
+        for doubling in range(4):
+            a, b = max(x_hat[p] - width[0], lo[p]), min(x_hat[p] + width[1], hi[p])
+            values = np.unique(np.clip(np.linspace(a, b, 33), lo[p], hi[p]))
+            prof = self.profile(p, values, nuisance, x_hat)
+            pll = np.where(np.isfinite(prof.fun), -prof.fun, -np.inf)
+            top = max(ll_hat, float(np.max(pll)))
+            thr = top - half
+            c = int(np.argmin(np.abs(values - x_hat[p])))
+            if pll[c] < thr:  # x_hat itself is outside: the region around the best value
+                c = int(np.argmax(pll))
+            left, right = c, c
+            while left > 0 and pll[left - 1] >= thr:
+                left -= 1
+            while right < len(values) - 1 and pll[right + 1] >= thr:
+                right += 1
+            short = [left == 0 and values[0] > lo[p], right == len(values) - 1 and values[-1] < hi[p]]
+            if not any(short) or doubling == 3:
+                break
+            width = [w * 2 if s else w for w, s in zip(width, short)]
+        moved = bool(np.max(pll) > ll_hat + 1e-9 * max(1.0, abs(ll_hat)))
+        ends = [values[left], values[right]]
+        at_bound = [left == 0 and values[0] <= lo[p], right == len(values) - 1 and values[-1] >= hi[p]]
+        open_side = [left == 0 and not at_bound[0], right == len(values) - 1 and not at_bound[1]]
+        # endpoints: 17 values inside each bracket, warm-started from the nearer coarse optimum
+        brackets = []
+        if left > 0:
+            brackets.append((0, left, left - 1))
+        if right < len(values) - 1:
+            brackets.append((1, right, right + 1))
+        if brackets:
+            inner, starts = [], []
+            for _, i_in, i_out in brackets:
+                v = np.linspace(values[i_in], values[i_out], 19)[1:-1]
+                inner.append(v)
+                near_in = np.abs(v - values[i_in]) <= np.abs(v - values[i_out])
+                xs_in = np.where(np.isfinite(prof.x[i_in]), prof.x[i_in], x_hat)
+                xs_out = np.where(np.isfinite(prof.x[i_out]), prof.x[i_out], xs_in)
+                starts.append(np.where(near_in[:, None], xs_in[None, :], xs_out[None, :]))
+            f, _, _ = self._refine_profile(p, np.concatenate(inner), np.concatenate(starts))
+            f = np.where(np.isfinite(f), -f, -np.inf)
+            at = 0
+            for (side, i_in, i_out), v in zip(brackets, inner):
+                vs = np.concatenate(([values[i_in]], v, [values[i_out]]))
+                fs = np.concatenate(([pll[i_in]], f[at:at + len(v)], [pll[i_out]]))
+                at += len(v)
+                k = 0
+                while fs[k + 1] >= thr:  # the last value is below the threshold
+                    k += 1
+                if np.isfinite(fs[k + 1]):
+                    ends[side] = vs[k] + (thr - fs[k]) * (vs[k + 1] - vs[k]) / (fs[k + 1] - fs[k])
+                else:
+                    ends[side] = vs[k]
+        disjoint = bool(np.any(pll[:left] >= thr) or np.any(pll[right + 1:] >= thr))
+        scale = self.err_scale if p == 1 else 1.0
+        return Interval(self.model.params[p], float(ends[0]) / scale, float(ends[1]) / scale, level,
+                        {'at_bound': any(at_bound), 'open': any(open_side), 'disjoint': disjoint, 'moved': moved},
+                        thr, values / scale, pll)
+
+
+class Profile:
+    """CoverageEstimator.profile: per profiled value (optimiser coordinates) the refined objective
+    (-loglikelihood; inf where the lattice had no finite point), its point, whether the refinement
+    converged, and the objective of the lattice row it started from."""
+
+    def __init__(self, values, fun, x, success, lattice_fun):
+        self.values, self.fun, self.x, self.success, self.lattice_fun = values, fun, x, success, lattice_fun
+
+
+class Interval:
+    """A likelihood-ratio interval [lo, hi] of one parameter (model coordinates) at `level`, its flags,
+    the profile log-likelihood threshold, and the coarse profile (values, log-likelihoods) it rests on."""
+
+    def __init__(self, param, lo, hi, level, flags, threshold, values, profile):
+        self.param, self.lo, self.hi, self.level, self.flags = param, lo, hi, level, flags
+        self.threshold, self.values, self.profile = threshold, values, profile
+
+    def __repr__(self):
+        return 'Interval(%s, [%r, %r], %s)' % (self.param, self.lo, self.hi,
+                                               [k for k, v in self.flags.items() if v])
 
 
 def candidate_lattice(model, guess, bounds, shape=None):
@@ -504,11 +745,18 @@ def main(args):
             polished, _ = estimator.polish(scaled)
             res = list(polished)
             res[1] /= err_scale
+        extra = None
+        if getattr(args, 'ci', None) is not None:
+            scaled = list(res)
+            scaled[1] *= err_scale
+            with running_time('Likelihood-ratio intervals'):
+                intervals = estimator.likelihood_intervals(scaled, level=args.ci)
+            extra = interval_report(hist_orig, model, sample_factor, intervals, args.ci)
         verbose_print('Device launches: {}, evaluations: {}'.format(
             estimator.launches, estimator.evaluations))
         print_output(hist_orig, model, success, sample_factor, res, guess, orig,
                      reads_size=args.reads_size, orig_sample_factor=orig_sample_factor,
-                     starting_points=args.starting_points, use_grid_search=args.grid)
+                     starting_points=args.starting_points, use_grid_search=args.grid, extra=extra)
     if args.plot is not None:
         model.plot_probs(res, guess, orig, cumulative=args.plot, log_scale=constants.PLOT_LOG_SCALE)
 
@@ -565,11 +813,29 @@ def build_parser():
                         '(evaluated on the device, sharded over the GPUs under torchrun) instead of -sp random starts')
     p.add_argument('--seed', type=int, default=None,
                    help='Seed Python\'s random (multi-start points, histogram sampling)')
+    p.add_argument('--ci', type=float, default=None, metavar='LEVEL',
+                   help='Add likelihood-ratio intervals at LEVEL (in (0, 1), e.g. 0.95) for every free parameter '
+                        'and the genome size to the report, from profile likelihoods on the device. The intervals '
+                        'rest on the estimate: use --polish, or the flag "moved" may report an L-BFGS-B optimum '
+                        'short of the maximum')
     return p
 
 
+def check_args(parser, args):
+    """Combinations argparse cannot check on its own (parser.error exits)."""
+    if args.ci is not None:
+        if not 0.0 < args.ci < 1.0:
+            parser.error('--ci LEVEL must lie in (0, 1), not %r' % args.ci)
+        if args.load:
+            parser.error('--ci needs an estimate: it cannot be combined with --load')
+        if args.ll_only:
+            parser.error('--ci needs an estimate: it cannot be combined with --ll-only')
+
+
 def run(argv=None):
-    args = build_parser().parse_args(argv)
+    parser = build_parser()
+    args = parser.parse_args(argv)
+    check_args(parser, args)
     if args.seed is not None:
         import random
         random.seed(args.seed)

@@ -56,6 +56,11 @@ struct cvb_ctx {
     size_t cap_axes = 0;
     unsigned long long *d_counter = nullptr;
     double *d_sink = nullptr;
+    /* per-segment keys and lattice indices of cvb_lattice_profile, its rows when they go to host memory */
+    unsigned long long *d_seg_key = nullptr, *d_seg_best = nullptr;
+    size_t cap_seg_key = 0, cap_seg_best = 0;
+    double *d_seg_rows = nullptr;
+    size_t cap_seg_rows = 0;
     /* timing */
     bool timing = false;
     std::vector<cudaEvent_t> ev;
@@ -192,7 +197,8 @@ extern "C" void cvb_ctx_destroy(cvb_ctx *ctx)
         cudaFree(p);
     void *bufs[] = {ctx->d_params, ctx->d_ll,      ctx->d_probs, ctx->d_cand_ll, ctx->d_sel_ll,
                     ctx->d_rows,   ctx->d_cand_idx, ctx->d_sel_idx, ctx->d_axes,   ctx->d_counter,
-                    ctx->d_sink,   ctx->d_topk_scratch, ctx->d_marked};
+                    ctx->d_sink,   ctx->d_topk_scratch, ctx->d_marked, ctx->d_seg_key, ctx->d_seg_best,
+                    ctx->d_seg_rows};
     for (void *p : bufs)
         if (p)
             cudaFree(p);
@@ -778,18 +784,13 @@ extern "C" int cvb_topk(cvb_ctx *ctx, int64_t n_points, const double *ll, const 
 /* slices with host output from this size on are evaluated in parts (measured on cfg3, 10^6 points: two parts cost
  * 0.11 ms of a 1.7 ms call on one GPU -- shorter K1 / K2p launches leave SMs idle at their ends) */
 #define CVB_LATTICE_PART_MIN ((int64_t)1 << 22)
-extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const double *axis_values,
-                                int64_t first, int64_t stride, int64_t block, int64_t count,
-                                double *out_ll, int k_best, double *out_rows, void *stream)
+
+/* The set-up of a lattice call (cvb_lattice_eval, cvb_lattice_profile): the stream ordering of the
+ * context, the axes and the slice checked, the axes on the device, `lat` and the host axes filled in. */
+static int lattice_setup(cvb_ctx *ctx, const int32_t *axis_len, const double *axis_values, int64_t first,
+                         int64_t stride, int64_t block, int64_t count, cudaStream_t s, CvLattice &lat,
+                         const double **axes_host)
 {
-    if (!ctx)
-        return CVB_EINVAL;
-    if (!axis_len || !axis_values || first < 0 || stride < 1 || block < 1 || count < 0)
-        return fail(ctx, CVB_EINVAL, "bad lattice arguments");
-    if (k_best < 0 || (k_best > 0 && !out_rows))
-        return fail(ctx, CVB_EINVAL, "k_best > 0 needs out_rows");
-    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
-    cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
     const int np = ctx->desc.n_param;
     ctx->timed_chunks = 0;
     ctx->last_launches = 0;
@@ -811,7 +812,6 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
     CU(grow(&ctx->d_axes, &ctx->cap_axes, total_vals), "cudaMalloc(axes)");
     CU(cudaMemcpyAsync(ctx->d_axes, axis_values, total_vals * sizeof(double), cudaMemcpyHostToDevice, s),
        "cudaMemcpyAsync(axes)");
-    CvLattice lat;
     memset(&lat, 0, sizeof(lat));
     lat.enabled = 1;
     lat.n_axes = np;
@@ -824,24 +824,55 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
     lat.first = first;
     lat.stride = stride;
     lat.block = block;
-    const double *axes_host[CV_MAX_PARAMS] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    for (int a = 0; a < CV_MAX_PARAMS; a++)
+        axes_host[a] = nullptr;
     at = 0;
     for (int a = 0; a < np; a++) {
         axes_host[a] = axis_values + at;
         at += (size_t)axis_len[a];
     }
-    const bool l_dev = out_ll && is_device_ptr(out_ll);
-    double *dl = l_dev ? out_ll : nullptr;
-    if (!dl) {
+    return CVB_OK;
+}
+
+/* Where a lattice call's values go: `out_dev` (device) or else the context's staging buffer, which is
+ * grown to `count` values; under COVEST_B200_POISON the staging and the term-by-term scratch are filled. */
+static int lattice_values(cvb_ctx *ctx, double *out_dev, int64_t count, cudaStream_t s, double **dl)
+{
+    *dl = out_dev;
+    if (!*dl) {
         CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)(count > 0 ? count : 1)), "cudaMalloc(loglik staging)");
-        dl = ctx->d_ll;
+        *dl = ctx->d_ll;
     }
     if (ctx->poison) {
-        if (int rc = poison_fill(ctx, l_dev ? nullptr : ctx->d_ll, (size_t)(count > 0 ? count : 1), s))
+        if (int rc = poison_fill(ctx, out_dev ? nullptr : ctx->d_ll, (size_t)(count > 0 ? count : 1), s))
             return rc;
         if (int rc = poison_fill(ctx, ctx->faith.scratch, faith_scratch_doubles(ctx), s))
             return rc;
     }
+    return CVB_OK;
+}
+
+extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const double *axis_values,
+                                int64_t first, int64_t stride, int64_t block, int64_t count,
+                                double *out_ll, int k_best, double *out_rows, void *stream)
+{
+    if (!ctx)
+        return CVB_EINVAL;
+    if (!axis_len || !axis_values || first < 0 || stride < 1 || block < 1 || count < 0)
+        return fail(ctx, CVB_EINVAL, "bad lattice arguments");
+    if (k_best < 0 || (k_best > 0 && !out_rows))
+        return fail(ctx, CVB_EINVAL, "k_best > 0 needs out_rows");
+    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
+    cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
+    const int np = ctx->desc.n_param;
+    CvLattice lat;
+    const double *axes_host[CV_MAX_PARAMS];
+    if (int rc = lattice_setup(ctx, axis_len, axis_values, first, stride, block, count, s, lat, axes_host))
+        return rc;
+    const bool l_dev = out_ll && is_device_ptr(out_ll);
+    double *dl = nullptr;
+    if (int rc = lattice_values(ctx, l_dev ? out_ll : nullptr, count, s, &dl))
+        return rc;
     bool need_sync = false, side_copy = false;
     /* A long slice whose values go to host memory is evaluated in parts of whole runs (and whole
      * (coverage, error_rate) groups), so that the values of a part travel while the next part is
@@ -918,6 +949,63 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
     if (int rc = order_leave(ctx, s))
         return rc;
     if (need_sync)
+        CU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+    return CVB_OK;
+}
+
+extern "C" int cvb_lattice_profile(cvb_ctx *ctx, const int32_t *axis_len, const double *axis_values,
+                                   int64_t first, int64_t stride, int64_t block, int64_t count,
+                                   uint32_t keep_mask, double *out_rows, void *stream)
+{
+    if (!ctx)
+        return CVB_EINVAL;
+    if (!axis_len || !axis_values || first < 0 || stride < 1 || block < 1 || count < 0)
+        return fail(ctx, CVB_EINVAL, "bad lattice arguments");
+    if (!out_rows)
+        return fail(ctx, CVB_EINVAL, "out_rows is NULL");
+    const int np = ctx->desc.n_param;
+    if (keep_mask == 0)
+        return fail(ctx, CVB_EINVAL, "keep_mask is 0: a profile keeps at least one axis");
+    if (keep_mask >> np)
+        return fail(ctx, CVB_EINVAL, "keep_mask has a bit at or above n_param");
+    int64_t n_seg = 1; /* an empty axis is refused by lattice_setup */
+    for (int a = 0; a < np; a++)
+        if (((keep_mask >> a) & 1) && axis_len[a] > 0 && __builtin_mul_overflow(n_seg, (int64_t)axis_len[a], &n_seg))
+            return fail(ctx, CVB_EINVAL, "the number of segments (product of the kept axis lengths) overflows int64");
+    int64_t row_bytes = 0;
+    if (__builtin_mul_overflow(n_seg, (int64_t)((1 + np) * sizeof(double)), &row_bytes))
+        return fail(ctx, CVB_EINVAL, "the rows of the segments overflow an int64 byte count");
+    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
+    cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
+    CvLattice lat;
+    const double *axes_host[CV_MAX_PARAMS];
+    if (int rc = lattice_setup(ctx, axis_len, axis_values, first, stride, block, count, s, lat, axes_host))
+        return rc;
+    double *dl = nullptr;
+    if (int rc = lattice_values(ctx, nullptr, count, s, &dl))
+        return rc;
+    if (count > 0)
+        if (int rc = launch_loglik(ctx, lat, axes_host, nullptr, count, 1, dl, nullptr, s))
+            return rc;
+    CU(grow(&ctx->d_seg_key, &ctx->cap_seg_key, (size_t)n_seg), "cudaMalloc(segment keys)");
+    CU(grow(&ctx->d_seg_best, &ctx->cap_seg_best, (size_t)n_seg), "cudaMalloc(segment indices)");
+    const bool r_dev = is_device_ptr(out_rows);
+    double *dr = out_rows;
+    if (!r_dev) {
+        CU(grow(&ctx->d_seg_rows, &ctx->cap_seg_rows, (size_t)n_seg * (1 + np)), "cudaMalloc(segment rows)");
+        dr = ctx->d_seg_rows;
+        if (ctx->poison)
+            if (int rc = poison_fill(ctx, dr, (size_t)n_seg * (1 + np), s))
+                return rc;
+    }
+    CU(cv_launch_lattice_profile(lat, keep_mask, dl, count, n_seg, ctx->d_seg_key, ctx->d_seg_best, dr, ctx->n_sm, s),
+       "lattice profile launch");
+    ctx->last_launches += count > 0 ? 4 : 2;
+    if (!r_dev)
+        CU(cudaMemcpyAsync(out_rows, dr, (size_t)row_bytes, cudaMemcpyDeviceToHost, s), "cudaMemcpyAsync(rows)");
+    if (int rc = order_leave(ctx, s))
+        return rc;
+    if (!r_dev) /* one synchronisation, and only when the rows went to host memory */
         CU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
     return CVB_OK;
 }

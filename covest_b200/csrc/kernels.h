@@ -55,6 +55,16 @@ cudaError_t cv_launch_gather_rows(const CvLattice &lat, const double *params, in
                                   const double *sel_ll, const long long *sel_idx, int K,
                                   double *out_rows, cudaStream_t stream);
 
+/* Best row per segment of a lattice slice (profile.cu): `ll` (device, n values) are the values of the
+ * slice points of `lat`; the segment of a point is the mixed-radix number of the digits of the axes set
+ * in keep_mask (axis order, last kept axis fastest).  out_rows (device, n_seg x (1 + n_axes)) receives
+ * per segment (value, axis values...) of its best point: larger value first, NaN as -inf, -0 tied with
+ * +0, ties to the lower lattice index; (-inf, NaN...) for a segment without a point.  seg_key /
+ * seg_best: device scratch of n_seg words each, initialised here. */
+cudaError_t cv_launch_lattice_profile(const CvLattice &lat, unsigned int keep_mask, const double *ll, long long n,
+                                      long long n_seg, unsigned long long *seg_key, unsigned long long *seg_best,
+                                      double *out_rows, int n_sm, cudaStream_t stream);
+
 /* Register-resident FP64 micro-benchmarks for the roofline denominator (DESIGN.md section 6):
  * kind 0 = DFMA chains, kind 1 = DMMA m8n8k4 chains.  Returns flop executed. */
 cudaError_t cv_launch_peak_probe(int kind, int n_cta, int iters, double *sink, double *flop,

@@ -105,11 +105,36 @@ def replace_none(dest, src):
     return [s if d is None else d for d, s in zip(dest, src)]
 
 
+def genome_size(hist_orig, model, coverage, sample_factor):
+    """The report's genome size at `coverage` (sampled data): k-mers over the corrected coverage of the
+    un-sampled data (data.py:152-154).  Decreasing in the coverage."""
+    kmers = sum(j * h for j, h in hist_orig.items())
+    return safe_int(round(kmers / model.correct_c(coverage * sample_factor)))
+
+
+def interval_report(hist_orig, model, sample_factor, intervals, level):
+    """The report's keys of likelihood-ratio intervals (CoverageEstimator.likelihood_intervals, model
+    coordinates): ci_level, <param>_ci = [lo, hi] per parameter (coverage times sample_factor, as the
+    estimate), genome_size_ci = [gs(coverage hi), gs(coverage lo)] and ci_flags = the flags set per
+    parameter."""
+    out = {'ci_level': float(level)}
+    for name, iv in intervals.items():
+        f = sample_factor if name == 'coverage' else 1
+        out['%s_ci' % name] = [float(iv.lo * f), float(iv.hi * f)]
+    if 'coverage' in intervals:
+        c = intervals['coverage']
+        out['genome_size_ci'] = [genome_size(hist_orig, model, c.hi, sample_factor),
+                                 genome_size(hist_orig, model, c.lo, sample_factor)]
+    out['ci_flags'] = {name: sorted(k for k, v in iv.flags.items() if v) for name, iv in intervals.items()}
+    return out
+
+
 def print_output(hist_orig, model, success, sample_factor, estimated=None, guess=None, orig=None,
                  reads_size=None, silent=False, orig_sample_factor=1, starting_points=1,
-                 use_grid_search=False):
+                 use_grid_search=False, extra=None):
     """Build (and unless `silent` print) the YAML report; keys and arithmetic as data.py:106-173.
-    The up-to-three log-likelihoods it needs are evaluated in one device launch."""
+    The up-to-three log-likelihoods it needs are evaluated in one device launch.  `extra`: further
+    keys (interval_report), added last."""
     def named(names, values):
         if values is None or names is None:
             return {}
@@ -150,8 +175,7 @@ def print_output(hist_orig, model, success, sample_factor, estimated=None, guess
         out.update(named(model.params, estimated))
         out['orig_coverage'] = float(estimated[0] * orig_sample_factor * sample_factor)
         out['loglikelihood'] = ll['loglikelihood']
-        kmers = sum(j * h for j, h in hist_orig.items())
-        out['genome_size'] = safe_int(round(kmers / model.correct_c(estimated[0] * sample_factor)))
+        out['genome_size'] = genome_size(hist_orig, model, estimated[0], sample_factor)
         if reads_size is not None:
             out['genome_size_reads'] = safe_int(
                 round(reads_size / (estimated[0] * sample_factor * orig_sample_factor)))
@@ -159,6 +183,8 @@ def print_output(hist_orig, model, success, sample_factor, estimated=None, guess
         out.update(named(['provided_%s' % name for name in model.params], orig))
         if 'provided_loglikelihood' in want:
             out['provided_loglikelihood'] = ll['provided_loglikelihood']
+    if extra:
+        out.update(extra)
     if not silent:
         print(yaml.dump(out, indent=4, default_flow_style=False))
     return out

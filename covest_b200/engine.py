@@ -68,6 +68,22 @@ def _stream_ptr(stream, like=None):
     return ctypes.c_void_p(value if value else CUDA_STREAM_LEGACY)
 
 
+def profile_segments(lens, keep_mask):
+    """Number of segments of a lattice profile (cvb_lattice_profile): the product of the lengths of the
+    axes whose bit is set in keep_mask.  The mask must keep at least one axis and name no axis beyond
+    len(lens); the product must fit an int64."""
+    keep_mask = int(keep_mask)
+    if keep_mask <= 0 or keep_mask >> len(lens):
+        raise ValueError('keep_mask must be a non-empty set of the bits 0..%d, not %d' % (len(lens) - 1, keep_mask))
+    n_seg = 1
+    for a, n in enumerate(lens):
+        if keep_mask >> a & 1:
+            n_seg *= int(n)
+    if n_seg >= 1 << 63:
+        raise ValueError('a profile of %d segments: more than an int64 counts' % n_seg)
+    return n_seg
+
+
 class LikelihoodContext:
     """Device copies of one histogram and its tables (models.py:19-31, :175-183 state)."""
 
@@ -199,17 +215,7 @@ class LikelihoodContext:
         first + i*stride, i < count.  Returns (ll or None, rows or None).  `out_ll` / `out_rows`
         may be CUDA tensors: the call then only enqueues work (on `stream`, default torch's
         current stream)."""
-        if len(axes) != self.n_param:
-            raise ValueError('need %d axes' % self.n_param)
-        lens = np.ascontiguousarray([len(a) for a in axes], dtype=np.int32)
-        vals = np.ascontiguousarray(np.concatenate([np.asarray(a, dtype=np.float64).ravel() for a in axes]))
-        total = int(np.prod(lens.astype(np.int64)))
-        if count is None:
-            runs = (total + block - 1) // block
-            mine = max(0, (runs - first + stride - 1) // stride)
-            count = mine * block
-            if mine and (first + (mine - 1) * stride + 1) * block > total:
-                count -= (first + (mine - 1) * stride + 1) * block - total
+        lens, vals, count = self._lattice_slice(axes, first, stride, block, count)
         ll = out_ll
         if ll is None and want_ll:
             ll = _host_out(count)
@@ -222,6 +228,41 @@ class LikelihoodContext:
                                                int(stride), int(block), int(count), _ptr(ll), int(k_best),
                                                _ptr(rows), _stream_ptr(stream, like)), 'cvb_lattice_eval')
         return ll, rows
+
+    def _lattice_slice(self, axes, first, stride, block, count):
+        """(axis lengths, concatenated axis values, count) of a lattice call; count None = every run
+        of the slice up to the end of the lattice."""
+        if len(axes) != self.n_param:
+            raise ValueError('need %d axes' % self.n_param)
+        lens = np.ascontiguousarray([len(a) for a in axes], dtype=np.int32)
+        vals = np.ascontiguousarray(np.concatenate([np.asarray(a, dtype=np.float64).ravel() for a in axes]))
+        total = int(np.prod(lens.astype(np.int64)))
+        if count is None:
+            runs = (total + block - 1) // block
+            mine = max(0, (runs - first + stride - 1) // stride)
+            count = mine * block
+            if mine and (first + (mine - 1) * stride + 1) * block > total:
+                count -= (first + (mine - 1) * stride + 1) * block - total
+        return lens, vals, count
+
+    def lattice_profile(self, axes, keep_mask, first=0, stride=1, block=1, count=None, out_rows=None, stream=None):
+        """For every segment of the slice of lattice_eval (the points that share the values of the axes
+        whose bit is set in `keep_mask`), the (loglik, params...) row of its best point: an
+        (n_seg, 1 + n_param) array, n_seg = the product of the kept axes' lengths, segments numbered
+        with the last kept axis fastest (include/covest_b200.h, cvb_lattice_profile).  `out_rows` may
+        be a CUDA tensor: the call then only enqueues work (on `stream`, default torch's current
+        stream)."""
+        lens, vals, count = self._lattice_slice(axes, first, stride, block, count)
+        keep_mask = int(keep_mask)
+        n_seg = profile_segments(lens, keep_mask)
+        rows = out_rows
+        if rows is None:
+            rows = np.empty((n_seg, 1 + self.n_param), dtype=np.float64)
+        self._check(self._lib.cvb_lattice_profile(self._ctx, lens.ctypes.data_as(_capi.c_int32_p),
+                                                  vals.ctypes.data_as(_capi.c_double_p), int(first), int(stride),
+                                                  int(block), int(count), keep_mask, _ptr(rows),
+                                                  _stream_ptr(stream, rows)), 'cvb_lattice_profile')
+        return rows
 
     # -- measurement -----------------------------------------------------------------------
     def fp64_peak(self, kind=0, reps=5):

@@ -192,3 +192,29 @@ def lattice_search(model, axes, k_best=64):
 
     rows = parallel.sharded_best_rows(evaluate_slice, total, k_best, block=block)
     return rows.cpu().numpy() if hasattr(rows, 'cpu') else np.asarray(rows)
+
+
+def lattice_profile(model, axes, keep_mask):
+    """The profile rows of a Cartesian lattice (LikelihoodContext.lattice_profile): for every segment --
+    every combination of values of the axes whose bit is set in keep_mask, last kept axis fastest -- the
+    (loglik, params...) row of its best point.  Sharded like lattice_search: every rank profiles its
+    whole (coverage, error_rate) groups, the (n_seg, 1 + n_param) blocks are all-gathered and merged
+    segment by segment on the host (parallel.merge_segments).  With ascending axes every rank returns
+    the rows of one call over the whole lattice, whatever the number of ranks."""
+    from . import parallel
+    lens = [len(a) for a in axes]
+    total = int(np.prod(lens))
+    block = int(np.prod(lens[2:])) if len(lens) > 2 else 1
+    ctx = model.device_context
+    rank, world = parallel.world()
+    first, stride, block, count = parallel.shard_blocked(total, block, rank, world)
+    rows = ctx.lattice_profile(axes, keep_mask, first=first, stride=stride, block=block, count=count)
+    if world == 1:
+        return rows
+    device = None
+    import torch.distributed as dist
+    if dist.get_backend() == 'nccl':
+        import torch
+        device = torch.device('cuda', ctx.device)
+    gathered = parallel.allgather_rows(parallel.to_comm(rows, device)).cpu().numpy()
+    return parallel.merge_segments(gathered.reshape(world, rows.shape[0], rows.shape[1]))

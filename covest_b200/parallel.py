@@ -127,6 +127,28 @@ def _merge_topk_device(rows, k_best):
     return out[:min(int(k_best), int(rows.shape[0]))]
 
 
+def merge_segments(blocks):
+    """Segment by segment, the best of W per-rank (n_seg, C) row blocks (a (W, n_seg, C) array): the
+    order of merge_topk -- larger column 0 first, NaN as -inf, ties by the other columns in ascending
+    lexicographic order with NaN last, then the lower rank.  A segment no rank has a point of keeps
+    (-inf, NaN...).  For a lattice with ascending axes the tie-break is the lattice index, so the result
+    is the rows of one cvb_lattice_profile call over the whole lattice.  Vectorised over the segments."""
+    blocks = np.asarray(blocks, dtype=np.float64)
+    best = blocks[0].copy()
+    for other in blocks[1:]:
+        a = np.where(np.isnan(other[:, 0]), -np.inf, other[:, 0])
+        b = np.where(np.isnan(best[:, 0]), -np.inf, best[:, 0])
+        take = a > b
+        undecided = a == b
+        for col in range(1, blocks.shape[2]):
+            u = np.where(np.isnan(other[:, col]), np.inf, other[:, col])
+            v = np.where(np.isnan(best[:, col]), np.inf, best[:, col])
+            take |= undecided & (u < v)
+            undecided &= u == v
+        best[take] = other[take]
+    return best
+
+
 def sharded_best_rows(evaluate_slice, total, k_best, block=1):
     """Every rank evaluates its slice (runs of `block` indices, dealt round-robin) with
     `evaluate_slice(first, stride, block, count)` -> (k_best, C) best-first rows, the row blocks

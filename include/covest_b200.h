@@ -127,6 +127,25 @@ CVB_API int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const double
                      int64_t first, int64_t stride, int64_t block, int64_t count, double *out_ll,
                      int k_best, double *out_rows, void *stream);
 
+/* The best point of every segment of a lattice slice: the building block of a profile likelihood
+ * (for each value of the kept parameters, the best log-likelihood over the others).  The lattice and
+ * the slice are those of cvb_lattice_eval (same arguments, same values).  Bit a of keep_mask set keeps
+ * axis a; the segment of a point is the mixed-radix number of its kept-axis digits in axis order, the
+ * last kept axis fastest, and n_seg is the product of the kept axes' lengths.  out_rows (host or
+ * device) receives n_seg rows of (1 + n_param) doubles, row-major: for each segment (loglik, params...)
+ * of its best slice point in the order of cvb_topk -- larger value first, NaN as -inf, -0 tied with +0,
+ * ties to the lower lattice index -- with the value cvb_topk reports for it (a NaN as -inf) and the
+ * axis values bit for bit.  A segment with no point in the slice gets (-inf, NaN...); a segment whose
+ * points are all -inf or NaN gets -inf and the axis values of its lowest lattice index.  For strictly
+ * increasing axes "lower lattice index" and "lexicographically smaller params" are the same, which is
+ * the tie-break of cvb_merge_rows: per-rank rows of a sharded lattice merge segment by segment into
+ * the rows of one call.  With a device out_rows the call only enqueues work; with a host out_rows it
+ * synchronises the stream once.  CVB_EINVAL for keep_mask == 0, a bit at or above n_param, or an n_seg
+ * (or its rows' byte count) that does not fit an int64. */
+CVB_API int cvb_lattice_profile(cvb_ctx *ctx, const int32_t *axis_len, const double *axis_values,
+                                int64_t first, int64_t stride, int64_t block, int64_t count,
+                                uint32_t keep_mask, double *out_rows, void *stream);
+
 /* Measures the FP64 roofline denominator on the context's device: kind 0 = dependent-free DFMA
  * chains, kind 1 = DMMA m8n8k4 chains, kind 2 = both at once (half of the warps each), all register
  * resident.  *out_tflops = best of `reps`. */
