@@ -88,6 +88,21 @@ def load():
     L.cvb_n_param.argtypes = [vp]
     L.cvb_device_sm_count.restype = ctypes.c_int
     L.cvb_device_sm_count.argtypes = [vp]
+    L.cvb_kmer_table_create.restype = ctypes.c_int
+    L.cvb_kmer_table_create.argtypes = [ctypes.c_int, i64, ctypes.c_int, ctypes.c_int, ctypes.c_int,
+                                        ctypes.POINTER(vp)]
+    L.cvb_kmer_table_destroy.restype = None
+    L.cvb_kmer_table_destroy.argtypes = [vp]
+    L.cvb_kmer_last_error.restype = ctypes.c_char_p
+    L.cvb_kmer_last_error.argtypes = [vp]
+    L.cvb_kmer_clear.restype = ctypes.c_int
+    L.cvb_kmer_clear.argtypes = [vp, vp]
+    L.cvb_kmer_count.restype = ctypes.c_int
+    L.cvb_kmer_count.argtypes = [vp, vp, i64, vp]
+    L.cvb_kmer_stats.restype = ctypes.c_int
+    L.cvb_kmer_stats.argtypes = [vp, vp, vp]
+    L.cvb_kmer_histogram.restype = ctypes.c_int
+    L.cvb_kmer_histogram.argtypes = [vp, i64, vp, vp]
     _lib = L
     return L
 
@@ -95,4 +110,5 @@ def load():
 EXPORTS = ('cvb_ctx_create', 'cvb_ctx_destroy', 'cvb_last_error', 'cvb_loglik_batch',
            'cvb_probs_batch', 'cvb_topk', 'cvb_loglik_topk', 'cvb_lattice_eval', 'cvb_lattice_profile', 'cvb_fp64_peak', 'cvb_set_timing',
            'cvb_last_kernel_ms', 'cvb_set_path', 'cvb_merge_rows', 'cvb_last_path_info', 'cvb_n_param', 'cvb_device_sm_count', 'cvb_version',
-           'cvb_abi_version')
+           'cvb_abi_version', 'cvb_kmer_table_create', 'cvb_kmer_table_destroy', 'cvb_kmer_last_error',
+           'cvb_kmer_clear', 'cvb_kmer_count', 'cvb_kmer_stats', 'cvb_kmer_histogram')

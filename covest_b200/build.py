@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_DIR = os.path.join(HERE, 'lib')
 LIB_PATH = os.path.join(LIB_DIR, 'libcovest_b200.so')
-SOURCES = ['kernels.cu', 'factored.cu', 'faithful.cu', 'topk.cu', 'profile.cu', 'capi.cu']
+SOURCES = ['kernels.cu', 'factored.cu', 'faithful.cu', 'topk.cu', 'profile.cu', 'kmers.cu', 'capi.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-Xcompiler', '-fvisibility=hidden', '-Xcompiler', '-ffp-contract=off',
               '--fmad=false']

@@ -19,6 +19,7 @@
 #include "factored.h"
 #include "faithful.h"
 #include "kernels.h"
+#include "kmers.h"
 
 #define CVB_CHUNK_POINTS (1LL << 22) /* staging granularity for host-resident batches */
 #define CVB_MAX_TIMED_CHUNKS 64
@@ -1099,5 +1100,303 @@ extern "C" int cvb_fp64_peak(cvb_ctx *ctx, int kind, int reps, double *out_tflop
     cudaEventDestroy(a);
     cudaEventDestroy(b);
     *out_tflops = best;
+    return CVB_OK;
+}
+
+/* ---- k-mer counting (kmers.cu) ------------------------------------------------------------ */
+#define CVB_KMER_STAGE ((int64_t)64 << 20) /* bytes of one of the two pinned staging buffers of host input */
+
+struct cvb_kmer_table {
+    int device = 0;
+    int n_sm = 0;
+    CvkTable t = {};
+    cudaStream_t stream = nullptr;
+    cudaStream_t copy_stream = nullptr; /* host -> device copies of staged parts */
+    cudaEvent_t copied[2] = {nullptr, nullptr};   /* the copy out of pinned[b] has finished */
+    cudaEvent_t consumed[2] = {nullptr, nullptr}; /* the kernel reading staged[b] has finished */
+    unsigned char *pinned[2] = {nullptr, nullptr};
+    unsigned char *staged[2] = {nullptr, nullptr};
+    long long *d_hist = nullptr; /* histogram staging when the output is host memory */
+    size_t cap_hist = 0;
+    long long *h_words = nullptr; /* pinned: CVK_STATE_WORDS words read back */
+    cudaEvent_t order_ev = nullptr; /* as cvb_ctx: a call on another stream waits for the previous call */
+    cudaStream_t last_stream = nullptr;
+    bool order_valid = false;
+    std::string err;
+};
+
+static int kfail(cvb_kmer_table *t, int code, const std::string &msg)
+{
+    if (t)
+        t->err = msg;
+    else
+        g_create_error = msg;
+    return code;
+}
+
+#define KU(call, what)                                                                       \
+    do {                                                                                     \
+        cudaError_t e_ = (call);                                                             \
+        if (e_ != cudaSuccess)                                                               \
+            return kfail(t, CVB_ECUDA, std::string(what) + ": " + cudaGetErrorString(e_));   \
+    } while (0)
+
+static int kmer_enter(cvb_kmer_table *t, void *stream, cudaStream_t *s)
+{
+    KU(cudaSetDevice(t->device), "cudaSetDevice");
+    *s = stream ? (cudaStream_t)stream : t->stream;
+    if (t->order_valid && t->last_stream != *s)
+        KU(cudaStreamWaitEvent(*s, t->order_ev, 0), "cudaStreamWaitEvent");
+    return CVB_OK;
+}
+
+static int kmer_leave(cvb_kmer_table *t, cudaStream_t s)
+{
+    if (!t->order_ev)
+        KU(cudaEventCreateWithFlags(&t->order_ev, cudaEventDisableTiming), "cudaEventCreate");
+    KU(cudaEventRecord(t->order_ev, s), "cudaEventRecord");
+    t->last_stream = s;
+    t->order_valid = true;
+    return CVB_OK;
+}
+
+extern "C" const char *cvb_kmer_last_error(const cvb_kmer_table *t)
+{
+    return t ? t->err.c_str() : g_create_error.c_str();
+}
+
+extern "C" void cvb_kmer_table_destroy(cvb_kmer_table *t)
+{
+    if (!t)
+        return;
+    cudaSetDevice(t->device);
+    if (t->stream)
+        cudaStreamSynchronize(t->stream);
+    if (t->copy_stream)
+        cudaStreamSynchronize(t->copy_stream);
+    for (int b = 0; b < 2; b++) {
+        if (t->copied[b])
+            cudaEventDestroy(t->copied[b]);
+        if (t->consumed[b])
+            cudaEventDestroy(t->consumed[b]);
+        if (t->pinned[b])
+            cudaFreeHost(t->pinned[b]);
+        if (t->staged[b])
+            cudaFree(t->staged[b]);
+    }
+    if (t->h_words)
+        cudaFreeHost(t->h_words);
+    void *bufs[] = {t->t.slots, t->t.state, t->d_hist};
+    for (void *p : bufs)
+        if (p)
+            cudaFree(p);
+    if (t->order_ev)
+        cudaEventDestroy(t->order_ev);
+    if (t->copy_stream)
+        cudaStreamDestroy(t->copy_stream);
+    if (t->stream)
+        cudaStreamDestroy(t->stream);
+    delete t;
+}
+
+extern "C" int cvb_kmer_table_create(int k, int64_t capacity, int part, int n_parts, int device,
+                                     cvb_kmer_table **out)
+{
+    cvb_kmer_table *t = nullptr; /* errors before the table exists go to the thread-local slot */
+    if (!out)
+        return kfail(t, CVB_EINVAL, "out is NULL");
+    *out = nullptr;
+    if (k < 1 || k > 31)
+        return kfail(t, CVB_EINVAL, "k must lie in [1, 31], not " + std::to_string(k));
+    if (capacity < 1 || (capacity & (capacity - 1)) || capacity > ((int64_t)1 << 36))
+        return kfail(t, CVB_EINVAL, "capacity must be a power of two in [1, 2^36], not " + std::to_string(capacity));
+    if (n_parts < 1 || n_parts > 65536 || part < 0 || part >= n_parts)
+        return kfail(t, CVB_EINVAL, "need 0 <= part < n_parts <= 65536, not part " + std::to_string(part) +
+                                        " of " + std::to_string(n_parts));
+    int n_dev = 0;
+    cudaError_t e = cudaGetDeviceCount(&n_dev);
+    if (e != cudaSuccess || n_dev == 0) {
+        cudaGetLastError();
+        return kfail(t, CVB_ECUDA, std::string("no CUDA device: ") + (e != cudaSuccess ? cudaGetErrorString(e) : "count is 0") +
+                                       " (libcovest_b200 has no CPU path)");
+    }
+    if (device < 0 || device >= n_dev)
+        return kfail(t, CVB_EINVAL, "device ordinal out of range");
+    if ((e = cudaSetDevice(device)) != cudaSuccess)
+        return kfail(t, CVB_ECUDA, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+    t = new cvb_kmer_table();
+    t->device = device;
+    t->t.k = k;
+    t->t.mask = (unsigned long long)capacity - 1;
+    const unsigned long long reserve = capacity / 8 > 1 ? (unsigned long long)capacity / 8 : 1;
+    t->t.limit = (unsigned long long)capacity - reserve;
+    t->t.part = (unsigned int)part;
+    t->t.n_parts = (unsigned int)n_parts;
+    int rc = CVB_OK;
+    do {
+        cudaDeviceProp prop;
+        if ((e = cudaGetDeviceProperties(&prop, device)) != cudaSuccess)
+            break;
+        t->n_sm = prop.multiProcessorCount;
+        if (prop.major < 10) {
+            rc = kfail(nullptr, CVB_ECUDA, std::string("device is ") + prop.name + "; this library holds sm_100a code only");
+            break;
+        }
+        if ((e = cudaStreamCreateWithFlags(&t->stream, cudaStreamNonBlocking)) != cudaSuccess)
+            break;
+        if ((e = cudaMalloc((void **)&t->t.slots, (size_t)capacity * sizeof(CvkSlot))) != cudaSuccess) {
+            rc = kfail(nullptr, CVB_ENOMEM, "cudaMalloc of " + std::to_string(capacity) + " slots (" +
+                                                std::to_string((size_t)capacity * sizeof(CvkSlot)) + " bytes): " +
+                                                cudaGetErrorString(e));
+            cudaGetLastError();
+            break;
+        }
+        if ((e = cudaMalloc((void **)&t->t.state, CVK_STATE_WORDS * sizeof(unsigned long long))) != cudaSuccess)
+            break;
+        if ((e = cudaMallocHost((void **)&t->h_words, CVK_STATE_WORDS * sizeof(long long))) != cudaSuccess)
+            break;
+        if ((e = cvk_launch_clear(t->t, t->n_sm, t->stream)) != cudaSuccess)
+            break;
+        e = cudaStreamSynchronize(t->stream);
+    } while (0);
+    if (rc == CVB_OK && e != cudaSuccess)
+        rc = kfail(nullptr, CVB_ECUDA, std::string("k-mer table setup: ") + cudaGetErrorString(e));
+    if (rc != CVB_OK) {
+        cvb_kmer_table_destroy(t);
+        return rc;
+    }
+    *out = t;
+    return CVB_OK;
+}
+
+extern "C" int cvb_kmer_clear(cvb_kmer_table *t, void *stream)
+{
+    if (!t)
+        return CVB_EINVAL;
+    cudaStream_t s;
+    if (int rc = kmer_enter(t, stream, &s))
+        return rc;
+    KU(cvk_launch_clear(t->t, t->n_sm, s), "k-mer clear launch");
+    return kmer_leave(t, s);
+}
+
+/* the two pinned and two device staging buffers of host input, made on first use */
+static int kmer_staging(cvb_kmer_table *t)
+{
+    if (t->copy_stream)
+        return CVB_OK;
+    for (int b = 0; b < 2; b++) {
+        KU(cudaMallocHost((void **)&t->pinned[b], CVB_KMER_STAGE), "cudaMallocHost(k-mer staging)");
+        KU(cudaMalloc((void **)&t->staged[b], CVB_KMER_STAGE), "cudaMalloc(k-mer staging)");
+        KU(cudaEventCreateWithFlags(&t->copied[b], cudaEventDisableTiming), "cudaEventCreate");
+        KU(cudaEventCreateWithFlags(&t->consumed[b], cudaEventDisableTiming), "cudaEventCreate");
+    }
+    KU(cudaStreamCreateWithFlags(&t->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
+    return CVB_OK;
+}
+
+extern "C" int cvb_kmer_count(cvb_kmer_table *t, const uint8_t *seq, int64_t n, void *stream)
+{
+    if (!t)
+        return CVB_EINVAL;
+    if (n < 0 || (n > 0 && !seq))
+        return kfail(t, CVB_EINVAL, "need n >= 0 and a buffer");
+    cudaStream_t s;
+    if (int rc = kmer_enter(t, stream, &s))
+        return rc;
+    if (n == 0)
+        return kmer_leave(t, s);
+    if (is_device_ptr(seq)) {
+        KU(cvk_launch_count(t->t, seq, n, t->n_sm, s), "k-mer count launch");
+        return kmer_leave(t, s);
+    }
+    if (int rc = kmer_staging(t))
+        return rc;
+    /* Parts of at most CVB_KMER_STAGE bytes; each after the first repeats the k - 1 bytes before it, so
+     * that every window of the buffer lies whole in exactly one part.  The host copies part i into
+     * pinned[i % 2] while the device copies and counts part i - 1. */
+    const int64_t halo = t->t.k - 1;
+    int64_t start = 0;
+    for (int64_t i = 0; start < n; i++) {
+        const int b = (int)(i & 1);
+        const int64_t lo = i == 0 ? 0 : start - halo;
+        const int64_t hi = std::min(n, lo + CVB_KMER_STAGE);
+        if (i >= 2)
+            KU(cudaEventSynchronize(t->copied[b]), "cudaEventSynchronize");
+        memcpy(t->pinned[b], seq + lo, (size_t)(hi - lo));
+        if (i >= 2)
+            KU(cudaStreamWaitEvent(t->copy_stream, t->consumed[b], 0), "cudaStreamWaitEvent");
+        KU(cudaMemcpyAsync(t->staged[b], t->pinned[b], (size_t)(hi - lo), cudaMemcpyHostToDevice, t->copy_stream),
+           "cudaMemcpyAsync(k-mer part)");
+        KU(cudaEventRecord(t->copied[b], t->copy_stream), "cudaEventRecord");
+        KU(cudaStreamWaitEvent(s, t->copied[b], 0), "cudaStreamWaitEvent");
+        KU(cvk_launch_count(t->t, t->staged[b], hi - lo, t->n_sm, s), "k-mer count launch");
+        KU(cudaEventRecord(t->consumed[b], s), "cudaEventRecord");
+        start = hi;
+    }
+    if (int rc = kmer_leave(t, s))
+        return rc;
+    KU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+    return CVB_OK;
+}
+
+extern "C" int cvb_kmer_stats(cvb_kmer_table *t, int64_t out[4], void *stream)
+{
+    if (!t)
+        return CVB_EINVAL;
+    if (!out)
+        return kfail(t, CVB_EINVAL, "out is NULL");
+    cudaStream_t s;
+    if (int rc = kmer_enter(t, stream, &s))
+        return rc;
+    KU(cudaMemsetAsync(t->t.state + CVK_DISTINCT, 0, 3 * sizeof(unsigned long long), s), "cudaMemsetAsync");
+    KU(cvk_launch_stats(t->t, t->n_sm, s), "k-mer stats launch");
+    const bool dev = is_device_ptr(out);
+    KU(cudaMemcpyAsync(dev ? (void *)out : (void *)t->h_words, t->t.state, 4 * sizeof(int64_t),
+                       dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s),
+       "cudaMemcpyAsync(stats)");
+    if (int rc = kmer_leave(t, s))
+        return rc;
+    if (!dev) {
+        KU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+        memcpy(out, t->h_words, 4 * sizeof(int64_t));
+    }
+    return CVB_OK;
+}
+
+extern "C" int cvb_kmer_histogram(cvb_kmer_table *t, int64_t n_bins, int64_t *out_hist, void *stream)
+{
+    if (!t)
+        return CVB_EINVAL;
+    if (n_bins < 1 || !out_hist)
+        return kfail(t, CVB_EINVAL, "need n_bins >= 1 and an output buffer");
+    cudaStream_t s;
+    if (int rc = kmer_enter(t, stream, &s))
+        return rc;
+    /* a table that dropped a k-mer has no right histogram: read the count first (one synchronisation) */
+    KU(cudaMemcpyAsync(t->h_words + CVK_DROPPED, t->t.state + CVK_DROPPED, sizeof(long long), cudaMemcpyDeviceToHost, s),
+       "cudaMemcpyAsync(dropped)");
+    KU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
+    if (int rc = kmer_leave(t, s))
+        return rc;
+    const long long dropped = t->h_words[CVK_DROPPED];
+    if (dropped)
+        return kfail(t, CVB_ENOMEM, "the k-mer table is full: " + std::to_string(dropped) +
+                                        " k-mers were dropped (a larger table or more parts holds them)");
+    const bool dev = is_device_ptr(out_hist);
+    long long *dh = (long long *)out_hist;
+    if (!dev) {
+        KU(grow(&t->d_hist, &t->cap_hist, (size_t)n_bins), "cudaMalloc(histogram)");
+        dh = t->d_hist;
+    }
+    KU(cudaMemsetAsync(dh, 0, (size_t)n_bins * sizeof(long long), s), "cudaMemsetAsync(histogram)");
+    KU(cvk_launch_histogram(t->t, n_bins, dh, t->n_sm, s), "k-mer histogram launch");
+    if (!dev)
+        KU(cudaMemcpyAsync(out_hist, dh, (size_t)n_bins * sizeof(long long), cudaMemcpyDeviceToHost, s),
+           "cudaMemcpyAsync(histogram)");
+    if (int rc = kmer_leave(t, s))
+        return rc;
+    if (!dev)
+        KU(cudaStreamSynchronize(s), "cudaStreamSynchronize");
     return CVB_OK;
 }

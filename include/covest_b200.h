@@ -193,6 +193,49 @@ CVB_API int cvb_n_param(const cvb_ctx *ctx);
 CVB_API int cvb_device_sm_count(const cvb_ctx *ctx);
 CVB_API const char *cvb_version(void);
 
+/* ---- k-mer counting (DESIGN.md section 11) ------------------------------------------------------
+ * The step before an estimate: canonical k-mers of sequence bytes counted in a device hash table,
+ * and the abundance histogram a context is created from.  A table has its own handle (a likelihood
+ * context needs a histogram to exist) and follows the conventions above: 0 or a negative CVB_E*,
+ * the message from cvb_kmer_last_error(t) (t may be NULL for a failed create), `stream` as void*
+ * (NULL = the table's own stream), host or device buffers, and one synchronisation per call with a
+ * host buffer.  Calls of one table on different streams are ordered as those of a context.
+ *
+ * The table is open-addressed with linear probing over `capacity` (a power of two, at most 2^36)
+ * 16-byte slots: a uint64 key, the 2-bit packed canonical k-mer (the smaller of the k-mer and its
+ * reverse complement, A=0 C=1 G=2 T=3), and a uint64 count.  At most capacity - max(1, capacity / 8)
+ * slots are ever occupied; a k-mer that finds no room then is *dropped* (counted, not inserted).
+ * With n_parts > 1 the table holds only the k-mers of part `part`, chosen by hash bits of the key
+ * that do not pick its slot: tables of parts 0..n_parts-1 together hold every k-mer once. */
+typedef struct cvb_kmer_table cvb_kmer_table;
+
+/* CVB_EINVAL for k outside [1, 31], a capacity that is not a power of two in [1, 2^36] and part
+ * outside [0, n_parts); CVB_ENOMEM when the device cannot hold the slots.  The table starts empty. */
+CVB_API int cvb_kmer_table_create(int k, int64_t capacity, int part, int n_parts, int device,
+                                  cvb_kmer_table **out);
+CVB_API void cvb_kmer_table_destroy(cvb_kmer_table *t);
+CVB_API const char *cvb_kmer_last_error(const cvb_kmer_table *t);
+
+/* empties the table and zeroes its statistics */
+CVB_API int cvb_kmer_clear(cvb_kmer_table *t, void *stream);
+
+/* Counts every window of k consecutive bases of seq[0, n) (host or device).  A base is one of
+ * ACGTacgt; any other byte (N, IUPAC codes, a separator between reads) ends the windows through it.
+ * Nothing is kept between calls: a k-mer across two calls is not counted, so cut at read
+ * boundaries.  A host buffer is staged through two pinned buffers of the table; the copy of one part
+ * overlaps the counting of the previous one. */
+CVB_API int cvb_kmer_count(cvb_kmer_table *t, const uint8_t *seq, int64_t n, void *stream);
+
+/* out (host or device) = {distinct k-mers, total k-mers (sum of counts), largest count, dropped
+ * k-mers} of the table (of its part). */
+CVB_API int cvb_kmer_stats(cvb_kmer_table *t, int64_t out[4], void *stream);
+
+/* out_hist[j - 1] (host or device, n_bins >= 1 entries) = number of distinct k-mers seen exactly j
+ * times; counts above n_bins go into out_hist[n_bins - 1].  Reads the dropped count first, so the call
+ * always synchronises the stream once; if anything was dropped it returns CVB_ENOMEM with the count in
+ * the message and leaves out_hist as it was. */
+CVB_API int cvb_kmer_histogram(cvb_kmer_table *t, int64_t n_bins, int64_t *out_hist, void *stream);
+
 /* Bumped whenever a signature or the meaning of an argument changes; a binding compares it with
  * the version it was written against before it calls anything else (covest_b200/_capi.py). */
 #define CVB_ABI_VERSION 2
