@@ -39,14 +39,13 @@ def is_stale():
     return any(os.path.getmtime(d) > t for d in _deps())
 
 
-def build_library(force=False, verbose=False, extra_flags=()):
-    """Compile the library if it is missing or older than its sources; returns its path.
-    extra_flags: additional nvcc flags (tuning experiments: -DCVF_PE=8 ...)."""
+def build_library(force=False, verbose=False):
+    """Compile the library if it is missing or older than its sources; returns its path."""
     if not force and not is_stale():
         return LIB_PATH
     os.makedirs(LIB_DIR, exist_ok=True)
     nvcc = find_nvcc()
-    cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + (['-Xptxas', '-v'] if verbose else []) + ['-shared'] + \
+    cmd = [nvcc] + NVCC_FLAGS + (['-Xptxas', '-v'] if verbose else []) + ['-shared'] + \
         [os.path.join(CSRC, s) for s in SOURCES] + ['-o', LIB_PATH]
     if verbose:
         print(' '.join(cmd), file=sys.stderr)
@@ -55,5 +54,4 @@ def build_library(force=False, verbose=False, extra_flags=()):
 
 
 if __name__ == '__main__':
-    print(build_library(force='--force' in sys.argv, verbose='-v' in sys.argv,
-                        extra_flags=[a for a in sys.argv[1:] if a.startswith('-D')]))
+    print(build_library(force='--force' in sys.argv, verbose='-v' in sys.argv))

@@ -23,7 +23,7 @@
 
 #define CVB_CHUNK_POINTS (1LL << 22) /* staging granularity for host-resident batches */
 #define CVB_MAX_TIMED_CHUNKS 64
-#define CVB_TOPK_SORT_MIN 32768 /* batches from this size on select their top-K by a radix sort */
+#define CVB_TOPK_RADIX_MIN 32768 /* batches from this size on select their top-K by a radix selection or sort */
 
 struct cvb_ctx {
     int device = 0;
@@ -349,10 +349,6 @@ extern "C" int cvb_ctx_create(int model_kind, int k, int r, int max_error, int n
         if (const char *pm = getenv("COVEST_B200_PATH"))
             c->path_mode = !strcmp(pm, "direct") ? 1 : !strcmp(pm, "factored") ? 2 : !strcmp(pm, "gemm") ? 3
                            : !strcmp(pm, "prefix") ? 4 : !strcmp(pm, "faithful") ? 5 : 0;
-        if (const char *pv = getenv("COVEST_B200_PREFIX_KERNEL")) /* which prefix kernel (factored.cu, cvf_eval) */
-            c->fw.prefix_version = atoi(pv);
-        if (const char *to = getenv("COVEST_B200_TILE_ORDER")) /* 0 = by descending cost, 1 = group by group */
-            c->fw.tile_interleave = atoi(to) != 0;
         if (const char *wl = getenv("COVEST_B200_PROFILE_MIB"))
             if (atoll(wl) > 0)
                 c->w_limit = (size_t)atoll(wl) * (1 << 20) / sizeof(double);
@@ -704,13 +700,13 @@ static int topk_device(cvb_ctx *ctx, const CvLattice &lat, const double *d_ll, c
         if ((rc = poison_fill(ctx, ctx->d_rows, (size_t)K * (1 + CV_MAX_PARAMS), s)))
             return rc;
     }
-    if (n >= CVB_TOPK_SORT_MIN && cv_topk_select_fits(n, K) && !getenv("COVEST_B200_TOPK_SORT")) {
+    if (n >= CVB_TOPK_RADIX_MIN && cv_topk_select_fits(n, K)) {
         /* large batch, few rows wanted: radix selection (topk.cu) */
         CU(grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, cv_topk_select_bytes()), "cudaMalloc(topk scratch)");
         CU(cv_launch_topk_radix_select(d_ll, n, K, ctx->d_topk_scratch, ctx->n_sm, ctx->d_sel_ll, ctx->d_sel_idx, s),
            "top-K selection");
         ctx->last_launches += 1;
-    } else if (n >= CVB_TOPK_SORT_MIN && n <= 0x7fffffffLL) { /* large batch: one radix sort (topk.cu) */
+    } else if (n >= CVB_TOPK_RADIX_MIN && n <= 0x7fffffffLL) { /* large batch: one radix sort (topk.cu) */
         const size_t need = cv_topk_sort_bytes(n);
         CU(grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, need), "cudaMalloc(topk scratch)");
         CU(cv_launch_topk_sort(d_ll, n, K, ctx->d_topk_scratch, ctx->cap_topk_scratch, ctx->d_sel_ll,

@@ -16,8 +16,6 @@
  *                       numbers, per point the three-term combination + epilogue (the default for
  *                       batches whose points share q, as lattices do); warps per CTA and slots per
  *                       thread are template parameters picked to cover a row in one pass
- *   cvf_prefix2_kernel  the same on bulk copies (TMA) through an mbarrier ring, 8 slots per
- *                       thread; selectable, slower (DESIGN.md section 5.2)
  *   cvf_weights_kernel, cvf_gemm_kernel   K1b, K2: one CTA per tile of 128 points: copy weights and
  *                       FP64 tensor-core GEMM + epilogue (batches that share (c, e) but not q)
  *
@@ -33,7 +31,6 @@
 #include <cub/device/device_scan.cuh>
 
 #include <algorithm>
-#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -71,7 +68,6 @@ struct CvfPlan {
     int obits;         /* bits of O_thr in the sort key: enough for max(hist) + padding */
     int tile_points;   /* points per tile of K2 (the prefix kernel's tiles are whole q-runs) */
     int prefix;        /* 1: sorted by (c, e), q, O_thr and tiled for the prefix kernel */
-    int pnq, ppb;      /* tiles of the prefix kernel: at most pnq q-runs with at most ppb points together */
 };
 
 /* slots a copy takes in a term tile of the profile kernel: S rounded up to a multiple of 4 */
@@ -183,12 +179,11 @@ __global__ void __launch_bounds__(256) cvf_group_starts(long long n, CvfPlan pl)
         atomicMax(pl.g_omax + (gid - 1), pl.othr[pl.idx_sorted[i]]);
 }
 
-/* Tiles of the prefix kernel of group g: up to pl.pnq consecutive whole q-runs with at most
- * pl.ppb points together (one batch of the kernel; CVF_PNQ / CVF_PPB for the first version of the
- * kernel, V2_NQ / V2_PB for the second), or one longer run alone, cut every CVF_PSPLIT points.
- * emit(first sorted position, points, first run, runs). */
-#define CVF_PNQ 4
-#define CVF_PPB 512
+/* Tiles of the prefix kernel of group g: up to CVF_NQ consecutive whole q-runs with at most
+ * CVF_PB points together (one batch of the kernel), or one longer run alone, cut every CVF_PSPLIT
+ * points.  emit(first sorted position, points, first run, runs). */
+#define CVF_NQ 4   /* q-runs whose running sums a thread of the prefix kernel holds */
+#define CVF_PB 512 /* points per batch of the prefix kernel */
 #define CVF_PSPLIT 2048
 template <class F>
 __device__ __forceinline__ int cvf_prefix_tiles(const CvfPlan &pl, int g, F emit)
@@ -198,9 +193,9 @@ __device__ __forceinline__ int cvf_prefix_tiles(const CvfPlan &pl, int g, F emit
     while (r < r1) {
         const int first = pl.r_start[r], rfirst = r;
         int end = first, runs = 0;
-        while (r < r1 && runs < pl.pnq) {
+        while (r < r1 && runs < CVF_NQ) {
             const int re = pl.r_start[r + 1];
-            if (runs > 0 && re - first > pl.ppb)
+            if (runs > 0 && re - first > CVF_PB)
                 break;
             end = re;
             r++;
@@ -393,27 +388,20 @@ cvf_lattice_fill(CvfPlan pl, CvfLatticeDev T, int G, int M, int R, int nq, int n
 }
 
 /* The order in which the CTAs draw the tiles of the groups g0 .. g1 - 1 (every group has the same
- * tiles).  interleave = 0: by descending cost over the whole range, i.e. first every group's costliest
- * tile -- the ones that stream the long copy series of the smallest q -- then the next ...;
- * interleave = 1: group by group, inside a group by descending cost, so that the CTAs in flight hold
- * all kinds of tiles and the HBM traffic of the long series spreads over the whole kernel.  Measured:
- * cfg3 1.50 ms against 1.44 ms (the costly tiles finishing last leave SMs idle at the end), cfg5
- * 27.4 against 27.8 ms -- the default stays 0 (COVEST_B200_TILE_ORDER). */
+ * tiles): by descending cost over the whole range, i.e. first every group's costliest tile -- the
+ * ones that stream the long copy series of the smallest q -- then the next ...  Group by group
+ * (inside a group by descending cost, so that the HBM traffic of the long series spreads over the
+ * whole kernel) measured cfg3 1.50 ms against 1.44 ms -- its costly tiles finishing last leave SMs
+ * idle at the end -- and cfg5 27.4 against 27.8 ms. */
 __global__ void __launch_bounds__(256)
-cvf_lattice_order(CvfLatticeDev T, int g0, int g1, int nT, int interleave, int *__restrict__ out)
+cvf_lattice_order(CvfLatticeDev T, int g0, int g1, int nT, int *__restrict__ out)
 {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const int ng = g1 - g0;
     if (i >= (long long)ng * nT)
         return;
-    int k, g;
-    if (interleave) {
-        g = g0 + (int)(i / nT);
-        k = (int)(i - (long long)(g - g0) * nT);
-    } else {
-        k = (int)(i / ng);
-        g = g0 + (int)(i - (long long)k * ng);
-    }
+    const int k = (int)(i / ng);
+    const int g = g0 + (int)(i - (long long)k * ng);
     out[i] = g * nT + T.tt_order[k];
 }
 
@@ -444,9 +432,10 @@ __device__ __forceinline__ int cvf_find_warp(const int *__restrict__ start, int 
  * their order, and -- when there are others -- one more line with the column sums of the others
  * (CvfSlots, factored.h): the bins without counts enter the result through the mass only, and the
  * mass is linear in the profiles.  Without a tail the mass does not enter at all: the tables K1 runs
- * on are then the row tables of the lines with counts, and the line of the sums holds zeros.  K1 writes 512 contiguous bytes per (copy, line) with one warp-wide store; the prefix
- * kernel fetches whole rows (a pass of 1024 slots = 8 KB contiguous) with bulk copies; K2 scatters
- * 16 rows x one line into its fragment order while loading. */
+ * on are then the row tables of the lines with counts, and the line of the sums holds zeros.  K1
+ * writes 512 contiguous bytes per (copy, line) with one warp-wide store; every thread of the prefix
+ * kernel fetches its own slots of a row, one double per slot, into a private cp.async ring; K2
+ * scatters 16 rows x one line into its fragment order while loading. */
 #define CVF_STAGE_DOUBLES (CV_GB * CV_NA_MAX * CV_W)
 
 /* The accumulators of a lane after the slices of ONE copy are its share of the profile of that
@@ -1032,21 +1021,11 @@ cvf_gemm_kernel(const __grid_constant__ CvModelDesc m, CvfPlan pl, int first_til
  * doubles of one copy and one N-step in the layout of K1); warp w takes the half-lines
  * u = i * NW + w, i < SL, lane l the double l of each.  Bins with counts usually are the
  * first ones of the histogram, so this deals them evenly to the warps. */
-#define CVF_NQ CVF_PNQ /* q-runs whose running sums a thread holds */
-#ifndef CVF_WARPS_SM
 #define CVF_WARPS_SM 16 /* warps per SM the register budget of the prefix kernel is cut for */
-#endif
-#define CVF_PB CVF_PPB /* points per batch */
-#ifndef CVF_PD
 #define CVF_PD 4       /* copies in flight per thread (cp.async ring in shared memory) */
-#endif
-#ifndef CVF_PL2
 #define CVF_PL2 6      /* copies ahead of the ring that are requested into L2 */
-#endif
-#ifndef CVF_PE
 #define CVF_PE 8       /* points whose lane partials wait in the transpose buffer of a warp (4: 1.45 ms on cfg3, 8: 1.35 ms) */
-#endif
-#define CVF_PEW 33     /* doubles per row of that buffer (odd: conflict-free both ways) */
+#define CVF_PEW 33    /* doubles per row of that buffer (odd: conflict-free both ways) */
 
 struct __align__(16) CvfEvent {
     double q1, two, many;
@@ -1080,12 +1059,8 @@ __device__ __forceinline__ void cvf_sts64(unsigned int a, double v)
     asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory");
 }
 
-#ifndef CVF_LOG_REP
-#define CVF_LOG_REP 1
-#endif
-/* CVF_LOG_REP: 8 interleaved copies make the lookups free of bank conflicts; measured: no gain (1.444 ms either way) */
 struct CvfPrefixSmem {
-    double log_tab[2 * CV_LOG_N * CVF_LOG_REP]; /* CVF_LOG_REP interleaved copies of cv_log_table */
+    double log_tab[2 * CV_LOG_N]; /* cv_log_table */
     /* the points of the batch by ascending cut-off (the schedule), 32 bytes each: weights of
      * copy 1, copy 2 and of the running sum; batch position | run << 16; copies = O_thr - 1 */
     CvfEvent ev[CVF_PB + 2];
@@ -1111,47 +1086,6 @@ static size_t cvf_prefix_smem_bytes(bool mass, int nw, int sl)
            planes * (size_t)nw * CVF_PE * CVF_PEW * sizeof(double);
 }
 
-/* ---- mbarrier and bulk-copy (TMA) primitives of the prefix kernels ---- */
-__device__ __forceinline__ void cvf_mbar_init(unsigned int bar, unsigned int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void cvf_mbar_expect_tx(unsigned int bar, unsigned int bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void cvf_mbar_arrive(unsigned int bar)
-{
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cvf_mbar_wait(unsigned int bar, unsigned int parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred P1;\n"
-        "CVF_MB_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-        "@P1 bra CVF_MB_DONE;\n"
-        "bra CVF_MB_WAIT;\n"
-        "CVF_MB_DONE:\n"
-        "}\n" ::"r"(bar),
-        "r"(parity)
-        : "memory");
-}
-/* global -> shared bulk copy (TMA), completion counted in bytes on the mbarrier */
-__device__ __forceinline__ void cvf_bulk_load(unsigned int dst, const void *src, unsigned int bytes, unsigned int bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar)
-                 : "memory");
-}
-
-/* a row segment on its way from HBM to L2, nothing lands in shared memory */
-__device__ __forceinline__ void cvf_bulk_prefetch_l2(const void *src, unsigned int bytes)
-{
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(src), "r"(bytes) : "memory");
-}
-
 /* safe_log (utils.py:32-35) off the fast path: below the band limit (cvmodel.h CV_PSCALE), zero,
  * negative, infinite, NaN */
 __device__ __noinline__ double cvf_log_rare(double x)
@@ -1167,57 +1101,34 @@ __device__ __noinline__ double cvf_log_rare(double x)
  * table at the shared-window address `tab_s`; everything else takes cvf_log_rare.
  *
  * |r| <= 2^-8 on every table interval, so log1p(r) - r = r^2 (-1/2 + r/3 - r^2/4 + r^3/5) leaves
- * r^6/6 <= 5.9e-16: with CVF_LOG_DEG 5 (the default) the logarithm is 9 FP64 instructions in four
- * dependent steps -- k ln 2 + logc in one FMA (|k| <= 1100: 0.3 ulp of the result from the rounded
- * ln 2), hi + r, and the polynomial joined by a last FMA.  Measured against logl over 4e7 arguments:
- * relative error <= 9.3e-16 for x < 0.6875 (every probability of a bin that is not ~1), absolute
- * error <= 5.8e-16 on [0.6875, 1.375).  CVF_LOG_DEG 7 is the earlier form (r^7 kept, ln 2 split in
- * two, 14 instructions in six steps, 2.5e-16 (1 + |log x|)): the count-weighted sum has a 1e-9 gate
- * and sees neither.  The coefficient of r^3 and those of r^5 .. r^7 are cut to 20 mantissa bits
- * (they fit the immediate field of the FP64 instructions; errors below 2^-58). */
-/* REP: copies of the table side by side (entry e of copy c at 16 (e REP + c) bytes; tab_s already points
- * at the lane's copy): with 8 copies the 8 lanes of a quarter warp read 8 different 16-byte bank groups
- * whatever their arguments -- the lookups are free of bank conflicts */
-#ifndef CVF_LOG_DEG
-#define CVF_LOG_DEG 5
-#endif
+ * r^6/6 <= 5.9e-16: the logarithm is 9 FP64 instructions in four dependent steps -- k ln 2 + logc in
+ * one FMA (|k| <= 1100: 0.3 ulp of the result from the rounded ln 2), hi + r, and the polynomial
+ * joined by a last FMA.  Measured against logl over 4e7 arguments: relative error <= 9.3e-16 for
+ * x < 0.6875 (every probability of a bin that is not ~1), absolute error <= 5.8e-16 on
+ * [0.6875, 1.375); the count-weighted sum has a 1e-9 gate.  The coefficient 1/5 of r^5 is cut to 20
+ * mantissa bits (it fits the immediate field of the FP64 instructions; error below 2^-58). */
 /* the fast path of cvf_safe_log alone: x positive, normal, finite */
-template <int REP = 1>
 __device__ __forceinline__ double cvf_log_fast(double x, unsigned int tab_s)
 {
     const int hi = __double2hiint(x);
     const int t = hi - (int)(CV_LOG_OFF >> 32);
     const double z = __hiloint2double(hi - (t & (int)0xfff00000), __double2loint(x));
-    const double2 c = REP == 8 ? cvf_lds128(tab_s + ((t >> 6) & ((CV_LOG_N - 1) << 7)))
-                                : cvf_lds128(tab_s + ((t >> 9) & ((CV_LOG_N - 1) << 4))); /* (invc, logc) of interval (t >> 13) & 127 */
+    const double2 c = cvf_lds128(tab_s + ((t >> 9) & ((CV_LOG_N - 1) << 4))); /* (invc, logc) of interval (t >> 13) & 127 */
     const double r = cv_fma(z, c.x, -1.0);
     const double kd = (double)((t >> 20) - CV_PSCALE_EXP); /* log(x 2^-128) */
     const double r2 = cv_mul(r, r);
     const double a = cv_fma(r, 1.0 / 3.0, -0.5);
     const double b = cv_fma(r, 0x1.9999ap-3 /* 1/5 */, -0.25);
-#if CVF_LOG_DEG == 5
     const double hi_part = cv_fma(kd, 0x1.62e42fefa39efp-1, c.y);
     const double p = cv_fma(r2, b, a);
     return cv_fma(r2, p, cv_add(hi_part, r)); /* hi_part + r does not wait for the polynomial */
-#else
-    const double hi_part = cv_fma(kd, 0x1.62e42p-1, c.y); /* ln 2 to 20 bits: k * ln2_hi stays exact */
-    /* log1p(r) - r = r^2 (-1/2 + r/3 - r^2/4 + r^3/5 - r^4/6 + r^5/7), in three short dependent
-     * steps (Estrin) instead of five */
-    const double c2 = cv_fma(r, 0x1.24925p-3 /* 1/7 */, -0x1.55555p-3 /* 1/6 */);
-    const double r4 = cv_mul(r2, r2);
-    const double ab = cv_fma(r2, b, a);
-    const double p = cv_fma(r4, c2, ab);
-    const double lo = cv_fma(r2, p, cv_mul(kd, 0x1.fdf473de6af28p-22)); /* ln 2 - 0x1.62e42p-1 */
-    return cv_add(cv_add(hi_part, r), lo);
-#endif
 }
 
-template <int REP = 1>
 __device__ __forceinline__ double cvf_safe_log(double x, unsigned int tab_s)
 {
     if ((unsigned int)(__double2hiint(x) - CVF_FAST_LO) >= CVF_FAST_SPAN)
         return cvf_log_rare(x);
-    return cvf_log_fast<REP>(x, tab_s);
+    return cvf_log_fast(x, tab_s);
 }
 
 /* number of entries of the ascending a[0..n) that are < x (strict) resp. <= x */
@@ -1267,12 +1178,11 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
     double *red_all = scratch + (size_t)blockIdx.x * (3 * PW_ * CVF_PB);
     double *red = red_all + warp * CVF_PB; /* plane stride PW_ * CVF_PB */
     const unsigned int ring_s = cvf_pin((unsigned int)__cvta_generic_to_shared(ring));
-    /* the lane's copy of the logarithm table */
-    const unsigned int log_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.log_tab) + (unsigned int)((lane & (CVF_LOG_REP - 1)) * 16));
+    const unsigned int log_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.log_tab));
     const unsigned int ev_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.ev));
     const unsigned int tbuf_s = cvf_pin((unsigned int)__cvta_generic_to_shared(tbuf + lane)); /* the lane's column */
-    for (int i = tid; i < 2 * CV_LOG_N * CVF_LOG_REP; i += PT_) /* entry e of copy c: doubles 2 (e REP + c) .. + 1 */
-        S.log_tab[i] = log_tab[2 * (i / (2 * CVF_LOG_REP)) + (i & 1)];
+    for (int i = tid; i < 2 * CV_LOG_N; i += PT_)
+        S.log_tab[i] = log_tab[i];
     /* nslots: the slots of a row that can be other than zero (a multiple of 32; the line of the sums ends after its first half) */
     const long long row_stride = (long long)nsteps * CVF_NS; /* doubles between the rows of consecutive copies */
 
@@ -1565,9 +1475,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                             CVF_CASE(0)
                             CVF_CASE(1)
                             CVF_CASE(2)
-#if CVF_PNQ > 3
                             CVF_CASE(3)
-#endif
 #undef CVF_CASE
                         }
                         while (o_done < need_next)
@@ -1583,9 +1491,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                             CVF_CASE(0)
                             CVF_CASE(1)
                             CVF_CASE(2)
-#if CVF_PNQ > 3
                             CVF_CASE(3)
-#endif
 #undef CVF_CASE
                         }
                         const int pt_a = info & 0xffff, pt_b = info_next & 0xffff;
@@ -1612,11 +1518,11 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                                                cb = (unsigned int)(__double2hiint(pb[0]) - CVF_FAST_LO);
                             double la, lb;
                             if (ca < CVF_FAST_SPAN && cb < CVF_FAST_SPAN) { /* both on the fast path */
-                                la = cvf_log_fast<CVF_LOG_REP>(pa[0], log_s);
-                                lb = cvf_log_fast<CVF_LOG_REP>(pb[0], log_s);
+                                la = cvf_log_fast(pa[0], log_s);
+                                lb = cvf_log_fast(pb[0], log_s);
                             } else {
-                                la = cvf_safe_log<CVF_LOG_REP>(pa[0], log_s);
-                                lb = cvf_safe_log<CVF_LOG_REP>(pb[0], log_s);
+                                la = cvf_safe_log(pa[0], log_s);
+                                lb = cvf_safe_log(pb[0], log_s);
                             }
                             sa = cv_mul(hcnt[0], la);
                             sb = cv_mul(hcnt[0], lb);
@@ -1629,8 +1535,8 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                              * of a slot without a count is not used */
 #pragma unroll
                             for (int i = 0; i < SL; i++) {
-                                const double la = cvf_log_fast<CVF_LOG_REP>(pa[i], log_s),
-                                             lb = cvf_log_fast<CVF_LOG_REP>(pb[i], log_s);
+                                const double la = cvf_log_fast(pa[i], log_s),
+                                             lb = cvf_log_fast(pb[i], log_s);
                                 double ta = cv_mul(hcnt[i], la), tb = cv_mul(hcnt[i], lb);
                                 if (hcnt[i] == 0.0)
                                     ta = tb = 0.0;
@@ -1645,11 +1551,11 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                                                        cb = (unsigned int)(__double2hiint(pb[i]) - CVF_FAST_LO);
                                     double la, lb;
                                     if (ca < CVF_FAST_SPAN && cb < CVF_FAST_SPAN) {
-                                        la = cvf_log_fast<CVF_LOG_REP>(pa[i], log_s);
-                                        lb = cvf_log_fast<CVF_LOG_REP>(pb[i], log_s);
+                                        la = cvf_log_fast(pa[i], log_s);
+                                        lb = cvf_log_fast(pb[i], log_s);
                                     } else {
-                                        la = cvf_safe_log<CVF_LOG_REP>(pa[i], log_s);
-                                        lb = cvf_safe_log<CVF_LOG_REP>(pb[i], log_s);
+                                        la = cvf_safe_log(pa[i], log_s);
+                                        lb = cvf_safe_log(pb[i], log_s);
                                     }
                                     double ta = cv_mul(hcnt[i], la), tb = cv_mul(hcnt[i], lb);
                                     if (hcnt[i] == 0.0)
@@ -1696,9 +1602,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                         CVF_CASE(0)
                         CVF_CASE(1)
                         CVF_CASE(2)
-#if CVF_PNQ > 3
                         CVF_CASE(3)
-#endif
 #undef CVF_CASE
                     }
                     q1 = qt_next.x;
@@ -1714,7 +1618,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                             cvf_two_sum_acc(mh, ml, p[i]);
                     }
                     if (ONE ? log_mask != 0 : log_mask == 1) { /* the usual case: the warp's first half-line holds the bins with counts */
-                        double term = cv_mul(hcnt[0], cvf_safe_log<CVF_LOG_REP>(p[0], log_s)); /* utils.py:32-35 */
+                        double term = cv_mul(hcnt[0], cvf_safe_log(p[0], log_s)); /* utils.py:32-35 */
                         if (hcnt[0] == 0.0) /* models.py:106 `if h` */
                             term = 0.0;
                         sum = term;
@@ -1722,7 +1626,7 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
 #pragma unroll
                         for (int i = 0; i < SL; i++)
                             if ((log_mask >> i) & 1) { /* some lane of the warp has a count in its slot i */
-                                double term = cv_mul(hcnt[i], cvf_safe_log<CVF_LOG_REP>(p[i], log_s));
+                                double term = cv_mul(hcnt[i], cvf_safe_log(p[i], log_s));
                                 if (hcnt[i] == 0.0)
                                     term = 0.0;
                                 sum = cv_add(sum, term);
@@ -1759,482 +1663,6 @@ cvf_prefix_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__
                     }
                 }
                 out_ll[pl.idx_sorted[b0 + t]] = MASS ? cv_point_finish(m, part) : part.sum;
-            }
-            b0 += npts;
-            __syncthreads();
-        }
-    }
-}
-
-/* ------------------------------------------------------------------------------------------- */
-/* K2p, second version: bulk-copy (TMA) pipeline, 8 slots per thread                            */
-/* ------------------------------------------------------------------------------------------- */
-/* Same computation as cvf_prefix_kernel (one running sum per q-run over the copy numbers, every
- * point finished when its copies are in), different machine mapping:
- *
- *   - the profile rows of the copies travel by cp.async.bulk (the TMA engine, UBLKCP in SASS): one
- *     elected thread asks for a whole row segment of a pass (1024 slots = 8 KB, contiguous in the
- *     row-major layout K1 writes) per copy; a stage holds V2_CPS copies, V2_NST stages form a ring
- *     with an mbarrier pair (full / empty) per stage.  The per-thread 8-byte cp.async ring of the
- *     first version (4 LDGSTS + ring addressing per copy and thread, bank conflicts between the
- *     rings) is gone; a thread reads its slots of a copy with four conflict-free LDS.128;
- *   - 4 warps per CTA and 8 slots per thread (a pass is still 1024 slots): the bookkeeping per
- *     point (schedule record, run dispatch, partial sums into the transpose buffer) is paid once
- *     per 8 bins instead of once per 4; two q-runs per tile keep the running sums in 32 registers;
- *     3 CTAs per SM (170 registers, nothing spills);
- *   - a thread's slots are whole pairs of the lines w, w + 4, w + 8, w + 12 of the pass (line = 64
- *     slots): the bins with counts -- the first ones of a histogram -- are again dealt evenly to
- *     the warps, two logarithms per lane and counted line, side by side. */
-#define V2_SL 8
-#define V2_PT 128
-#define V2_PW (V2_PT / 32)
-#define V2_NQ 2
-#define V2_PB 256
-#define V2_PE 4
-#define V2_PEW 33
-#define V2_NST 3
-#define V2_CPS 2
-#define V2_PFG 8 /* groups ahead of the ring whose rows are prefetched into L2 */
-#define V2_PASS (V2_PT * V2_SL)
-#define V2_COPY_BYTES (V2_PASS * 8)
-#define V2_TBUF_DOUBLES (V2_PW * V2_PE * V2_PEW)
-
-struct CvfPrefix2Smem {
-    unsigned long long full_bar[V2_NST], empty_bar[V2_NST];
-    double log_tab[2 * CV_LOG_N];
-    CvfEvent ev[V2_PB + 2];
-    int need[V2_PB];
-    double base[V2_NQ];
-    int seg[V2_NQ + 1];
-    int tile, bend;
-    /* then: double stage[V2_NST][V2_CPS][V2_PASS] (128-byte aligned),
-     *       double tbuf[planes][V2_PW][V2_PE][V2_PEW] */
-};
-
-static size_t cvf_prefix2_stage_offset() { return (sizeof(CvfPrefix2Smem) + 127) & ~(size_t)127; }
-static size_t cvf_prefix2_smem_bytes(bool mass)
-{
-    return cvf_prefix2_stage_offset() + (size_t)V2_NST * V2_CPS * V2_COPY_BYTES +
-           (mass ? 3 : 2) * V2_TBUF_DOUBLES * sizeof(double);
-}
-
-template <bool MASS, bool FULL>
-__global__ void __launch_bounds__(V2_PT, 3)
-cvf_prefix2_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__ CvLattice lat,
-                   const double *__restrict__ params, int clip, CvfPlan pl, int first_tile, int n_tiles,
-                   const double *__restrict__ W, long long w_base, const double2 *__restrict__ slot_mh,
-                   const double *__restrict__ log_tab, int nsteps, double *__restrict__ out_ll,
-                   unsigned long long *counter, double *__restrict__ scratch)
-{
-    extern __shared__ __align__(128) unsigned char cvf_smem_raw[];
-    CvfPrefix2Smem &S = *reinterpret_cast<CvfPrefix2Smem *>(cvf_smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const size_t stage_off = (sizeof(CvfPrefix2Smem) + 127) & ~(size_t)127;
-    double *tbuf = reinterpret_cast<double *>(cvf_smem_raw + stage_off + (size_t)V2_NST * V2_CPS * V2_COPY_BYTES) +
-                   warp * (V2_PE * V2_PEW); /* plane stride V2_TBUF_DOUBLES */
-    double *red_all = scratch + (size_t)blockIdx.x * (3 * V2_PW * V2_PB);
-    double *red = red_all + warp * V2_PB; /* plane stride V2_PW * V2_PB */
-    const unsigned int stage_s = cvf_pin((unsigned int)__cvta_generic_to_shared(cvf_smem_raw + stage_off));
-    /* the thread's pair `lane` of line `warp` of copy 0 of stage 0 */
-    const unsigned int mine_s = cvf_pin(stage_s + (unsigned int)((warp * 64 + 2 * lane) * 8));
-    const unsigned int full_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.full_bar));
-    const unsigned int empty_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.empty_bar));
-    const unsigned int log_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.log_tab));
-    const unsigned int ev_s = cvf_pin((unsigned int)__cvta_generic_to_shared(S.ev));
-    const unsigned int tbuf_s = cvf_pin((unsigned int)__cvta_generic_to_shared(tbuf + lane)); /* the lane's column */
-    for (int i = tid; i < 2 * CV_LOG_N; i += V2_PT)
-        S.log_tab[i] = log_tab[i];
-    if (tid == 0) {
-        for (int s = 0; s < V2_NST; s++) {
-            cvf_mbar_init(full_s + 8 * s, 1);       /* the producer's arrive.expect_tx */
-            cvf_mbar_init(empty_s + 8 * s, V2_PW);  /* one arrival per consumer warp */
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    const int nslots = nsteps * CVF_NS;
-    const long long row_stride = (long long)nslots;
-    /* groups of copies consumed so far by this CTA: every thread counts the same sequence */
-    unsigned int gcount = 0;
-
-    for (;;) {
-        __syncthreads();
-        if (tid == 0)
-            S.tile = (int)atomicAdd(counter, 1ULL);
-        __syncthreads();
-        if (S.tile >= n_tiles)
-            break;
-        const int tile = pl.t_sorted[S.tile];
-        const int tfirst = pl.t_first[tile], tend = tfirst + pl.t_cnt[tile];
-        const double *Wg = W + (pl.w_off[pl.t_group[tile]] - w_base);
-
-        for (int b0 = tfirst; b0 < tend;) {
-            /* ---- the batch: up to V2_PB points in up to V2_NQ q-runs ---- */
-            const int nload = min(V2_PB, tend - b0);
-            const int rid0 = pl.rid[b0];
-            if (tid == 0)
-                S.bend = nload;
-            if (tid <= V2_NQ)
-                S.seg[tid] = nload;
-            __syncthreads();
-            for (int t = tid; t < nload; t += V2_PT) {
-                const int rel = pl.rid[b0 + t] - rid0;
-                if (rel >= V2_NQ)
-                    atomicMin(&S.bend, t);
-                else if (t == 0 || pl.head2[b0 + t])
-                    S.seg[rel] = t;
-            }
-            __syncthreads();
-            const int npts = S.bend;
-            constexpr int PPT = V2_PB / V2_PT;
-            double pq1[PPT], ptwo[PPT], pmany[PPT];
-#pragma unroll
-            for (int j = 0; j < PPT; j++) {
-                const int t = tid + j * V2_PT;
-                pq1[j] = ptwo[j] = pmany[j] = 0.0;
-                if (t < npts) {
-                    const unsigned int pi = pl.idx_sorted[b0 + t];
-                    double row[CV_MAX_PARAMS];
-                    cvf_raw_row(m, lat, params, pi, row);
-                    const double q1 = cvf_clipped(m, row, clip, 2), q2 = cvf_clipped(m, row, clip, 3),
-                                 qq = cvf_clipped(m, row, clip, 4);
-                    const int need = pl.othr[pi] - 1;
-                    /* copies beyond the cut-off do not enter (models.py:235): exact zero weights */
-                    pq1[j] = need >= 1 ? q1 : 0.0;
-                    ptwo[j] = need >= 2 ? cv_mul(cv_sub(1.0, q1), q2) : 0.0;
-                    pmany[j] = need >= 3 ? cv_mul(cv_mul(cv_sub(1.0, q1), cv_sub(1.0, q2)), qq) : 0.0;
-                    S.need[t] = need;
-                    if (t == 0 || pl.head2[b0 + t])
-                        S.base[pl.rid[b0 + t] - rid0] = cv_sub(1.0, qq);
-                }
-            }
-            __syncthreads();
-            int seg0[V2_NQ], seg_end[V2_NQ], last_need[V2_NQ];
-            double base[V2_NQ];
-            int omax_b = 0;
-#pragma unroll
-            for (int s = 0; s < V2_NQ; s++) {
-                seg0[s] = min(S.seg[s], npts);
-                seg_end[s] = s + 1 < V2_NQ ? min(S.seg[s + 1], npts) : npts;
-                if (seg_end[s] < seg0[s])
-                    seg_end[s] = seg0[s];
-                base[s] = seg_end[s] > seg0[s] ? S.base[s] : 0.0;
-                last_need[s] = seg_end[s] > seg0[s] ? S.need[seg_end[s] - 1] : -1;
-                omax_b = max(omax_b, last_need[s]);
-            }
-            /* the schedule: rank of a point = points before it by (copies, run, position) */
-#pragma unroll
-            for (int j = 0; j < PPT; j++) {
-                const int t = tid + j * V2_PT;
-                if (t < npts) {
-                    const int need = S.need[t];
-                    int rank = 0, mine = 0;
-#pragma unroll
-                    for (int s = 0; s < V2_NQ; s++)
-                        if (t >= seg0[s] && t < seg_end[s]) {
-                            mine = s;
-                            rank += t - seg0[s];
-                        }
-#pragma unroll
-                    for (int s = 0; s < V2_NQ; s++)
-                        if (s != mine && seg_end[s] > seg0[s])
-                            rank += cvf_count_below(S.need + seg0[s], seg_end[s] - seg0[s], need, s < mine);
-                    CvfEvent e;
-                    e.q1 = pq1[j];
-                    e.two = ptwo[j];
-                    e.many = pmany[j];
-                    e.info = t | (mine << 16);
-                    e.need = need;
-                    S.ev[rank] = e;
-                }
-            }
-            if (tid < 2) { /* read ahead by the loop below, never used */
-                CvfEvent e;
-                e.q1 = e.two = e.many = 0.0;
-                e.info = e.need = 0;
-                S.ev[npts + tid] = e;
-            }
-            __syncthreads();
-
-            /* ---- passes over the slots ---- */
-            const int n_groups_pass = (omax_b + V2_CPS - 1) / V2_CPS;
-            for (int pass0 = 0; pass0 < nslots; pass0 += V2_PASS) {
-                const unsigned int pass_bytes = (unsigned int)(min(V2_PASS, nslots - pass0) * 8);
-                const double *src_pass = Wg + pass0; /* row 0 (copy 1), first slot of the pass */
-                /* the thread's slots: pair `lane` of the lines i * V2_PW + warp, i < 4 */
-                bool live[4];
-                int log_mask = 0;
-                const int slot0 = pass0 + warp * 64 + 16 * (lane >> 3) + (lane & 7);
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    live[i] = FULL || pass0 + (i * V2_PW + warp) * 64 < nslots;
-                    bool counted = false;
-                    if (live[i])
-                        counted = __ldg(&slot_mh[slot0 + i * V2_PW * 64].y) != 0.0 ||
-                                  __ldg(&slot_mh[slot0 + i * V2_PW * 64 + 8].y) != 0.0;
-                    log_mask |= (__any_sync(CV_FULL_MASK, counted) ? 1 : 0) << i;
-                }
-                const double h0a = live[0] ? __ldg(&slot_mh[slot0].y) : 0.0, h0b = live[0] ? __ldg(&slot_mh[slot0 + 8].y) : 0.0;
-                /* the producer: group g of the pass holds copies g * V2_CPS + 1 .. of which those up
-                 * to omax_b exist; it goes to stage (gbase + g) % V2_NST once every warp has
-                 * released the group that used the stage before */
-                const unsigned int gbase = gcount;
-                auto produce = [&](int g) {
-                    const unsigned int G = gbase + (unsigned int)g;
-                    const unsigned int st = G % V2_NST;
-                    if (G >= V2_NST)
-                        cvf_mbar_wait(empty_s + 8 * st, ((G / V2_NST) & 1) ^ 1);
-                    const int o_first = g * V2_CPS + 1;
-                    const int ncp = min(V2_CPS, omax_b - o_first + 1);
-                    cvf_mbar_expect_tx(full_s + 8 * st, pass_bytes * (unsigned int)ncp);
-                    for (int c = 0; c < ncp; c++)
-                        cvf_bulk_load(stage_s + (st * V2_CPS + c) * V2_COPY_BYTES,
-                                      src_pass + (long long)(o_first - 1 + c) * row_stride, pass_bytes,
-                                      full_s + 8 * st);
-                    /* the rows of the copies V2_PFG groups further on start their way from HBM to L2
-                     * (the ring itself only covers L2 latency) */
-                    for (int c = 0; c < V2_CPS; c++) {
-                        const int o_far = o_first + V2_PFG * V2_CPS + c;
-                        if (o_far <= omax_b)
-                            cvf_bulk_prefetch_l2(src_pass + (long long)(o_far - 1) * row_stride, pass_bytes);
-                    }
-                };
-                if (tid == 0) {
-                    for (int o = V2_NST * V2_CPS + 1; o <= min(omax_b, V2_PFG * V2_CPS); o++)
-                        cvf_bulk_prefetch_l2(src_pass + (long long)(o - 1) * row_stride, pass_bytes);
-                    for (int g = 0; g < V2_NST && g < n_groups_pass; g++)
-                        produce(g);
-                }
-                int g_local = 0, cidx = 0, o_taken = 0;
-                unsigned int stage = gbase % V2_NST, fparity = (gbase / V2_NST) & 1;
-                auto take = [&](double *x) { /* the next copy's profile for the thread's slots */
-                    if (cidx == 0) {
-                        cvf_mbar_wait(full_s + 8 * stage, fparity);
-                        /* the stage the previous group has left is refilled by one thread, a
-                         * different warp's each time */
-                        if (g_local >= 1 && g_local - 1 + V2_NST < n_groups_pass && tid == ((g_local % V2_PW) << 5))
-                            produce(g_local - 1 + V2_NST);
-                    }
-                    const unsigned int at = mine_s + (stage * V2_CPS + cidx) * V2_COPY_BYTES;
-#pragma unroll
-                    for (int i = 0; i < 4; i++) {
-                        const double2 v = cvf_lds128(at + i * (V2_PW * 64 * 8));
-                        x[2 * i] = live[i] ? v.x : 0.0;
-                        x[2 * i + 1] = live[i] ? v.y : 0.0;
-                    }
-                    cidx++;
-                    o_taken++;
-                    if (cidx == V2_CPS || o_taken == omax_b) { /* the group is consumed */
-                        __syncwarp();
-                        if (lane == 0)
-                            cvf_mbar_arrive(empty_s + 8 * stage);
-                        cidx = 0;
-                        g_local++;
-                        gcount++;
-                        if (++stage == V2_NST) {
-                            stage = 0;
-                            fparity ^= 1;
-                        }
-                    }
-                };
-                double P1[V2_SL], P2[V2_SL];
-#pragma unroll
-                for (int i = 0; i < V2_SL; i++)
-                    P1[i] = P2[i] = 0.0;
-                if (omax_b >= 1)
-                    take(P1);
-                if (omax_b >= 2)
-                    take(P2);
-                double R[V2_NQ][V2_SL], w[V2_NQ];
-#pragma unroll
-                for (int s = 0; s < V2_NQ; s++) {
-#pragma unroll
-                    for (int i = 0; i < V2_SL; i++)
-                        R[s][i] = 0.0;
-                    w[s] = 1.0;
-                }
-                const bool first_pass = pass0 == 0;
-                int pending = 0; /* points in the transpose buffer */
-                int mypt = 0;    /* lane e: the point in row e of the buffer */
-                auto flush = [&]() {
-                    __syncwarp();
-                    /* lane group g = lane / V2_PE takes the columns g * V2_PE .. + V2_PE - 1 of row e */
-                    const int e = lane & (V2_PE - 1), c0 = (lane / V2_PE) * V2_PE;
-                    const double *rowp = tbuf + e * V2_PEW + c0;
-                    double acc0 = rowp[0], acc1 = rowp[V2_TBUF_DOUBLES], acc2 = 0.0;
-                    if (MASS)
-                        acc2 = rowp[2 * V2_TBUF_DOUBLES];
-#pragma unroll
-                    for (int c = 1; c < V2_PE; c++) {
-                        acc0 = cv_add(acc0, rowp[c]);
-                        if (MASS) {
-                            cvf_two_sum_acc(acc1, acc2, rowp[V2_TBUF_DOUBLES + c]);
-                            acc2 = cv_add(acc2, rowp[2 * V2_TBUF_DOUBLES + c]);
-                        } else {
-                            acc1 = cv_add(acc1, rowp[V2_TBUF_DOUBLES + c]);
-                        }
-                    }
-#pragma unroll
-                    for (int d = V2_PE; d <= 16; d <<= 1) {
-                        acc0 = cv_add(acc0, __shfl_xor_sync(CV_FULL_MASK, acc0, d));
-                        const double oh = __shfl_xor_sync(CV_FULL_MASK, acc1, d);
-                        if (MASS) {
-                            const double ol = __shfl_xor_sync(CV_FULL_MASK, acc2, d);
-                            cvf_two_sum_acc(acc1, acc2, oh);
-                            acc2 = cv_add(acc2, ol);
-                        } else {
-                            acc1 = cv_add(acc1, oh);
-                        }
-                    }
-                    const int pt = __shfl_sync(CV_FULL_MASK, mypt, e);
-                    if (lane < pending) {
-                        double *r0 = red + pt, *r1 = r0 + V2_PW * V2_PB, *r2 = r1 + V2_PW * V2_PB;
-                        if (first_pass) {
-                            *r0 = acc0;
-                            *r1 = acc1;
-                            if (MASS)
-                                *r2 = acc2;
-                        } else {
-                            *r0 = cv_add(*r0, acc0);
-                            if (MASS) {
-                                double h = *r1, l = *r2;
-                                cvf_two_sum_acc(h, l, acc1);
-                                *r1 = h;
-                                *r2 = cv_add(l, acc2);
-                            } else {
-                                *r1 = cv_add(*r1, acc1);
-                            }
-                        }
-                    }
-                    pending = 0;
-                    __syncwarp();
-                };
-                int o_done = min(omax_b, 2);
-                unsigned int ev_a = ev_s;
-                double q1, two, many;
-                int info, need;
-                {
-                    const double2 qt = cvf_lds128(ev_a);
-                    q1 = qt.x;
-                    two = qt.y;
-                    cvf_lds_event(ev_a, many, info, need);
-                }
-                unsigned int tb_a = tbuf_s; /* row `pending` of the transpose buffer */
-                for (int k = 0; k < npts; k++) {
-                    /* the next point's record travels while this one is worked on */
-                    ev_a += (unsigned int)sizeof(CvfEvent);
-                    const double2 qt_next = cvf_lds128(ev_a);
-                    double many_next;
-                    int info_next, need_next;
-                    cvf_lds_event(ev_a, many_next, info_next, need_next);
-                    while (o_done < need) { /* one more copy into the running sums */
-                        o_done++;
-                        double x[V2_SL];
-                        take(x);
-#pragma unroll
-                        for (int s = 0; s < V2_NQ; s++)
-                            if (o_done <= last_need[s]) { /* runs whose points are all out need no more copies */
-#pragma unroll
-                                for (int i = 0; i < V2_SL; i++)
-                                    R[s][i] = cv_fma(w[s], x[i], R[s][i]);
-                                w[s] = cv_mul(w[s], base[s]);
-                            }
-                    }
-                    /* the three-term combination for the thread's slots, models.py:235-241 */
-                    const int pt = info & 0xffff;
-                    double p[V2_SL];
-#pragma unroll
-                    for (int i = 0; i < V2_SL; i++)
-                        p[i] = cv_fma(two, P2[i], cv_mul(q1, P1[i]));
-                    if ((info >> 16) & 1) {
-#pragma unroll
-                        for (int i = 0; i < V2_SL; i++)
-                            p[i] = cv_fma(many, R[1][i], p[i]);
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < V2_SL; i++)
-                            p[i] = cv_fma(many, R[0][i], p[i]);
-                    }
-                    q1 = qt_next.x;
-                    two = qt_next.y;
-                    many = many_next;
-                    info = info_next;
-                    need = need_next;
-                    /* models.py:100-107 for the thread's slots: the mass ... */
-                    double mh, ml = 0.0;
-                    if (MASS) {
-                        mh = 0.0;
-#pragma unroll
-                        for (int i = 0; i < V2_SL; i++)
-                            cvf_two_sum_acc(mh, ml, p[i]);
-                    } else {
-                        mh = cv_add(cv_add(cv_add(p[0], p[1]), cv_add(p[2], p[3])),
-                                    cv_add(cv_add(p[4], p[5]), cv_add(p[6], p[7])));
-                    }
-                    /* ... and the logarithms of the lines that hold bins with counts, two side by side.
-                     * The bins with counts usually are the first ones of the histogram: the thread's
-                     * first line, whose counts stay in registers. */
-                    double sum = 0.0;
-                    auto two_logs = [&](double pa, double pb, double ha, double hb) {
-                        const unsigned int ca = (unsigned int)(__double2hiint(pa) - CVF_FAST_LO),
-                                           cb = (unsigned int)(__double2hiint(pb) - CVF_FAST_LO);
-                        double la, lb;
-                        if (ca < CVF_FAST_SPAN && cb < CVF_FAST_SPAN) {
-                            la = cvf_log_fast(pa, log_s);
-                            lb = cvf_log_fast(pb, log_s);
-                        } else {
-                            la = cvf_safe_log(pa, log_s); /* utils.py:32-35 */
-                            lb = cvf_safe_log(pb, log_s);
-                        }
-                        double ta = cv_mul(ha, la), tb = cv_mul(hb, lb);
-                        if (ha == 0.0) /* models.py:106 `if h` */
-                            ta = 0.0;
-                        if (hb == 0.0)
-                            tb = 0.0;
-                        sum = cv_add(sum, cv_add(ta, tb));
-                    };
-                    if (log_mask & 1)
-                        two_logs(p[0], p[1], h0a, h0b);
-                    if (log_mask & 14) {
-#pragma unroll
-                        for (int i = 1; i < 4; i++)
-                            if ((log_mask >> i) & 1)
-                                two_logs(p[2 * i], p[2 * i + 1], __ldg(&slot_mh[slot0 + i * V2_PW * 64].y),
-                                         __ldg(&slot_mh[slot0 + i * V2_PW * 64 + 8].y));
-                    }
-                    cvf_sts64(tb_a, sum);
-                    cvf_sts64(tb_a + V2_TBUF_DOUBLES * 8, mh);
-                    if (MASS)
-                        cvf_sts64(tb_a + 2 * V2_TBUF_DOUBLES * 8, ml);
-                    tb_a += V2_PEW * 8;
-                    if (lane == pending)
-                        mypt = pt;
-                    if (++pending == V2_PE) {
-                        flush();
-                        tb_a = tbuf_s;
-                    }
-                }
-                if (pending)
-                    flush();
-                /* copies nobody needed (none: the schedule ends at omax_b) -- every produced group
-                 * has been consumed, the ring is balanced for the next pass */
-            }
-            __syncthreads();
-            for (int t = tid; t < npts; t += V2_PT) {
-                CvPartial part;
-                part.sum = red_all[t];
-                part.mass_h = red_all[V2_PW * V2_PB + t];
-                part.mass_l = MASS ? red_all[2 * V2_PW * V2_PB + t] : 0.0;
-                for (int wv = 1; wv < V2_PW; wv++) {
-                    part.sum = cv_add(part.sum, red_all[wv * V2_PB + t]);
-                    if (MASS) {
-                        cvf_two_sum_acc(part.mass_h, part.mass_l, red_all[(V2_PW + wv) * V2_PB + t]);
-                        part.mass_l = cv_add(part.mass_l, red_all[(2 * V2_PW + wv) * V2_PB + t]);
-                    } else {
-                        part.mass_h = cv_add(part.mass_h, red_all[(V2_PW + wv) * V2_PB + t]);
-                    }
-                }
-                out_ll[pl.idx_sorted[b0 + t]] = cv_point_finish(m, part);
             }
             b0 += npts;
             __syncthreads();
@@ -2293,7 +1721,7 @@ static double cvf_host_clip(const CvModelDesc &m, double v, int clip, int a)
 }
 
 static void cvf_lattice_template(const CvModelDesc &m, int clip, const double *q1v, int n1, const double *q2v,
-                                 int n2, const double *qv, int nq, int pnq, int ppb, CvfLatticeCache &T)
+                                 int n2, const double *qv, int nq, CvfLatticeCache &T)
 {
     const int R = n1 * n2, M = R * nq;
     T.M = M;
@@ -2339,9 +1767,9 @@ static void cvf_lattice_template(const CvModelDesc &m, int clip, const double *q
     for (int r = 0; r < nq;) {
         const int first = r * R, rfirst = r;
         int end = first, runs = 0;
-        while (r < nq && runs < pnq) {
+        while (r < nq && runs < CVF_NQ) {
             const int re = (r + 1) * R;
-            if (runs > 0 && re - first > ppb)
+            if (runs > 0 && re - first > CVF_PB)
                 break;
             end = re;
             r++;
@@ -2497,13 +1925,6 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
     if (wk.timed)
         CVF_CK(cudaEventRecord(wk.ev[0], stream));
 
-    /* which prefix kernel: 1 = cvf_prefix_kernel (8 warps, 4 slots per thread, thread-private cp.async
-     * rings: the default, it is the faster one -- DESIGN.md section 5.2); 2 = cvf_prefix2_kernel (4 warps,
-     * 8 slots per thread, rows by bulk copies through an mbarrier ring) */
-    const int pver = wk.prefix_version == 2 ? 2 : 1;
-    pl.pnq = pver == 2 ? V2_NQ : CVF_PNQ;
-    pl.ppb = pver == 2 ? V2_PB : CVF_PPB;
-
     /* K0 .. totals for one ordering of the points; ends with the header on the host */
     auto build_plan = [&](int prefix) -> cudaError_t {
         pl.prefix = prefix;
@@ -2551,10 +1972,8 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
         CvfLatticeCache &T = wk.lattice;
         const int n1 = lat.len[2], n2 = lat.len[3], nq = lat.len[4];
         std::vector<double> key;
-        key.reserve(6 + n1 + n2 + nq);
+        key.reserve(4 + n1 + n2 + nq);
         key.push_back((double)clip);
-        key.push_back((double)pl.pnq);
-        key.push_back((double)pl.ppb);
         key.push_back((double)n1);
         key.push_back((double)n2);
         key.push_back((double)nq);
@@ -2564,8 +1983,7 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
         const bool same = key.size() == T.key.size() && T.dev &&
                           memcmp(key.data(), T.key.data(), key.size() * sizeof(double)) == 0;
         if (!same) {
-            cvf_lattice_template(m, clip, lat_axes_host[2], n1, lat_axes_host[3], n2, lat_axes_host[4], nq, pl.pnq,
-                                 pl.ppb, T);
+            cvf_lattice_template(m, clip, lat_axes_host[2], n1, lat_axes_host[3], n2, lat_axes_host[4], nq, T);
             const size_t ints = T.host.size();
             if (ints > T.dev_cap) {
                 if (T.dev)
@@ -2770,11 +2188,6 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
     CVF_CK(cudaFuncSetAttribute(cvf_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)sizeof(CvfSmem)));
     CVF_CK(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kp_smem));
-    const size_t kp2_smem = cvf_prefix2_smem_bytes(want_mass);
-    const bool full2 = (nsteps * CVF_NS) % V2_PASS == 0;
-    auto kp2 = want_mass ? (full2 ? cvf_prefix2_kernel<true, true> : cvf_prefix2_kernel<true, false>)
-                         : (full2 ? cvf_prefix2_kernel<false, true> : cvf_prefix2_kernel<false, false>);
-    CVF_CK(cudaFuncSetAttribute(kp2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kp2_smem));
     if (wk.timed)
         CVF_CK(cudaEventRecord(wk.ev[1], stream));
     for (size_t i = 0; i + 1 < cut.size(); i++) {
@@ -2805,7 +2218,7 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
             /* tiles of the range by descending cost: the long ones start first */
             if (analytic) {
                 cvf_lattice_order<<<(unsigned int)((tiles + tb - 1) / tb), tb, 0, stream>>>(
-                    TD, g0, g1, (int)(n_tiles / n_groups), wk.tile_interleave, pl.t_order_alt + tile0);
+                    TD, g0, g1, (int)(n_tiles / n_groups), pl.t_order_alt + tile0);
                 CVF_CK(cudaGetLastError());
                 pl.t_sorted = pl.t_order_alt + tile0;
             } else {
@@ -2819,20 +2232,11 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
                 CVF_CK(cudaEventRecord(wk.ev[2], stream));
             int grid = tiles < 2 * n_sm ? tiles : 2 * n_sm;
             if (prefix) {
-                int per_sm = std::max(1, std::min(CVF_WARPS_SM / kp_nw, (int)((size_t)smem_max / (kp_smem + 1024))));
-                if (const char *lim = getenv("COVEST_B200_PREFIX_CTAS")) /* development: CTAs per SM */
-                    per_sm = std::max(1, std::min(per_sm, atoi(lim)));
-                if (pver == 2) {
-                    per_sm = std::max(1, std::min(3, (int)((size_t)smem_max / (kp2_smem + 1024))));
-                    grid = tiles < per_sm * n_sm ? tiles : per_sm * n_sm;
-                    kp2<<<grid, V2_PT, kp2_smem, stream>>>(m, lat, params, clip, pl, tile0, tiles, wk.W, w0, slot_mh,
-                                                            log_tab, nsteps, out_ll, wk.d_counters + 1, wk.d_scratch);
-                } else {
-                    grid = tiles < per_sm * n_sm ? tiles : per_sm * n_sm;
-                    kp<<<grid, 32 * kp_nw, kp_smem, stream>>>(m, lat, params, clip, pl, tile0, tiles, wk.W, w0, slot_mh,
-                                                               log_tab, nsteps, kp_slots, out_ll, wk.d_counters + 1,
-                                                               wk.d_scratch);
-                }
+                const int per_sm = std::max(1, std::min(CVF_WARPS_SM / kp_nw, (int)((size_t)smem_max / (kp_smem + 1024))));
+                grid = tiles < per_sm * n_sm ? tiles : per_sm * n_sm;
+                kp<<<grid, 32 * kp_nw, kp_smem, stream>>>(m, lat, params, clip, pl, tile0, tiles, wk.W, w0, slot_mh,
+                                                           log_tab, nsteps, kp_slots, out_ll, wk.d_counters + 1,
+                                                           wk.d_scratch);
             } else {
                 cvf_gemm_kernel<<<grid, CVF_THREADS, sizeof(CvfSmem), stream>>>(
                     m, pl, tile0, tiles, wk.W, w0, A, a0, slot_mh, step_mask, log_tab, nsteps, out_ll,

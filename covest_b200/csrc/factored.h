@@ -56,8 +56,6 @@ struct CvFactorWork {
     long long n_groups = 0, n_tiles = 0, n_items = 0, w_doubles = 0, n_runs = 0;
     int prefix = 0; /* 1: the prefix kernel ran, 0: the GEMM */
     int launches = 0;
-    int prefix_version = 1; /* 1: cvf_prefix_kernel (cp.async rings), 2: cvf_prefix2_kernel (bulk copies, mbarrier ring) */
-    int tile_interleave = 0; /* lattice plans: tiles by descending cost over all groups (0, default) or group by group (1) */
     int analytic = 0; /* 1: the plan came from the lattice axes (no sort, no host synchronisation) */
     int poison = 0;   /* tests (COVEST_B200_POISON): byte W and d_scratch are filled with at each evaluation, 0 = off */
     CvfLatticeCache lattice;

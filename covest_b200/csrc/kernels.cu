@@ -14,8 +14,6 @@
  */
 #include "kernels.h"
 
-#include <cstdlib>
-
 #include "kdevice.h"
 
 __device__ __forceinline__ CvPartial cv_partial_shfl_down(const CvPartial &p, int delta)
@@ -145,9 +143,6 @@ static void cv_loglik_config(const CvModelDesc &m, int smem_max, int *n_warps, i
     long long w = ((long long)smem_max - (long long)tab) / (long long)wb;
     if (w > CV_WARPS_MAX)
         w = CV_WARPS_MAX;
-    if (const char *cap = getenv("COVEST_B200_WARPS")) /* development: occupancy experiments */
-        if (atoi(cap) >= 1 && atoi(cap) < w)
-            w = atoi(cap);
     if (w < 1)
         w = 0; /* the group tables do not fit next to one warp: the caller reports it */
     *n_warps = (int)w;

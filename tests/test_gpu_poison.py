@@ -165,10 +165,10 @@ def _basic_axes():
 
 
 # ---- part A: poisoned = clean ---------------------------------------------------------------------
-PATHS = {'auto': 0, 'per_point': 1, 'gemm': 3, 'prefix': 4, 'prefix2': 4, 'term_by_term': 5}
+PATHS = {'auto': 0, 'per_point': 1, 'gemm': 3, 'prefix': 4, 'term_by_term': 5}
 # histogram -> (k, r).  Rows per group NA: e05 1, cfg2 2, dense400 4, cfg3 8, trim120 1 with a tail of 175.
 # cfg4 (k = 31, r = 150) runs the prefix kernel's 8 x 4 geometry in several passes.  sparse700 has a tail
-# and a line of sums, whose second half only the mass reads (GEMM, second prefix kernel).
+# and a line of sums, whose second half only the GEMM reads (its mass sums whole lines).
 HISTS = {
     'e05_repeats': (21, 100), 'cfg2_repeats': (21, 100), 'dense400': (21, 100), 'cfg3_repeats_dense1000': (21, 100),
     'cfg2_repeats_trim120': (21, 100), 'cfg4_repeats_k31': (31, 150), 'sparse700': (21, 100)}
@@ -191,14 +191,14 @@ def _cases():
             for path in ('gemm', 'prefix', 'per_point'):
                 out.append((name, max(21, S - 1), 100, S, 'repeats', path, 'lattice', ()))
         for S in (1, 8, 12, 17, 32):
-            for path in ('gemm', 'prefix') + (('prefix2', 'auto') if S == 8 else ()):
+            for path in ('gemm', 'prefix') + (('auto',) if S == 8 else ()):
                 out.append((name, max(21, S - 1), 100, S, 'repeats', path, 'cuts', ()))
-    for path in ('gemm', 'prefix', 'prefix2', 'per_point'):
+    for path in ('gemm', 'prefix', 'per_point'):
         out.append(('cfg2_repeats', 21, 100, 8, 'repeats', path, 'nan_first', ()))
     for path in ('gemm', 'prefix'):
         out.append(('cfg3_repeats_dense1000', 21, 100, 8, 'repeats', path, 'lattice', (('COVEST_B200_PROFILE_MIB', '1'),)))
         out.append(('cfg3_repeats_dense1000', 21, 100, 8, 'repeats', path, 'nan_first', (('COVEST_B200_PROFILE_MIB', '1'),)))
-    for path in ('gemm', 'prefix', 'prefix2'):
+    for path in ('gemm', 'prefix'):
         out.append(('cfg2_repeats', 21, 100, 8, 'repeats', path, 'lattice', (('COVEST_B200_ROWS', 'full'),)))
     return out
 
@@ -256,11 +256,10 @@ def test_poisoned_scratch_gives_the_clean_values(case):
     name, k, r, S, kind, path, pts_kind, env = case
     m = _oracle(kind, name, k, r, S)
     pts = _points(name, pts_kind)[1]
-    env = tuple(env) + ((('COVEST_B200_PREFIX_KERNEL', '2'),) if path == 'prefix2' else ())
     with _context(m, None, env) as ctx:
         clean = _evaluate(ctx, name, path, pts_kind)
         info = ctx.last_path_info()
-    if S <= 32 and path in ('gemm', 'prefix', 'prefix2'):
+    if S <= 32 and path in ('gemm', 'prefix'):
         assert info['kernel'] == ('cvf_gemm_kernel' if path == 'gemm' else 'cvf_prefix_kernel')
     if path == 'auto' and kind == 'repeats' and len(pts) >= 2048:
         assert info['path'] == 'factored'

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """Small batches through every kernel of the library, for compute-sanitizer (memcheck, racecheck,
 synccheck, initcheck): the per-point kernel (basic and repeats, with per-bin probabilities), the plan
-kernels (general and from lattice axes), the profile kernel, both prefix kernels, the GEMM path, the
-term-by-term re-evaluation, the three top-K selections and the row merge.
+kernels (general and from lattice axes), the profile kernel, the prefix kernel (with and without a
+tail), the GEMM path, the term-by-term re-evaluation, the three top-K selections and the row merge.
 
     compute-sanitizer --tool racecheck python tools/sanitize_target.py
     compute-sanitizer --tool initcheck python tools/sanitize_target.py
@@ -29,8 +29,7 @@ p = basic.probabilities_batch(np.array([[10, .03], [25, .01]]))
 basic.close()
 done.append('basic')
 
-for tail, prefix_kernel in ((0, '2'), (1234, '2'), (0, '1')):
-    os.environ['COVEST_B200_PREFIX_KERNEL'] = prefix_kernel
+for tail in (0, 1234):
     model = RepeatsModel(21, 100, hist, tail, max_error=8)
     ctx = model.device_context
     axes = [np.geomspace(10, 90, 5), np.geomspace(.01, .09, 3), np.linspace(.3, 1, 5), np.linspace(0, 1, 5),
@@ -56,7 +55,7 @@ for tail, prefix_kernel in ((0, '2'), (1234, '2'), (0, '1')):
     ctx.topk(big, np.tile(pts, (12, 1))[:40000], 16)
     ctx.topk(b[:5000], pts[:5000], 8)
     model.close()
-    done.append('repeats tail=%s prefix kernel %s' % (tail, prefix_kernel))
+    done.append('repeats tail=%s' % tail)
 
 import torch  # noqa: E402
 rows = torch.from_numpy(np.random.default_rng(1).normal(size=(128, 6))).cuda()
