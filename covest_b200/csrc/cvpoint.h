@@ -37,7 +37,7 @@
 #define CV_CT 32       /* mixture terms per tile: one per lane */
 #define CV_RUNMAX 4    /* longest run of groups anchored from one exp() */
 #define CV_MAX_PARAMS 5
-#define CV_WARPS_MAX 12 /* warps (= points in flight) per CTA; one CTA per SM */
+#define CV_WARPS_MAX 12 /* warps (= points in flight) per CTA of the per-point kernel; one CTA per SM */
 #define CV_COPY_PAD 40  /* copies past max(hist) that copy_log still covers */
 
 /* record of a group in CvTables::grp */

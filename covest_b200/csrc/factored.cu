@@ -436,7 +436,17 @@ __device__ __forceinline__ int cvf_find_warp(const int *__restrict__ start, int 
  * writes 512 contiguous bytes per (copy, line) with one warp-wide store; every thread of the prefix
  * kernel fetches its own slots of a row, one double per slot, into a private cp.async ring; K2
  * scatters 16 rows x one line into its fragment order while loading. */
-#define CVF_STAGE_DOUBLES (CV_GB * CV_NA_MAX * CV_W)
+/* doubles of a warp's profile stage: one block of accumulators, NA rows per group */
+__host__ __device__ constexpr int cvf_stage_doubles(int na) { return CV_GB * na * CV_W; }
+/* Warps per CTA (one CTA per SM) of the K1 instantiation for NA rows per group.  Much of K1's time is
+ * the per-item header, the per-term set-up and the transpose of its stores, which wait on latency,
+ * not on a pipe: more warps hide more of it, as long as the register cap they impose does not cost
+ * more instructions.  Measured on cfg3's row tables (NA = 2): 12 warps 0.323 ms, 14 0.302, 16 0.296,
+ * 18 0.307, 20 0.305 (96 registers) -- 16 for NA <= 4.  NA = 8 spills at 16 warps and keeps 12
+ * (DESIGN.md section 6).
+ * Fewer run when the group records of a long histogram and the working sets of a large S do not
+ * fit the shared memory (the launch). */
+__host__ __device__ constexpr int cvf_k1_warps(int na) { return na <= 4 ? 16 : 12; }
 
 /* The accumulators of a lane after the slices of ONE copy are its share of the profile of that
  * copy over block `blk`: rows mt of group r, columns 8 nt + 2 q + c.  They are transposed through
@@ -527,7 +537,8 @@ __device__ __forceinline__ void cvf_profile_item(int lane, const CvModelDesc &m,
     }
 }
 
-__global__ void __launch_bounds__(32 * CV_WARPS_MAX, 1)
+template <int NA>
+__global__ void __launch_bounds__(32 * cvf_k1_warps(NA), 1)
 cvf_profile_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant__ CvLattice lat,
                    const double *__restrict__ params, int clip, CvfPlan pl, int n_groups,
                    int first_item, int n_items, double *__restrict__ W, long long w_base, int nsteps,
@@ -549,7 +560,7 @@ cvf_profile_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant_
     }
     double *stage = reinterpret_cast<double *>(cv_smem_raw + (size_t)groups_staged * CV_GD * sizeof(double) +
                                                (size_t)(blockDim.x >> 5) * cv_warp_bytes(S)) +
-                    (size_t)warp * CVF_STAGE_DOUBLES;
+                    (size_t)warp * cvf_stage_doubles(NA);
     __syncthreads();
     for (;;) {
         long long it = 0;
@@ -571,12 +582,7 @@ cvf_profile_kernel(const __grid_constant__ CvModelDesc m, const __grid_constant_
         __syncwarp();
         double *Wg = W + (pl.w_off[g] - w_base);
         const int o0 = kchunk * CVF_KC + 1;
-        switch (m.na) {
-        case 1: cvf_profile_item<1>(lane, m, M, o0, omax4, nsteps, line_map, sum_line, Wg, stage); break;
-        case 2: cvf_profile_item<2>(lane, m, M, o0, omax4, nsteps, line_map, sum_line, Wg, stage); break;
-        case 4: cvf_profile_item<4>(lane, m, M, o0, omax4, nsteps, line_map, sum_line, Wg, stage); break;
-        default: cvf_profile_item<8>(lane, m, M, o0, omax4, nsteps, line_map, sum_line, Wg, stage); break;
-        }
+        cvf_profile_item<NA>(lane, m, M, o0, omax4, nsteps, line_map, sum_line, Wg, stage);
     }
 }
 
@@ -2125,8 +2131,14 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
     const size_t wb = cv_warp_bytes(m.n_err);
     const int groups_staged = m.n_blocks * CV_GB;
     const size_t tab = (size_t)groups_staged * CV_GD * sizeof(double);
-    const size_t wb1 = wb + CVF_STAGE_DOUBLES * sizeof(double); /* working set + profile stage */
-    int k1_warps = (int)std::min<long long>(CV_WARPS_MAX, ((long long)smem_max - (long long)tab) / (long long)wb1);
+    typedef decltype(&cvf_profile_kernel<1>) CvfProfileFn;
+    const int k1_na = m.na == 1 || m.na == 2 || m.na == 4 ? m.na : 8;
+    const CvfProfileFn k1 = k1_na == 1 ? cvf_profile_kernel<1> : k1_na == 2 ? cvf_profile_kernel<2>
+                            : k1_na == 4 ? cvf_profile_kernel<4> : cvf_profile_kernel<8>;
+    const size_t wb1 = wb + cvf_stage_doubles(k1_na) * sizeof(double); /* working set + profile stage */
+    /* the instantiation's warps, or as many as the shared memory holds (NA = 8, S = 32 and 15 blocks
+     * of group records: 11) */
+    int k1_warps = (int)std::min<long long>(cvf_k1_warps(k1_na), ((long long)smem_max - (long long)tab) / (long long)wb1);
     if (k1_warps < 1)
         return cudaErrorInvalidConfiguration;
     const size_t k1_smem = tab + (size_t)k1_warps * wb1;
@@ -2184,7 +2196,7 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
                                       : (counts_first ? cvf_prefix_kernel<false, false, true, 8, 4> : cvf_prefix_kernel<false, false, false, 8, 4>));
     }
 #undef CVF_PICK
-    CVF_CK(cudaFuncSetAttribute(cvf_profile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1_smem));
+    CVF_CK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1_smem));
     CVF_CK(cudaFuncSetAttribute(cvf_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                 (int)sizeof(CvfSmem)));
     CVF_CK(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kp_smem));
@@ -2202,7 +2214,7 @@ cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *c
             int grid = (items + k1_warps - 1) / k1_warps;
             if (grid > n_sm)
                 grid = n_sm;
-            cvf_profile_kernel<<<grid, 32 * k1_warps, k1_smem, stream>>>(
+            k1<<<grid, 32 * k1_warps, k1_smem, stream>>>(
                 m, lat, params, clip, pl, (int)n_groups, item0, items, wk.W, w0, nsteps, sl.line_map, sl.sum_line,
                 wk.d_counters, groups_staged);
             CVF_CK(cudaGetLastError());
