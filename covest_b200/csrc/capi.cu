@@ -67,18 +67,14 @@ struct cvb_ctx {
     std::vector<cudaEvent_t> ev;
     int timed_chunks = 0;
     int last_launches = 0;
-    cudaStream_t timed_stream = nullptr;
     /* the factored path of the repeats model (factored.h) */
     CvFactorWork fw;
     CvModelDesc fdesc;         /* desc with the row tables of the batched path (cv_build_row_tables), or desc itself */
     CvfSlots slots;            /* the row layout of the profiles (factored.h) */
     const double *d_log_tab = nullptr;
-    int path_mode = 0;         /* 0 auto, 1 per-point kernel only, 2 factored whenever supported */
+    int path_mode = 0;         /* cvb_set_path */
     size_t w_limit = (size_t)2 << 30; /* doubles: 16 GiB of profiles per group range */
-    double min_group = 12.0;   /* auto: points per (c, e) group below which the per-point kernel runs */
-    long long min_points = 2048; /* auto: batches below this go straight to the per-point kernel */
-    int last_path = 0;         /* 1 per-point, 2 factored (GEMM), 3 factored (prefix kernel) */
-    double min_run = 4.0;      /* auto: points per q-run below which the GEMM runs instead of the prefix kernel */
+    int last_path = 0;         /* out[0] of cvb_last_path_info */
     /* re-evaluation of marked points (faithful.h) */
     CvFaithTables faith = {nullptr, nullptr, 0, 0, nullptr, 0};
     unsigned long long *d_fixed = nullptr; /* two words: marked points of the most recent evaluation, work cursor */
@@ -122,21 +118,6 @@ static bool is_device_ptr(const void *p)
         return false;
     }
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
-
-template <typename T>
-static cudaError_t grow(T **buf, size_t *cap, size_t want)
-{
-    if (want <= *cap)
-        return cudaSuccess;
-    if (*buf)
-        cudaFree(*buf);
-    *buf = nullptr;
-    *cap = 0;
-    cudaError_t e = cudaMalloc((void **)buf, want * sizeof(T));
-    if (e == cudaSuccess)
-        *cap = want;
-    return e;
 }
 
 template <typename T>
@@ -346,9 +327,11 @@ extern "C" int cvb_ctx_create(int model_kind, int k, int r, int max_error, int n
             cv_log_table(lt.data());
             if ((e = upload(c, lt, &c->d_log_tab)) != cudaSuccess) break;
         }
-        if (const char *pm = getenv("COVEST_B200_PATH"))
-            c->path_mode = !strcmp(pm, "direct") ? 1 : !strcmp(pm, "factored") ? 2 : !strcmp(pm, "gemm") ? 3
-                           : !strcmp(pm, "prefix") ? 4 : !strcmp(pm, "faithful") ? 5 : 0;
+        static const char *const path_names[] = {"auto", "direct", "factored", "gemm", "prefix", "faithful"};
+        const char *pm = getenv("COVEST_B200_PATH"); /* a name of a mode of cvb_set_path; any other: auto */
+        for (int i = 0; pm && i < 6; i++)
+            if (!strcmp(pm, path_names[i]))
+                c->path_mode = i;
         if (const char *wl = getenv("COVEST_B200_PROFILE_MIB"))
             if (atoll(wl) > 0)
                 c->w_limit = (size_t)atoll(wl) * (1 << 20) / sizeof(double);
@@ -436,6 +419,13 @@ extern "C" int cvb_last_kernel_ms(cvb_ctx *ctx, double *out_ms, int *out_launche
     return CVB_OK;
 }
 
+/* the automatic path: batches below this go straight to the per-point kernel */
+#define CVB_MIN_POINTS 2048
+
+/* what the factored path is asked to run, by path mode (cvb_set_path; modes 1 and 5 do not ask) */
+static const CvfRequest factored_request[6] = {CvfRequest::Auto, CvfRequest::Auto, CvfRequest::Forced,
+                                               CvfRequest::Gemm, CvfRequest::Prefix, CvfRequest::Auto};
+
 /* one evaluation of n points on the device, optionally bracketed by events: the factored path
  * when the batch is large and groups well (never when per-bin probabilities are wanted), else the
  * per-point kernel */
@@ -446,34 +436,31 @@ static int launch_loglik(cvb_ctx *ctx, const CvLattice &lat, const double *const
     bool timed = ctx->timing && ctx->timed_chunks < CVB_MAX_TIMED_CHUNKS;
     if (timed)
         CU(cudaEventRecord(ctx->ev[2 * ctx->timed_chunks], s), "cudaEventRecord");
-    int used = 0;
-    const bool forced = ctx->path_mode >= 2;
     const bool faithful_only = ctx->path_mode == 5 && !d_probs;
+    const CvfRequest req = factored_request[ctx->path_mode];
     const bool try_factored = !d_probs && ctx->path_mode != 1 && !faithful_only && cvf_supported(ctx->desc) &&
-                              (forced || n >= ctx->min_points);
+                              (req != CvfRequest::Auto || n >= CVB_MIN_POINTS);
+    CvfRan ran = CvfRan::None;
     if (faithful_only) {
         CU(cv_launch_mark_all(d_ll, n, s), "cv_mark_all_kernel launch");
         ctx->last_launches++;
-        used = 3;
     }
     if (try_factored) {
         ctx->fw.timed = ctx->timing;
-        CU(cvf_eval(ctx->fdesc, lat, lat_axes_host, d_params, n, clip, d_ll, ctx->slots,
-                    ctx->d_log_tab, ctx->fw, ctx->n_sm,
-                    ctx->smem_max, ctx->w_limit, forced ? 0.0 : ctx->min_group, ctx->min_run,
-                    ctx->path_mode == 3 ? 1 : ctx->path_mode == 4 ? 2 : 0, s, &used),
+        CU(cvf_eval(ctx->fdesc, lat, lat_axes_host, d_params, n, clip, d_ll, ctx->slots, ctx->d_log_tab, ctx->fw,
+                    ctx->n_sm, ctx->smem_max, ctx->w_limit, req, s, &ran),
            "factored evaluation");
         ctx->last_launches += ctx->fw.launches;
     }
-    if (!used) {
+    if (!faithful_only && ran == CvfRan::None) {
         CU(cv_launch_loglik(ctx->desc, lat, d_params, n, clip, d_ll, d_probs, ctx->d_counter, ctx->n_sm,
                             ctx->smem_max, s),
            "cv_loglik_kernel launch");
         ctx->last_launches++;
     }
-    ctx->last_path = used ? 1 + used : 1;
+    ctx->last_path = faithful_only ? 4 : ran == CvfRan::Gemm ? 2 : ran == CvfRan::Prefix ? 3 : 1;
     /* points whose value hinges on the reference's subnormal roundings: again, term by term */
-    CU(grow(&ctx->d_marked, &ctx->cap_marked, 2 * (size_t)n), "cudaMalloc(marked points)");
+    CU(cv_grow(&ctx->d_marked, &ctx->cap_marked, 2 * (size_t)n), "cudaMalloc(marked points)");
     CU(cv_launch_faithful(ctx->desc, lat, d_params, n, clip, d_ll, ctx->faith, ctx->n_sm, ctx->d_marked,
                           ctx->d_fixed, s),
        "cv_faithful_kernel launch");
@@ -521,6 +508,27 @@ static int order_leave(cvb_ctx *ctx, cudaStream_t s)
     return CVB_OK;
 }
 
+/* Enqueues the copy of n values to host memory: on the call's stream s, or with `side` on the
+ * context's copy stream after what s holds so far, so that what s does next (a top-K, the next part
+ * of a slice) runs beside it.  After its last side copy a call records copy_done on the copy stream,
+ * and s waits for that event before the call ends. */
+static int copy_values_out(cvb_ctx *ctx, double *dst, const double *src, int64_t n, cudaStream_t s, bool side)
+{
+    if (side) {
+        if (!ctx->copy_stream)
+            CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
+        if (!ctx->copy_ev)
+            CU(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming), "cudaEventCreate");
+        if (!ctx->copy_done)
+            CU(cudaEventCreateWithFlags(&ctx->copy_done, cudaEventDisableTiming), "cudaEventCreate");
+        CU(cudaEventRecord(ctx->copy_ev, s), "cudaEventRecord");
+        CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev, 0), "cudaStreamWaitEvent");
+    }
+    CU(cudaMemcpyAsync(dst, src, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, side ? ctx->copy_stream : s),
+       "cudaMemcpyAsync(loglik)");
+    return CVB_OK;
+}
+
 static int eval_batch(cvb_ctx *ctx, int64_t n_points, const double *params, int clip, double *out_p,
                       double *out_ll, int k_best, double *out_rows, void *stream)
 {
@@ -563,13 +571,13 @@ static int eval_batch(cvb_ctx *ctx, int64_t n_points, const double *params, int 
     if (chunk > n_points)
         chunk = n_points;
     if (!p_dev)
-        CU(grow(&ctx->d_params, &ctx->cap_params, (size_t)chunk * np), "cudaMalloc(params staging)");
+        CU(cv_grow(&ctx->d_params, &ctx->cap_params, (size_t)chunk * np), "cudaMalloc(params staging)");
     if (!l_dev || !out_ll)
-        CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)chunk), "cudaMalloc(loglik staging)");
+        CU(cv_grow(&ctx->d_ll, &ctx->cap_ll, (size_t)chunk), "cudaMalloc(loglik staging)");
     const double *dp_all = p_dev ? params : ctx->d_params;
     const double *dl_all = (out_ll && l_dev) ? out_ll : ctx->d_ll;
     if (out_p && !q_dev)
-        CU(grow(&ctx->d_probs, &ctx->cap_probs, (size_t)chunk * nb), "cudaMalloc(probs staging)");
+        CU(cv_grow(&ctx->d_probs, &ctx->cap_probs, (size_t)chunk * nb), "cudaMalloc(probs staging)");
     if (ctx->poison) {
         if (int rc = poison_fill(ctx, dl_all == ctx->d_ll ? ctx->d_ll : nullptr, (size_t)chunk, s))
             return rc;
@@ -596,23 +604,12 @@ static int eval_batch(cvb_ctx *ctx, int64_t n_points, const double *params, int 
             return rc;
         if (out_ll && !l_dev) {
             /* with a top-K to follow the values leave on a stream of their own, next to it */
-            cudaStream_t cs = s;
-            if (k_best > 0 && n >= (1 << 16)) {
-                if (!ctx->copy_stream)
-                    CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-                if (!ctx->copy_ev)
-                    CU(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming), "cudaEventCreate");
-                if (!ctx->copy_done)
-                    CU(cudaEventCreateWithFlags(&ctx->copy_done, cudaEventDisableTiming), "cudaEventCreate");
-                CU(cudaEventRecord(ctx->copy_ev, s), "cudaEventRecord");
-                CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev, 0), "cudaStreamWaitEvent");
-                cs = ctx->copy_stream;
-                side_copy = true;
-            }
-            CU(cudaMemcpyAsync(out_ll + off, dl, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, cs),
-               "cudaMemcpyAsync(loglik)");
-            if (cs != s)
-                CU(cudaEventRecord(ctx->copy_done, cs), "cudaEventRecord");
+            const bool side = k_best > 0 && n >= (1 << 16);
+            if (int rc = copy_values_out(ctx, out_ll + off, dl, n, s, side))
+                return rc;
+            if (side)
+                CU(cudaEventRecord(ctx->copy_done, ctx->copy_stream), "cudaEventRecord");
+            side_copy = side_copy || side;
         }
         if (out_p && !q_dev)
             CU(cudaMemcpyAsync(out_p + off * nb, dq, (size_t)n * nb * sizeof(double),
@@ -702,13 +699,13 @@ static int topk_device(cvb_ctx *ctx, const CvLattice &lat, const double *d_ll, c
     }
     if (n >= CVB_TOPK_RADIX_MIN && cv_topk_select_fits(n, K)) {
         /* large batch, few rows wanted: radix selection (topk.cu) */
-        CU(grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, cv_topk_select_bytes()), "cudaMalloc(topk scratch)");
+        CU(cv_grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, cv_topk_select_bytes()), "cudaMalloc(topk scratch)");
         CU(cv_launch_topk_radix_select(d_ll, n, K, ctx->d_topk_scratch, ctx->n_sm, ctx->d_sel_ll, ctx->d_sel_idx, s),
            "top-K selection");
         ctx->last_launches += 1;
     } else if (n >= CVB_TOPK_RADIX_MIN && n <= 0x7fffffffLL) { /* large batch: one radix sort (topk.cu) */
         const size_t need = cv_topk_sort_bytes(n);
-        CU(grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, need), "cudaMalloc(topk scratch)");
+        CU(cv_grow(&ctx->d_topk_scratch, &ctx->cap_topk_scratch, need), "cudaMalloc(topk scratch)");
         CU(cv_launch_topk_sort(d_ll, n, K, ctx->d_topk_scratch, ctx->cap_topk_scratch, ctx->d_sel_ll,
                                ctx->d_sel_idx, s),
            "top-K sort");
@@ -751,7 +748,7 @@ extern "C" int cvb_topk(cvb_ctx *ctx, int64_t n_points, const double *ll, const 
         return rc;
     const double *dl = ll, *dp = params;
     if (n_points > 0 && !is_device_ptr(ll)) {
-        CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)n_points), "cudaMalloc(loglik staging)");
+        CU(cv_grow(&ctx->d_ll, &ctx->cap_ll, (size_t)n_points), "cudaMalloc(loglik staging)");
         if (ctx->poison)
             if (int rc = poison_fill(ctx, ctx->d_ll, (size_t)n_points, s))
                 return rc;
@@ -760,7 +757,7 @@ extern "C" int cvb_topk(cvb_ctx *ctx, int64_t n_points, const double *ll, const 
         dl = ctx->d_ll;
     }
     if (n_points > 0 && !is_device_ptr(params)) {
-        CU(grow(&ctx->d_params, &ctx->cap_params, (size_t)n_points * np), "cudaMalloc(params staging)");
+        CU(cv_grow(&ctx->d_params, &ctx->cap_params, (size_t)n_points * np), "cudaMalloc(params staging)");
         CU(cudaMemcpyAsync(ctx->d_params, params, (size_t)n_points * np * sizeof(double),
                            cudaMemcpyHostToDevice, s),
            "cudaMemcpyAsync(params)");
@@ -806,7 +803,7 @@ static int lattice_setup(cvb_ctx *ctx, const int32_t *axis_len, const double *ax
         if (((double)first + (double)last_run * (double)stride) * (double)block + (double)last_in >= total_pts)
             return fail(ctx, CVB_EINVAL, "lattice slice runs past the end of the lattice");
     }
-    CU(grow(&ctx->d_axes, &ctx->cap_axes, total_vals), "cudaMalloc(axes)");
+    CU(cv_grow(&ctx->d_axes, &ctx->cap_axes, total_vals), "cudaMalloc(axes)");
     CU(cudaMemcpyAsync(ctx->d_axes, axis_values, total_vals * sizeof(double), cudaMemcpyHostToDevice, s),
        "cudaMemcpyAsync(axes)");
     memset(&lat, 0, sizeof(lat));
@@ -837,7 +834,7 @@ static int lattice_values(cvb_ctx *ctx, double *out_dev, int64_t count, cudaStre
 {
     *dl = out_dev;
     if (!*dl) {
-        CU(grow(&ctx->d_ll, &ctx->cap_ll, (size_t)(count > 0 ? count : 1)), "cudaMalloc(loglik staging)");
+        CU(cv_grow(&ctx->d_ll, &ctx->cap_ll, (size_t)(count > 0 ? count : 1)), "cudaMalloc(loglik staging)");
         *dl = ctx->d_ll;
     }
     if (ctx->poison) {
@@ -870,13 +867,14 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
     double *dl = nullptr;
     if (int rc = lattice_values(ctx, l_dev ? out_ll : nullptr, count, s, &dl))
         return rc;
-    bool need_sync = false, side_copy = false;
     /* A long slice whose values go to host memory is evaluated in parts of whole runs (and whole
      * (coverage, error_rate) groups), so that the values of a part travel while the next part is
      * evaluated: at 8 bytes per point the copy is otherwise up to a third of the call (cfg5: 100 MB per
      * rank; and the ranks of a box finish together and share the way to host memory). */
-    int64_t part = 0;
-    if (out_ll && !l_dev && count >= CVB_LATTICE_PART_MIN) {
+    const bool to_host = out_ll && !l_dev;
+    int64_t part = count; /* a slice that is not split is one part */
+    bool split = false;
+    if (to_host && count >= CVB_LATTICE_PART_MIN) {
         int64_t unit = block;
         if (block == 1 && stride == 1 && np == 5)
             unit = (int64_t)axis_len[2] * axis_len[3] * axis_len[4];
@@ -884,57 +882,25 @@ extern "C" int cvb_lattice_eval(cvb_ctx *ctx, const int32_t *axis_len, const dou
         int64_t n_parts = count >> 21;
         n_parts = n_parts < 2 ? 2 : n_parts > 8 ? 8 : n_parts;
         const int64_t want = (count + n_parts - 1) / n_parts;
-        if (unit >= 1 && unit <= want && (block > 1 || first % unit == 0))
+        split = unit >= 1 && unit <= want && (block > 1 || first % unit == 0);
+        if (split)
             part = (want + unit - 1) / unit * unit;
     }
-    if (part > 0) {
-        if (!ctx->copy_stream)
-            CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-        if (!ctx->copy_ev)
-            CU(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming), "cudaEventCreate");
-        if (!ctx->copy_done)
-            CU(cudaEventCreateWithFlags(&ctx->copy_done, cudaEventDisableTiming), "cudaEventCreate");
-        for (int64_t off = 0; off < count; off += part) {
-            const int64_t n_part = count - off < part ? count - off : part;
-            CvLattice lp = lat;
-            lp.first = first + (off / block) * stride;
-            int rc = launch_loglik(ctx, lp, axes_host, nullptr, n_part, 1, dl + off, nullptr, s);
-            if (rc != CVB_OK)
-                return rc;
-            CU(cudaEventRecord(ctx->copy_ev, s), "cudaEventRecord");
-            CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev, 0), "cudaStreamWaitEvent");
-            CU(cudaMemcpyAsync(out_ll + off, dl + off, (size_t)n_part * sizeof(double), cudaMemcpyDeviceToHost,
-                               ctx->copy_stream),
-               "cudaMemcpyAsync(loglik)");
-        }
-        CU(cudaEventRecord(ctx->copy_done, ctx->copy_stream), "cudaEventRecord");
-        side_copy = true;
-        need_sync = true;
-    } else if (count > 0) {
-        int rc = launch_loglik(ctx, lat, axes_host, nullptr, count, 1, dl, nullptr, s);
-        if (rc != CVB_OK)
+    /* the values of the parts, or of a whole slice with a top-K to follow, leave on the copy stream */
+    const bool side_copy = to_host && (split || (k_best > 0 && count >= (1 << 16)));
+    for (int64_t off = 0; off < count; off += part) {
+        const int64_t n_part = count - off < part ? count - off : part;
+        CvLattice lp = lat;
+        lp.first = first + (off / block) * stride;
+        if (int rc = launch_loglik(ctx, lp, axes_host, nullptr, n_part, 1, dl + off, nullptr, s))
             return rc;
+        if (to_host)
+            if (int rc = copy_values_out(ctx, out_ll + off, dl + off, n_part, s, side_copy))
+                return rc;
     }
-    if (out_ll && !l_dev && count > 0 && part == 0) {
-        cudaStream_t cs = s;
-        if (k_best > 0 && count >= (1 << 16)) { /* the values leave next to the top-K, on a stream of their own */
-            if (!ctx->copy_stream)
-                CU(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking), "cudaStreamCreate");
-            if (!ctx->copy_ev)
-                CU(cudaEventCreateWithFlags(&ctx->copy_ev, cudaEventDisableTiming), "cudaEventCreate");
-            if (!ctx->copy_done)
-                CU(cudaEventCreateWithFlags(&ctx->copy_done, cudaEventDisableTiming), "cudaEventCreate");
-            CU(cudaEventRecord(ctx->copy_ev, s), "cudaEventRecord");
-            CU(cudaStreamWaitEvent(ctx->copy_stream, ctx->copy_ev, 0), "cudaStreamWaitEvent");
-            cs = ctx->copy_stream;
-            side_copy = true;
-        }
-        CU(cudaMemcpyAsync(out_ll, dl, (size_t)count * sizeof(double), cudaMemcpyDeviceToHost, cs),
-           "cudaMemcpyAsync(loglik)");
-        if (side_copy)
-            CU(cudaEventRecord(ctx->copy_done, cs), "cudaEventRecord");
-        need_sync = true;
-    }
+    if (side_copy)
+        CU(cudaEventRecord(ctx->copy_done, ctx->copy_stream), "cudaEventRecord");
+    bool need_sync = to_host && count > 0;
     if (k_best > 0) {
         int rc = topk_device(ctx, lat, dl, nullptr, count, k_best, out_rows, s);
         if (rc != CVB_OK)
@@ -984,12 +950,12 @@ extern "C" int cvb_lattice_profile(cvb_ctx *ctx, const int32_t *axis_len, const 
     if (count > 0)
         if (int rc = launch_loglik(ctx, lat, axes_host, nullptr, count, 1, dl, nullptr, s))
             return rc;
-    CU(grow(&ctx->d_seg_key, &ctx->cap_seg_key, (size_t)n_seg), "cudaMalloc(segment keys)");
-    CU(grow(&ctx->d_seg_best, &ctx->cap_seg_best, (size_t)n_seg), "cudaMalloc(segment indices)");
+    CU(cv_grow(&ctx->d_seg_key, &ctx->cap_seg_key, (size_t)n_seg), "cudaMalloc(segment keys)");
+    CU(cv_grow(&ctx->d_seg_best, &ctx->cap_seg_best, (size_t)n_seg), "cudaMalloc(segment indices)");
     const bool r_dev = is_device_ptr(out_rows);
     double *dr = out_rows;
     if (!r_dev) {
-        CU(grow(&ctx->d_seg_rows, &ctx->cap_seg_rows, (size_t)n_seg * (1 + np)), "cudaMalloc(segment rows)");
+        CU(cv_grow(&ctx->d_seg_rows, &ctx->cap_seg_rows, (size_t)n_seg * (1 + np)), "cudaMalloc(segment rows)");
         dr = ctx->d_seg_rows;
         if (ctx->poison)
             if (int rc = poison_fill(ctx, dr, (size_t)n_seg * (1 + np), s))
@@ -1382,7 +1348,7 @@ extern "C" int cvb_kmer_histogram(cvb_kmer_table *t, int64_t n_bins, int64_t *ou
     const bool dev = is_device_ptr(out_hist);
     long long *dh = (long long *)out_hist;
     if (!dev) {
-        KU(grow(&t->d_hist, &t->cap_hist, (size_t)n_bins), "cudaMalloc(histogram)");
+        KU(cv_grow(&t->d_hist, &t->cap_hist, (size_t)n_bins), "cudaMalloc(histogram)");
         dh = t->d_hist;
     }
     KU(cudaMemsetAsync(dh, 0, (size_t)n_bins * sizeof(long long), s), "cudaMemsetAsync(histogram)");

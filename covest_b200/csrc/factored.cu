@@ -32,6 +32,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <type_traits>
 #include <vector>
 
 #include "kdevice.h"
@@ -1685,8 +1686,8 @@ void cvf_release(CvFactorWork &wk)
         cudaFree(wk.plan);
     if (wk.W)
         cudaFree(wk.W);
-    if (wk.h_header)
-        cudaFreeHost(wk.h_header);
+    if (wk.h_sizes)
+        cudaFreeHost(wk.h_sizes);
     if (wk.d_counters)
         cudaFree(wk.d_counters);
     if (wk.d_scratch)
@@ -1706,7 +1707,7 @@ void cvf_release(CvFactorWork &wk)
         }
     wk.plan = nullptr;
     wk.W = nullptr;
-    wk.h_header = nullptr;
+    wk.h_sizes = nullptr;
     wk.d_counters = nullptr;
     wk.plan_cap = wk.w_cap = 0;
 }
@@ -1719,6 +1720,7 @@ static size_t cvf_align(size_t x) { return (x + 255) & ~(size_t)255; }
         if (e_ != cudaSuccess)    \
             return e_;            \
     } while (0)
+
 
 /* ---- the template of a lattice's groups, on the host ---- */
 static double cvf_host_clip(const CvModelDesc &m, double v, int clip, int a)
@@ -1825,441 +1827,419 @@ static bool cvf_lattice_aligned(const CvModelDesc &m, const CvLattice &lat, long
     return lat.block == 1 && lat.stride == 1 && lat.first % M == 0;
 }
 
-cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *const *lat_axes_host,
-                     const double *params, long long n,
-                     int clip, double *out_ll, const CvfSlots &sl,
-                     const double *log_tab, CvFactorWork &wk, int n_sm, int smem_max, size_t w_limit,
-                     double min_group, double min_run, int kernel_mode, cudaStream_t stream,
-                     int *used)
-{
-    *used = 0;
-    wk.launches = 0;
-    if (n <= 0 || n > 0x7fffffffLL || !cvf_supported(m))
-        return cudaSuccess;
-    /* the slots of a profile row as the batch kernels see them (cvf_build_slots) */
-    const int nsteps = sl.nsteps;
-    const int slots_padded = nsteps * CVF_NS;
-    const double2 *slot_mh = sl.slot_mh;
-    const int *step_mask = sl.step_mask;
+/* The automatic policy (CvfRequest): points per (c, e) group on average below which the per-point
+ * kernel runs, points per q-run below which the GEMM runs instead of the prefix kernel */
+static constexpr double CVF_MIN_GROUP = 12.0;
+static constexpr double CVF_MIN_RUN = 4.0;
+static constexpr int CVF_PLAN_TB = 256; /* threads per CTA of the plan kernels */
 
-    /* ---- carve the plan ---- */
+/* bytes of the prefix kernel's scratch: per CTA the partials of a batch, at most 32 warps per SM */
+static size_t cvf_scratch_bytes(int n_sm) { return (size_t)n_sm * 32 * 3 * CVF_PB * sizeof(double); }
+
+/* the inputs of one evaluation, as cvf_eval receives them */
+struct CvfCall {
+    const CvModelDesc &m;
+    const CvLattice &lat;
+    const double *params;
+    long long n;
+    int clip;
+    double *out_ll;
+    const CvfSlots &sl;
+    const double *log_tab;
+    int n_sm, smem_max;
+    cudaStream_t stream;
+};
+
+/* the plan of one evaluation as the host holds it */
+struct CvfHostPlan {
+    CvfPlan pl;       /* the tables on the device */
+    unsigned char *tmp; /* cub scratch */
+    size_t tmp_bytes;
+    CvfSizes size;
+    bool analytic;    /* made from the lattice axes (cvf_plan_lattice) */
+    CvfLatticeDev TD; /* analytic: the template on the device */
+};
+
+/* The plan buffers of a batch of n points, carved in this order out of one allocation at `base`
+ * (nullptr: only counted).  Returns the bytes they take. */
+static size_t cvf_plan_layout(unsigned char *base, long long n, size_t tmp_bytes, CvfPlan &pl, unsigned char *&tmp)
+{
+    const size_t n1 = (size_t)n + 1;
+    size_t off = 0;
+    auto take = [&](auto *&field, size_t count) {
+        typedef std::remove_reference_t<decltype(*field)> T;
+        field = base ? (T *)(base + off) : nullptr;
+        off += cvf_align(count * sizeof(T));
+    };
+    take(pl.keys, n); take(pl.keys_alt, n); take(pl.idx, n); take(pl.idx_alt, n);
+    take(pl.othr, n); take(pl.head, n); take(pl.gid, n); take(pl.head2, n); take(pl.rid, n);
+    take(pl.g_omax, n1); take(pl.r_start, n1); take(pl.g_rfirst, n1); take(pl.flags2, n);
+    take(pl.g_start, n1); take(pl.tile_start, n1); take(pl.item_start, n1); take(pl.w_off, n1); take(pl.a_start, n1);
+    for (int **t : {&pl.t_first, &pl.t_cnt, &pl.t_nkc, &pl.t_aoff, &pl.t_group, &pl.t_key, &pl.t_key_alt,
+                    &pl.t_order, &pl.t_order_alt})
+        take(*t, n1);
+    take(pl.header, sizeof(CvfSizes) / sizeof(long long));
+    take(tmp, tmp_bytes);
+    return off;
+}
+
+/* the plan in wk.plan, and the other buffers of an evaluation on first use */
+static cudaError_t cvf_plan_alloc(const CvfCall &c, CvFactorWork &wk, CvfHostPlan &P)
+{
+    const int n = (int)c.n;
     size_t sort_tmp = 0, sort_tmp_t = 0, scan_tmp_i = 0, scan_tmp_l = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (unsigned long long *)nullptr,
                                     (unsigned long long *)nullptr, (unsigned int *)nullptr,
-                                    (unsigned int *)nullptr, (int)n, 0, 64, stream);
+                                    (unsigned int *)nullptr, n, 0, 64, c.stream);
     cub::DeviceRadixSort::SortPairsDescending(nullptr, sort_tmp_t, (int *)nullptr, (int *)nullptr,
-                                              (int *)nullptr, (int *)nullptr, (int)n, 0, 32, stream);
+                                              (int *)nullptr, (int *)nullptr, n, 0, 32, c.stream);
     cub::DeviceScan::InclusiveSum(nullptr, scan_tmp_i, (unsigned long long *)nullptr, (unsigned long long *)nullptr,
-                                  (int)n + 1, stream);
-    cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp_l, (long long *)nullptr, (long long *)nullptr,
-                                  (int)n + 1, stream);
-    const size_t tmp_bytes = std::max(std::max(sort_tmp, sort_tmp_t), std::max(scan_tmp_i, scan_tmp_l)) + 256;
-    const size_t n1 = (size_t)n + 1;
-    size_t off = 0;
-    auto take = [&](size_t bytes) {
-        size_t at = off;
-        off += cvf_align(bytes);
-        return at;
-    };
-    const size_t o_keys = take(n * 8), o_keys_alt = take(n * 8), o_idx = take(n * 4), o_idx_alt = take(n * 4);
-    const size_t o_othr = take(n * 4), o_head = take(n * 4), o_gid = take(n * 4);
-    const size_t o_head2 = take(n * 4), o_rid = take(n * 4), o_gomax = take(n1 * 4);
-    const size_t o_rstart = take(n1 * 4), o_grfirst = take(n1 * 4), o_flags2 = take(n * 8);
-    const size_t o_gstart = take(n1 * 4), o_tile = take(n1 * 4), o_item = take(n1 * 4), o_woff = take(n1 * 8);
-    const size_t o_astart = take(n1 * 4);
-    size_t o_t[9];
-    for (size_t &o : o_t)
-        o = take(n1 * 4);
-    const size_t o_header = take(64), o_tmp = take(tmp_bytes);
-    if (off > wk.plan_cap) {
-        if (wk.plan)
-            cudaFree(wk.plan);
-        wk.plan = nullptr;
-        wk.plan_cap = 0;
-        CVF_CK(cudaMalloc(&wk.plan, off));
-        wk.plan_cap = off;
-    }
-    if (!wk.h_header)
-        CVF_CK(cudaMallocHost((void **)&wk.h_header, 64));
+                                  n + 1, c.stream);
+    cub::DeviceScan::ExclusiveSum(nullptr, scan_tmp_l, (long long *)nullptr, (long long *)nullptr, n + 1, c.stream);
+    P.tmp_bytes = std::max(std::max(sort_tmp, sort_tmp_t), std::max(scan_tmp_i, scan_tmp_l)) + 256;
+    CVF_CK(cv_grow(&wk.plan, &wk.plan_cap, cvf_plan_layout(nullptr, c.n, P.tmp_bytes, P.pl, P.tmp)));
+    if (!wk.h_sizes)
+        CVF_CK(cudaMallocHost((void **)&wk.h_sizes, sizeof(CvfSizes)));
     if (!wk.d_counters)
         CVF_CK(cudaMalloc((void **)&wk.d_counters, 2 * sizeof(unsigned long long)));
-    /* the CTAs of the prefix kernel own a scratch of partials each: at most 32 warps per SM */
     if (!wk.d_scratch)
-        CVF_CK(cudaMalloc((void **)&wk.d_scratch, (size_t)n_sm * 32 * 3 * CVF_PB * sizeof(double)));
+        CVF_CK(cudaMalloc((void **)&wk.d_scratch, cvf_scratch_bytes(c.n_sm)));
     if (wk.timed && !wk.ev[0])
         for (cudaEvent_t &e : wk.ev)
             CVF_CK(cudaEventCreate(&e));
-    unsigned char *base = (unsigned char *)wk.plan;
-    CvfPlan pl;
-    pl.keys = (unsigned long long *)(base + o_keys);
-    pl.keys_alt = (unsigned long long *)(base + o_keys_alt);
-    pl.idx = (unsigned int *)(base + o_idx);
-    pl.idx_alt = (unsigned int *)(base + o_idx_alt);
-    pl.idx_sorted = nullptr;
-    pl.othr = (int *)(base + o_othr);
-    pl.head = (int *)(base + o_head);
-    pl.gid = (int *)(base + o_gid);
-    pl.head2 = (int *)(base + o_head2);
-    pl.rid = (int *)(base + o_rid);
-    pl.g_omax = (int *)(base + o_gomax);
-    pl.flags2 = (unsigned long long *)(base + o_flags2);
-    pl.r_start = (int *)(base + o_rstart);
-    pl.g_rfirst = (int *)(base + o_grfirst);
-    pl.g_start = (int *)(base + o_gstart);
-    pl.tile_start = (int *)(base + o_tile);
-    pl.item_start = (int *)(base + o_item);
-    pl.w_off = (long long *)(base + o_woff);
-    pl.a_start = (int *)(base + o_astart);
-    pl.t_first = (int *)(base + o_t[0]);
-    pl.t_cnt = (int *)(base + o_t[1]);
-    pl.t_nkc = (int *)(base + o_t[2]);
-    pl.t_aoff = (int *)(base + o_t[3]);
-    pl.t_group = (int *)(base + o_t[4]);
-    pl.t_key = (int *)(base + o_t[5]);
-    pl.t_key_alt = (int *)(base + o_t[6]);
-    pl.t_order = (int *)(base + o_t[7]);
-    pl.t_order_alt = (int *)(base + o_t[8]);
-    pl.t_sorted = nullptr;
-    pl.header = (long long *)(base + o_header);
-    pl.obits = 1;
-    while ((1 << pl.obits) <= m.max_bin + CV_COPY_PAD)
-        pl.obits++;
-    void *tmp = base + o_tmp;
+    cvf_plan_layout(wk.plan, c.n, P.tmp_bytes, P.pl, P.tmp);
+    P.pl.obits = 1;
+    while ((1 << P.pl.obits) <= c.m.max_bin + CV_COPY_PAD)
+        P.pl.obits++;
+    return cudaSuccess;
+}
 
-    const int tb = 256;
-    const unsigned int nb = (unsigned int)((n + tb - 1) / tb), nb1 = (unsigned int)((n + 1 + tb - 1) / tb);
-    if (wk.timed)
-        CVF_CK(cudaEventRecord(wk.ev[0], stream));
-
-    /* K0 .. totals for one ordering of the points; ends with the header on the host */
-    auto build_plan = [&](int prefix) -> cudaError_t {
-        pl.prefix = prefix;
-        pl.tile_points = CVF_M;
-        pl.keys = (unsigned long long *)(base + o_keys);
-        pl.keys_alt = (unsigned long long *)(base + o_keys_alt);
-        pl.idx = (unsigned int *)(base + o_idx);
-        pl.idx_alt = (unsigned int *)(base + o_idx_alt);
-        cvf_point_keys<<<nb, tb, 0, stream>>>(m, lat, params, n, clip, pl);
-        CVF_CK(cudaGetLastError());
-        {
-            cub::DoubleBuffer<unsigned long long> dk(pl.keys, pl.keys_alt);
-            cub::DoubleBuffer<unsigned int> dv(pl.idx, pl.idx_alt);
-            size_t tb_ = tmp_bytes;
-            CVF_CK(cub::DeviceRadixSort::SortPairs(tmp, tb_, dk, dv, (int)n, 0, 64, stream));
-            pl.idx_sorted = dv.Current();
-        }
-        cvf_heads<<<nb, tb, 0, stream>>>(m, lat, params, n, clip, pl);
-        CVF_CK(cudaGetLastError());
-        {
-            size_t tb_ = tmp_bytes;
-            CVF_CK(cub::DeviceScan::InclusiveSum(tmp, tb_, pl.flags2, pl.flags2, (int)n, stream));
-        }
-        CVF_CK(cudaMemsetAsync(pl.g_omax, 0, n1 * sizeof(int), stream));
-        cvf_group_starts<<<nb, tb, 0, stream>>>(n, pl);
-        CVF_CK(cudaGetLastError());
-        cvf_group_counts<<<nb1, tb, 0, stream>>>(n, slots_padded, pl);
-        CVF_CK(cudaGetLastError());
-        cvf_group_scan<<<1, 1024, 0, stream>>>(pl);
-        CVF_CK(cudaGetLastError());
-        CVF_CK(cudaMemcpyAsync(wk.h_header, pl.header, 6 * sizeof(long long), cudaMemcpyDeviceToHost, stream));
-        CVF_CK(cudaStreamSynchronize(stream));
-        wk.launches += 17; /* K0, radix sort (10), heads, one scan (2), starts, counts, group scan */
+/* The template of the lattice's groups in T, made and uploaded when the (q1, q2, q) axes or the
+ * clipping differ from those of the last upload */
+static cudaError_t cvf_lattice_upload(const CvfCall &c, const double *const *axes, CvfLatticeCache &T)
+{
+    const int n1 = c.lat.len[2], n2 = c.lat.len[3], nq = c.lat.len[4];
+    std::vector<double> key = {(double)c.clip, (double)n1, (double)n2, (double)nq};
+    key.insert(key.end(), axes[2], axes[2] + n1);
+    key.insert(key.end(), axes[3], axes[3] + n2);
+    key.insert(key.end(), axes[4], axes[4] + nq);
+    if (key.size() == T.key.size() && T.dev && memcmp(key.data(), T.key.data(), key.size() * sizeof(double)) == 0)
         return cudaSuccess;
-    };
-    /* ---- a lattice handed over as axes: the plan follows from the axes (no sort, no sync) ---- */
-    int prefix = kernel_mode != 1;
-    long long latM = 0;
-    bool analytic = false;
-    CvfLatticeDev TD;
-    memset(&TD, 0, sizeof(TD));
-    long long n_groups = 0, n_tiles = 0, n_items = 0, w_total = 0, a_total = 0;
-    if (prefix && lat_axes_host && cvf_lattice_aligned(m, lat, n, &latM) && (double)latM >= min_group &&
-        (double)(lat.len[2] * (long long)lat.len[3]) >= (kernel_mode == 0 ? min_run : 1.0)) {
-        CvfLatticeCache &T = wk.lattice;
-        const int n1 = lat.len[2], n2 = lat.len[3], nq = lat.len[4];
-        std::vector<double> key;
-        key.reserve(4 + n1 + n2 + nq);
-        key.push_back((double)clip);
-        key.push_back((double)n1);
-        key.push_back((double)n2);
-        key.push_back((double)nq);
-        key.insert(key.end(), lat_axes_host[2], lat_axes_host[2] + n1);
-        key.insert(key.end(), lat_axes_host[3], lat_axes_host[3] + n2);
-        key.insert(key.end(), lat_axes_host[4], lat_axes_host[4] + nq);
-        const bool same = key.size() == T.key.size() && T.dev &&
-                          memcmp(key.data(), T.key.data(), key.size() * sizeof(double)) == 0;
-        if (!same) {
-            cvf_lattice_template(m, clip, lat_axes_host[2], n1, lat_axes_host[3], n2, lat_axes_host[4], nq, T);
-            const size_t ints = T.host.size();
-            if (ints > T.dev_cap) {
-                if (T.dev)
-                    cudaFree(T.dev);
-                T.dev = nullptr;
-                T.dev_cap = 0;
-                CVF_CK(cudaMalloc((void **)&T.dev, ints * sizeof(int)));
-                T.dev_cap = ints;
-            }
-            if (!T.uploaded)
-                CVF_CK(cudaEventCreateWithFlags(&T.uploaded, cudaEventDisableTiming));
-            else
-                CVF_CK(cudaEventSynchronize(T.uploaded)); /* the staging buffer is free again */
-            if (ints > T.pinned_cap) {
-                if (T.pinned)
-                    cudaFreeHost(T.pinned);
-                T.pinned = nullptr;
-                T.pinned_cap = 0;
-                CVF_CK(cudaMallocHost((void **)&T.pinned, ints * sizeof(int)));
-                T.pinned_cap = ints;
-            }
-            memcpy(T.pinned, T.host.data(), ints * sizeof(int));
-            T.key.clear(); /* not valid until the copy is enqueued */
-            CVF_CK(cudaMemcpyAsync(T.dev, T.pinned, ints * sizeof(int), cudaMemcpyHostToDevice, stream));
-            CVF_CK(cudaEventRecord(T.uploaded, stream));
-            T.key = key;
-        }
-        const int M = T.M, nT = T.nT;
-        const int G = (int)(n / M);
-        const int items = (T.omax + CVF_KC - 1) / CVF_KC;
-        const long long wpg = (long long)items * CVF_KC * slots_padded;
-        TD.perm = T.dev;
-        TD.othr = T.dev + M;
-        TD.tt_first = T.dev + 2 * (size_t)M;
-        TD.tt_cnt = TD.tt_first + nT;
-        TD.tt_kmax = TD.tt_cnt + nT;
-        TD.tt_order = TD.tt_kmax + nT;
-        pl.prefix = 1;
-        pl.tile_points = CVF_M;
-        pl.idx_sorted = pl.idx;
-        const long long work = std::max<long long>(n, (long long)G * T.nq + 1);
-        cvf_lattice_fill<<<(unsigned int)((work + tb - 1) / tb), tb, 0, stream>>>(pl, TD, G, M, T.R, T.nq, nT, T.omax,
-                                                                                items, wpg);
-        CVF_CK(cudaGetLastError());
-        wk.launches += 1;
-        analytic = true;
-        n_groups = G;
-        n_tiles = (long long)G * nT;
-        n_items = (long long)G * items;
-        w_total = (long long)G * wpg;
-        a_total = 0;
-        wk.n_groups = G;
-        wk.n_runs = (long long)G * T.nq;
-    }
-    wk.analytic = analytic ? 1 : 0;
-    if (!analytic) {
-        /* ordering for the prefix kernel first: it also tells how many q-runs the batch has */
-        CVF_CK(build_plan(prefix));
-        wk.n_groups = wk.h_header[0];
-        wk.n_runs = wk.h_header[5];
-        if (wk.n_groups <= 0 || (double)n < min_group * (double)wk.n_groups)
-            return cudaSuccess; /* too little sharing: the per-point kernel is the better tool */
-        if (prefix && kernel_mode == 0 && (double)n < min_run * (double)wk.n_runs) {
-            prefix = 0; /* few points per q-run: the GEMM shares the profiles between all points of a group */
-            CVF_CK(build_plan(0));
-        }
-        n_groups = wk.h_header[0];
-        n_tiles = wk.h_header[1];
-        n_items = wk.h_header[2];
-        w_total = wk.h_header[3];
-        a_total = wk.h_header[4];
-        cvf_tile_table<<<(unsigned int)((n_groups + 127) / 128), 128, 0, stream>>>((int)n_groups, pl);
-        CVF_CK(cudaGetLastError());
-        wk.launches++;
-    }
-    wk.n_tiles = n_tiles;
-    wk.n_items = n_items;
-    wk.w_doubles = w_total;
-    wk.prefix = prefix;
+    cvf_lattice_template(c.m, c.clip, axes[2], n1, axes[3], n2, axes[4], nq, T);
+    const size_t ints = T.host.size();
+    CVF_CK(cv_grow(&T.dev, &T.dev_cap, ints));
+    if (!T.uploaded)
+        CVF_CK(cudaEventCreateWithFlags(&T.uploaded, cudaEventDisableTiming));
+    else
+        CVF_CK(cudaEventSynchronize(T.uploaded)); /* the staging buffer is free again */
+    CVF_CK(cv_grow(&T.pinned, &T.pinned_cap, ints, true));
+    memcpy(T.pinned, T.host.data(), ints * sizeof(int));
+    T.key.clear(); /* not valid until the copy is enqueued */
+    CVF_CK(cudaMemcpyAsync(T.dev, T.pinned, ints * sizeof(int), cudaMemcpyHostToDevice, c.stream));
+    CVF_CK(cudaEventRecord(T.uploaded, c.stream));
+    T.key = key;
+    return cudaSuccess;
+}
 
-    /* ---- group ranges whose profiles fit the workspace ---- */
-    std::vector<int> cut; /* group boundaries */
-    cut.push_back(0);
-    std::vector<int> h_tile, h_item, h_achunk;
-    std::vector<long long> h_woff;
-    if ((size_t)w_total > w_limit) {
-        h_tile.resize(n_groups + 1);
-        h_item.resize(n_groups + 1);
-        h_achunk.resize(n_groups + 1);
-        h_woff.resize(n_groups + 1);
-        if (analytic) { /* every group has the same tiles, items and profile size */
-            for (long long g = 0; g <= n_groups; g++) {
-                h_tile[g] = (int)(g * (n_tiles / n_groups));
-                h_item[g] = (int)(g * (n_items / n_groups));
-                h_achunk[g] = 0;
-                h_woff[g] = g * (w_total / n_groups);
-            }
-        } else {
-        CVF_CK(cudaMemcpyAsync(h_tile.data(), pl.tile_start, (n_groups + 1) * 4, cudaMemcpyDeviceToHost, stream));
-        CVF_CK(cudaMemcpyAsync(h_item.data(), pl.item_start, (n_groups + 1) * 4, cudaMemcpyDeviceToHost, stream));
-        CVF_CK(cudaMemcpyAsync(h_achunk.data(), pl.a_start, (n_groups + 1) * 4, cudaMemcpyDeviceToHost, stream));
-        CVF_CK(cudaMemcpyAsync(h_woff.data(), pl.w_off, (n_groups + 1) * 8, cudaMemcpyDeviceToHost, stream));
-        CVF_CK(cudaStreamSynchronize(stream));
-        }
-        int g0 = 0;
-        while (g0 < n_groups) {
-            int g1 = g0 + 1;
-            while (g1 < n_groups && (size_t)(h_woff[g1 + 1] - h_woff[g0]) <= w_limit)
-                g1++;
-            cut.push_back(g1);
-            g0 = g1;
+/* A lattice handed over as axes: the plan follows from the axes (no sort, no sync).  One launch
+ * writes the tables of all groups from the template; the sizes are counted here. */
+static cudaError_t cvf_plan_lattice(const CvfCall &c, const double *const *axes, CvFactorWork &wk, CvfHostPlan &P)
+{
+    const CvfLatticeCache &T = wk.lattice;
+    CVF_CK(cvf_lattice_upload(c, axes, wk.lattice));
+    const int M = T.M, nT = T.nT;
+    const int G = (int)(c.n / M);
+    const int items = (T.omax + CVF_KC - 1) / CVF_KC;
+    const long long wpg = (long long)items * CVF_KC * c.sl.nsteps * CVF_NS;
+    P.TD.perm = T.dev;
+    P.TD.othr = T.dev + M;
+    P.TD.tt_first = T.dev + 2 * (size_t)M;
+    P.TD.tt_cnt = P.TD.tt_first + nT;
+    P.TD.tt_kmax = P.TD.tt_cnt + nT;
+    P.TD.tt_order = P.TD.tt_kmax + nT;
+    P.pl.prefix = 1;
+    P.pl.tile_points = CVF_M;
+    P.pl.idx_sorted = P.pl.idx;
+    const long long work = std::max<long long>(c.n, (long long)G * T.nq + 1);
+    cvf_lattice_fill<<<(unsigned int)((work + CVF_PLAN_TB - 1) / CVF_PLAN_TB), CVF_PLAN_TB, 0, c.stream>>>(
+        P.pl, P.TD, G, M, T.R, T.nq, nT, T.omax, items, wpg);
+    CVF_CK(cudaGetLastError());
+    wk.launches += 1;
+    P.size = {G, (long long)G * nT, (long long)G * items, (long long)G * wpg, 0, (long long)G * T.nq};
+    wk.n_groups = P.size.groups;
+    wk.n_runs = P.size.runs;
+    return cudaSuccess;
+}
+
+/* K0 .. totals for one ordering of the points (prefix: tiled for the prefix kernel); ends with the
+ * sizes on the host */
+static cudaError_t cvf_sort_plan(const CvfCall &c, CvFactorWork &wk, CvfHostPlan &P, bool prefix)
+{
+    CvfPlan &pl = P.pl;
+    const int tb = CVF_PLAN_TB;
+    const unsigned int nb = (unsigned int)((c.n + tb - 1) / tb), nb1 = (unsigned int)((c.n + 1 + tb - 1) / tb);
+    pl.prefix = prefix;
+    pl.tile_points = CVF_M;
+    cvf_point_keys<<<nb, tb, 0, c.stream>>>(c.m, c.lat, c.params, c.n, c.clip, pl);
+    CVF_CK(cudaGetLastError());
+    {
+        cub::DoubleBuffer<unsigned long long> dk(pl.keys, pl.keys_alt);
+        cub::DoubleBuffer<unsigned int> dv(pl.idx, pl.idx_alt);
+        size_t tb_ = P.tmp_bytes;
+        CVF_CK(cub::DeviceRadixSort::SortPairs(P.tmp, tb_, dk, dv, (int)c.n, 0, 64, c.stream));
+        pl.idx_sorted = dv.Current();
+    }
+    cvf_heads<<<nb, tb, 0, c.stream>>>(c.m, c.lat, c.params, c.n, c.clip, pl);
+    CVF_CK(cudaGetLastError());
+    {
+        size_t tb_ = P.tmp_bytes;
+        CVF_CK(cub::DeviceScan::InclusiveSum(P.tmp, tb_, pl.flags2, pl.flags2, (int)c.n, c.stream));
+    }
+    CVF_CK(cudaMemsetAsync(pl.g_omax, 0, ((size_t)c.n + 1) * sizeof(int), c.stream));
+    cvf_group_starts<<<nb, tb, 0, c.stream>>>(c.n, pl);
+    CVF_CK(cudaGetLastError());
+    cvf_group_counts<<<nb1, tb, 0, c.stream>>>(c.n, c.sl.nsteps * CVF_NS, pl);
+    CVF_CK(cudaGetLastError());
+    cvf_group_scan<<<1, 1024, 0, c.stream>>>(pl);
+    CVF_CK(cudaGetLastError());
+    static_assert(sizeof(CvfSizes) == 6 * sizeof(long long), "CvfSizes mirrors CvfPlan::header");
+    CVF_CK(cudaMemcpyAsync(wk.h_sizes, pl.header, sizeof(CvfSizes), cudaMemcpyDeviceToHost, c.stream));
+    CVF_CK(cudaStreamSynchronize(c.stream));
+    wk.launches += 17; /* K0, radix sort (10), heads, one scan (2), starts, counts, group scan */
+    P.size = *wk.h_sizes;
+    return cudaSuccess;
+}
+
+/* The plan of a batch of explicit points.  *shared = false when too few points share a (c, e) group:
+ * the per-point kernel is the better tool, and nothing more is enqueued. */
+static cudaError_t cvf_plan_general(const CvfCall &c, CvFactorWork &wk, CvfHostPlan &P, bool prefix,
+                                    double min_group, bool pick_kernel, bool *shared)
+{
+    /* ordering for the prefix kernel first: it also tells how many q-runs the batch has */
+    CVF_CK(cvf_sort_plan(c, wk, P, prefix));
+    wk.n_groups = P.size.groups;
+    wk.n_runs = P.size.runs;
+    *shared = P.size.groups > 0 && (double)c.n >= min_group * (double)P.size.groups;
+    if (!*shared)
+        return cudaSuccess;
+    if (prefix && pick_kernel && (double)c.n < CVF_MIN_RUN * (double)P.size.runs) /* few points per q-run: */
+        CVF_CK(cvf_sort_plan(c, wk, P, false)); /* the GEMM shares the profiles between all points of a group */
+    cvf_tile_table<<<(unsigned int)((P.size.groups + 127) / 128), 128, 0, c.stream>>>((int)P.size.groups, P.pl);
+    CVF_CK(cudaGetLastError());
+    wk.launches++;
+    return cudaSuccess;
+}
+
+/* The group ranges whose profiles fit w_limit (cvf_group_ranges): one range when all of them fit,
+ * else from the plan's per-group prefix tables -- computed for a lattice, whose groups are all alike,
+ * read back otherwise */
+static cudaError_t cvf_plan_ranges(const CvfCall &c, const CvfHostPlan &P, size_t w_limit,
+                                   std::vector<CvfRange> &ranges)
+{
+    const CvfSizes &s = P.size;
+    if ((size_t)s.w_doubles <= w_limit) {
+        ranges.assign(1, CvfRange{0, (int)s.groups, 0, (int)s.tiles, 0, (int)s.items, 0, s.w_doubles, 0, s.a_chunks});
+        return cudaSuccess;
+    }
+    const size_t ng1 = (size_t)s.groups + 1;
+    std::vector<int> tile(ng1), item(ng1), achunk(ng1);
+    std::vector<long long> woff(ng1);
+    if (P.analytic) { /* every group has the same tiles, items and profile size, and no copy weights */
+        for (long long g = 0; g <= s.groups; g++) {
+            tile[g] = (int)(g * (s.tiles / s.groups));
+            item[g] = (int)(g * (s.items / s.groups));
+            woff[g] = g * (s.w_doubles / s.groups);
         }
     } else {
-        cut.push_back((int)n_groups);
+        CVF_CK(cudaMemcpyAsync(tile.data(), P.pl.tile_start, ng1 * 4, cudaMemcpyDeviceToHost, c.stream));
+        CVF_CK(cudaMemcpyAsync(item.data(), P.pl.item_start, ng1 * 4, cudaMemcpyDeviceToHost, c.stream));
+        CVF_CK(cudaMemcpyAsync(achunk.data(), P.pl.a_start, ng1 * 4, cudaMemcpyDeviceToHost, c.stream));
+        CVF_CK(cudaMemcpyAsync(woff.data(), P.pl.w_off, ng1 * 8, cudaMemcpyDeviceToHost, c.stream));
+        CVF_CK(cudaStreamSynchronize(c.stream));
     }
-    const bool ranged = !h_woff.empty();
-    size_t w_need = 0, a_need = 0;
-    for (size_t i = 0; i + 1 < cut.size(); i++) {
-        const long long wa = ranged ? h_woff[cut[i]] : 0, wb_ = ranged ? h_woff[cut[i + 1]] : w_total;
-        const long long aa = ranged ? h_achunk[cut[i]] : 0, ab = ranged ? h_achunk[cut[i + 1]] : a_total;
-        w_need = std::max(w_need, (size_t)(wb_ - wa));
-        a_need = std::max(a_need, (size_t)(ab - aa) * (CVF_M * CVF_KC));
-    }
-    if (w_need + a_need > wk.w_cap) { /* profiles, then the copy-weight tiles */
-        if (wk.W)
-            cudaFree(wk.W);
-        wk.W = nullptr;
-        wk.w_cap = 0;
-        CVF_CK(cudaMalloc((void **)&wk.W, std::max(w_need + a_need, (size_t)2) * sizeof(double)));
-        wk.w_cap = w_need + a_need;
-    }
-    double *A = wk.W + w_need;
-    if (wk.poison) { /* tests: what this evaluation reads of W and the partials, it must have written first */
-        CVF_CK(cudaMemsetAsync(wk.W, wk.poison, (w_need + a_need) * sizeof(double), stream));
-        CVF_CK(cudaMemsetAsync(wk.d_scratch, wk.poison, (size_t)n_sm * 32 * 3 * CVF_PB * sizeof(double), stream));
-    }
+    ranges = cvf_group_ranges(tile, item, achunk, woff, w_limit);
+    return cudaSuccess;
+}
 
-    /* ---- K1, then K1b + K2 or the prefix kernel, per range ---- */
-    const size_t wb = cv_warp_bytes(m.n_err);
-    const int groups_staged = m.n_blocks * CV_GB;
-    const size_t tab = (size_t)groups_staged * CV_GD * sizeof(double);
-    typedef decltype(&cvf_profile_kernel<1>) CvfProfileFn;
-    const int k1_na = m.na == 1 || m.na == 2 || m.na == 4 ? m.na : 8;
-    const CvfProfileFn k1 = k1_na == 1 ? cvf_profile_kernel<1> : k1_na == 2 ? cvf_profile_kernel<2>
-                            : k1_na == 4 ? cvf_profile_kernel<4> : cvf_profile_kernel<8>;
-    const size_t wb1 = wb + cvf_stage_doubles(k1_na) * sizeof(double); /* working set + profile stage */
-    /* the instantiation's warps, or as many as the shared memory holds (NA = 8, S = 32 and 15 blocks
-     * of group records: 11) */
-    int k1_warps = (int)std::min<long long>(cvf_k1_warps(k1_na), ((long long)smem_max - (long long)tab) / (long long)wb1);
-    if (k1_warps < 1)
+/* wk.W: the profiles of the largest range, then (*A) the copy-weight tiles of the largest */
+static cudaError_t cvf_workspace(const CvfCall &c, CvFactorWork &wk, const std::vector<CvfRange> &ranges, double **A)
+{
+    size_t w_need = 0, a_need = 0;
+    for (const CvfRange &r : ranges) {
+        w_need = std::max(w_need, (size_t)(r.w1 - r.w0));
+        a_need = std::max(a_need, (size_t)(r.a1 - r.a0) * (CVF_M * CVF_KC));
+    }
+    CVF_CK(cv_grow(&wk.W, &wk.w_cap, w_need + a_need));
+    *A = wk.W + w_need;
+    if (wk.poison) { /* tests: what this evaluation reads of W and the partials, it must have written first */
+        CVF_CK(cudaMemsetAsync(wk.W, wk.poison, (w_need + a_need) * sizeof(double), c.stream));
+        CVF_CK(cudaMemsetAsync(wk.d_scratch, wk.poison, cvf_scratch_bytes(c.n_sm), c.stream));
+    }
+    return cudaSuccess;
+}
+
+struct CvfProfileLaunch { decltype(&cvf_profile_kernel<1>) fn; int warps; size_t smem; };
+
+/* K1: the instantiation for the model's rows per group, with its warps, or as many as the shared
+ * memory holds (NA = 8, S = 32 and 15 blocks of group records: 11) */
+static cudaError_t cvf_pick_profile(const CvModelDesc &m, int smem_max, CvfProfileLaunch &k)
+{
+    int na = m.na;
+    switch (na) {
+    case 1: k.fn = cvf_profile_kernel<1>; break;
+    case 2: k.fn = cvf_profile_kernel<2>; break;
+    case 4: k.fn = cvf_profile_kernel<4>; break;
+    default: k.fn = cvf_profile_kernel<8>; na = 8;
+    }
+    const size_t tab = (size_t)(m.n_blocks * CV_GB) * CV_GD * sizeof(double); /* the staged group records */
+    const size_t wb = cv_warp_bytes(m.n_err) + cvf_stage_doubles(na) * sizeof(double); /* working set + profile stage */
+    k.warps = (int)std::min<long long>(cvf_k1_warps(na), ((long long)smem_max - (long long)tab) / (long long)wb);
+    if (k.warps < 1)
         return cudaErrorInvalidConfiguration;
-    const size_t k1_smem = tab + (size_t)k1_warps * wb1;
-    const bool want_mass = m.tail != 0.0;
-    /* warps of the prefix kernel's CTAs: one pass over the row when 768 slots or fewer do it */
+    k.smem = tab + (size_t)k.warps * wb;
+    return cudaSuccess;
+}
+
+typedef decltype(&cvf_prefix_kernel<false, false, false, 1, 3>) CvfPrefixFn;
+#define CVF_KP(nw, sl, one)                                                                         \
+    {{cvf_prefix_kernel<false, false, one, nw, sl>, cvf_prefix_kernel<false, true, one, nw, sl>},  \
+     {cvf_prefix_kernel<true, false, one, nw, sl>, cvf_prefix_kernel<true, true, one, nw, sl>}}
+/* The instantiations of the prefix kernel: per geometry (cvf_prefix_geometry) by [ONE][MASS][FULL].
+ * Only the 8-warp geometry, the one of long rows, has the ONE variants. */
+static const struct {
+    CvfPrefixGeometry g;
+    CvfPrefixFn fn[2][2][2];
+} cvf_prefix_fns[] = {
+    {{1, 3}, {CVF_KP(1, 3, false)}}, {{1, 4}, {CVF_KP(1, 4, false)}}, {{2, 3}, {CVF_KP(2, 3, false)}},
+    {{2, 4}, {CVF_KP(2, 4, false)}}, {{3, 3}, {CVF_KP(3, 3, false)}}, {{3, 4}, {CVF_KP(3, 4, false)}},
+    {{4, 4}, {CVF_KP(4, 4, false)}}, {{6, 3}, {CVF_KP(6, 3, false)}}, {{6, 4}, {CVF_KP(6, 4, false)}},
+    {{8, 4}, {CVF_KP(8, 4, false), CVF_KP(8, 4, true)}},
+};
+#undef CVF_KP
+
+struct CvfPrefixLaunch { CvfPrefixFn fn; CvfPrefixGeometry g; size_t smem; int slots; }; /* slots: of a row, read */
+
+/* K2p for the row layout */
+static CvfPrefixLaunch cvf_pick_prefix(const CvfSlots &sl, bool mass)
+{
+    CvfPrefixLaunch k = {};
     /* The line of the sums is half a line with a tail and not read without one -- except when no line
      * has a count: then its first half (zeros, written by K1) is read, so that every point's sum is
      * formed by a pass (0, models.py:106) and the epilogue reads partials this launch wrote. */
-    const int kp_slots = slots_padded - (sl.sum_line >= 0 ? (want_mass || nsteps == 1 ? 32 : CVF_NS) : 0);
-    /* Geometry of the prefix kernel: warps per CTA and slots per thread so that one pass covers the
-     * row when 32 half-lines or fewer do it -- the fewest warps, then the fewest slots (measured on
-     * the 9 half-lines of cfg3 with a mass: 3 warps x 3 slots 0.82 ms, 3 x 4 0.91 ms; on its 8 half-lines
-     * without one: 2 x 4 0.685 ms, 3 x 3 0.745 ms) */
-    const int kp_half = kp_slots / 32;
-    int kp_nw = 8, kp_sl = 4;
-    if (kp_half <= 24) {
-        static const int nws[] = {1, 2, 3, 4, 6, 8};
-        int n3 = 8, n4 = 8;
-        for (int i = 5; i >= 0; i--) {
-            if (nws[i] * 3 >= kp_half && nws[i] != 4 && nws[i] != 8)
-                n3 = nws[i];
-            if (nws[i] * 4 >= kp_half)
-                n4 = nws[i];
-        }
-        if (n3 <= n4) {
-            kp_nw = n3;
-            kp_sl = 3;
-        } else {
-            kp_nw = n4;
-        }
+    k.slots = sl.nsteps * CVF_NS - (sl.sum_line >= 0 ? (mass || sl.nsteps == 1 ? 32 : CVF_NS) : 0);
+    k.g = cvf_prefix_geometry(k.slots / 32);
+    k.smem = cvf_prefix_smem_bytes(mass, k.g.nw, k.g.sl);
+    /* FULL: the row is a whole number of passes (for the one-pass geometries: exactly one pass) */
+    const bool full = k.slots % (32 * k.g.nw * k.g.sl) == 0;
+    const bool one = k.g.nw == 8 && sl.counts_first;
+    for (const auto &e : cvf_prefix_fns)
+        if (e.g.nw == k.g.nw && e.g.sl == k.g.sl)
+            k.fn = e.fn[one][mass][full];
+    return k;
+}
+
+/* K1, then K1b + K2 or the prefix kernel, over the groups of one range; `last`: the last range */
+static cudaError_t cvf_launch_range(const CvfCall &c, CvFactorWork &wk, CvfHostPlan &P, const CvfRange &r,
+                                    const CvfProfileLaunch &k1, const CvfPrefixLaunch &kp, double *A, bool last)
+{
+    CvfPlan &pl = P.pl;
+    CVF_CK(cudaMemsetAsync(wk.d_counters, 0, 2 * sizeof(unsigned long long), c.stream));
+    if (r.item1 > r.item0) {
+        const int items = r.item1 - r.item0;
+        const int grid = std::min((items + k1.warps - 1) / k1.warps, c.n_sm);
+        k1.fn<<<grid, 32 * k1.warps, k1.smem, c.stream>>>(c.m, c.lat, c.params, c.clip, pl, (int)P.size.groups,
+                                                          r.item0, items, wk.W, r.w0, c.sl.nsteps, c.sl.line_map,
+                                                          c.sl.sum_line, wk.d_counters, c.m.n_blocks * CV_GB);
+        CVF_CK(cudaGetLastError());
+        wk.launches++;
     }
-    const size_t kp_smem = cvf_prefix_smem_bytes(want_mass, kp_nw, kp_sl);
-    const bool full_passes = kp_slots % (8 * 32 * 4) == 0;
-    const bool counts_first = sl.counts_first;
-    typedef decltype(&cvf_prefix_kernel<true, true, true, 8, 4>) CvfPrefixFn;
-    CvfPrefixFn kp = nullptr;
-    const bool full_one = kp_slots == kp_nw * 32 * kp_sl; /* the one pass of a small geometry has no idle thread */
-#define CVF_PICK(nw_, sl_)                                                                                          \
-    (full_one ? (want_mass ? cvf_prefix_kernel<true, true, false, nw_, sl_> : cvf_prefix_kernel<false, true, false, nw_, sl_>) \
-              : (want_mass ? cvf_prefix_kernel<true, false, false, nw_, sl_> : cvf_prefix_kernel<false, false, false, nw_, sl_>))
-    switch (kp_nw * 10 + kp_sl) {
-    case 13: kp = CVF_PICK(1, 3); break;
-    case 14: kp = CVF_PICK(1, 4); break;
-    case 23: kp = CVF_PICK(2, 3); break;
-    case 24: kp = CVF_PICK(2, 4); break;
-    case 33: kp = CVF_PICK(3, 3); break;
-    case 34: kp = CVF_PICK(3, 4); break;
-    case 44: kp = CVF_PICK(4, 4); break;
-    case 63: kp = CVF_PICK(6, 3); break;
-    case 64: kp = CVF_PICK(6, 4); break;
-    default:
-        kp = want_mass ? (full_passes ? (counts_first ? cvf_prefix_kernel<true, true, true, 8, 4> : cvf_prefix_kernel<true, true, false, 8, 4>)
-                                      : (counts_first ? cvf_prefix_kernel<true, false, true, 8, 4> : cvf_prefix_kernel<true, false, false, 8, 4>))
-                       : (full_passes ? (counts_first ? cvf_prefix_kernel<false, true, true, 8, 4> : cvf_prefix_kernel<false, true, false, 8, 4>)
-                                      : (counts_first ? cvf_prefix_kernel<false, false, true, 8, 4> : cvf_prefix_kernel<false, false, false, 8, 4>));
+    if (r.tile1 <= r.tile0)
+        return cudaSuccess;
+    const int tiles = r.tile1 - r.tile0;
+    if (!pl.prefix) {
+        cvf_weights_kernel<<<tiles, CVF_THREADS, 0, c.stream>>>(c.m, c.lat, c.params, c.clip, pl, r.tile0, tiles, A,
+                                                                r.a0);
+        CVF_CK(cudaGetLastError());
+        wk.launches++;
     }
-#undef CVF_PICK
-    CVF_CK(cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1_smem));
-    CVF_CK(cudaFuncSetAttribute(cvf_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                (int)sizeof(CvfSmem)));
-    CVF_CK(cudaFuncSetAttribute(kp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kp_smem));
+    /* tiles of the range by descending cost: the long ones start first */
+    if (P.analytic) {
+        cvf_lattice_order<<<(unsigned int)((tiles + CVF_PLAN_TB - 1) / CVF_PLAN_TB), CVF_PLAN_TB, 0, c.stream>>>(
+            P.TD, r.g0, r.g1, (int)(P.size.tiles / P.size.groups), pl.t_order_alt + r.tile0);
+        CVF_CK(cudaGetLastError());
+        pl.t_sorted = pl.t_order_alt + r.tile0;
+    } else {
+        cub::DoubleBuffer<int> dk(pl.t_key + r.tile0, pl.t_key_alt + r.tile0);
+        cub::DoubleBuffer<int> dv(pl.t_order + r.tile0, pl.t_order_alt + r.tile0);
+        size_t tb_ = P.tmp_bytes;
+        CVF_CK(cub::DeviceRadixSort::SortPairsDescending(P.tmp, tb_, dk, dv, tiles, 0, 32, c.stream));
+        pl.t_sorted = dv.Current();
+    }
+    if (wk.timed && last)
+        CVF_CK(cudaEventRecord(wk.ev[2], c.stream));
+    if (pl.prefix) {
+        const int per_sm = std::max(1, std::min(CVF_WARPS_SM / kp.g.nw, (int)((size_t)c.smem_max / (kp.smem + 1024))));
+        kp.fn<<<std::min(tiles, per_sm * c.n_sm), 32 * kp.g.nw, kp.smem, c.stream>>>(
+            c.m, c.lat, c.params, c.clip, pl, r.tile0, tiles, wk.W, r.w0, c.sl.slot_mh, c.log_tab, c.sl.nsteps,
+            kp.slots, c.out_ll, wk.d_counters + 1, wk.d_scratch);
+    } else {
+        cvf_gemm_kernel<<<std::min(tiles, 2 * c.n_sm), CVF_THREADS, sizeof(CvfSmem), c.stream>>>(
+            c.m, pl, r.tile0, tiles, wk.W, r.w0, A, r.a0, c.sl.slot_mh, c.sl.step_mask, c.log_tab, c.sl.nsteps,
+            c.out_ll, wk.d_counters + 1);
+    }
+    CVF_CK(cudaGetLastError());
+    wk.launches += 2;
+    return cudaSuccess;
+}
+
+cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *const *lat_axes_host,
+                     const double *params, long long n, int clip, double *out_ll, const CvfSlots &sl,
+                     const double *log_tab, CvFactorWork &wk, int n_sm, int smem_max, size_t w_limit,
+                     CvfRequest req, cudaStream_t stream, CvfRan *ran)
+{
+    *ran = CvfRan::None;
+    wk.launches = 0;
+    if (n <= 0 || n > 0x7fffffffLL || !cvf_supported(m))
+        return cudaSuccess;
+    const CvfCall c = {m, lat, params, n, clip, out_ll, sl, log_tab, n_sm, smem_max, stream};
+    CvfHostPlan P = {};
+    CVF_CK(cvf_plan_alloc(c, wk, P));
+    if (wk.timed)
+        CVF_CK(cudaEventRecord(wk.ev[0], stream));
+
+    /* the plan: from the lattice axes when its groups are whole and share enough, else by sorting */
+    const double min_group = req == CvfRequest::Auto ? CVF_MIN_GROUP : 0.0;
+    const bool pick_kernel = req == CvfRequest::Auto || req == CvfRequest::Forced;
+    long long latM = 0;
+    P.analytic = req != CvfRequest::Gemm && lat_axes_host && cvf_lattice_aligned(m, lat, n, &latM) &&
+                 (double)latM >= min_group &&
+                 (double)(lat.len[2] * (long long)lat.len[3]) >= (pick_kernel ? CVF_MIN_RUN : 1.0);
+    bool shared = true;
+    CVF_CK(P.analytic ? cvf_plan_lattice(c, lat_axes_host, wk, P)
+                      : cvf_plan_general(c, wk, P, req != CvfRequest::Gemm, min_group, pick_kernel, &shared));
+    wk.analytic = P.analytic ? 1 : 0;
+    if (!shared)
+        return cudaSuccess;
+    wk.n_tiles = P.size.tiles;
+    wk.n_items = P.size.items;
+    wk.w_doubles = P.size.w_doubles;
+
+    std::vector<CvfRange> ranges;
+    CVF_CK(cvf_plan_ranges(c, P, w_limit, ranges));
+    double *A = nullptr;
+    CVF_CK(cvf_workspace(c, wk, ranges, &A));
+    CvfProfileLaunch k1;
+    CVF_CK(cvf_pick_profile(m, smem_max, k1));
+    const CvfPrefixLaunch kp = cvf_pick_prefix(sl, m.tail != 0.0);
+    CVF_CK(cudaFuncSetAttribute(k1.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k1.smem));
+    CVF_CK(cudaFuncSetAttribute(cvf_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CvfSmem)));
+    CVF_CK(cudaFuncSetAttribute(kp.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kp.smem));
     if (wk.timed)
         CVF_CK(cudaEventRecord(wk.ev[1], stream));
-    for (size_t i = 0; i + 1 < cut.size(); i++) {
-        const int g0 = cut[i], g1 = cut[i + 1];
-        const int item0 = ranged ? h_item[g0] : 0, item1 = ranged ? h_item[g1] : (int)n_items;
-        const int tile0 = ranged ? h_tile[g0] : 0, tile1 = ranged ? h_tile[g1] : (int)n_tiles;
-        const long long w0 = ranged ? h_woff[g0] : 0;
-        const long long a0 = ranged ? h_achunk[g0] : 0;
-        CVF_CK(cudaMemsetAsync(wk.d_counters, 0, 2 * sizeof(unsigned long long), stream));
-        if (item1 > item0) {
-            const int items = item1 - item0;
-            int grid = (items + k1_warps - 1) / k1_warps;
-            if (grid > n_sm)
-                grid = n_sm;
-            k1<<<grid, 32 * k1_warps, k1_smem, stream>>>(
-                m, lat, params, clip, pl, (int)n_groups, item0, items, wk.W, w0, nsteps, sl.line_map, sl.sum_line,
-                wk.d_counters, groups_staged);
-            CVF_CK(cudaGetLastError());
-            wk.launches++;
-        }
-        if (tile1 > tile0) {
-            const int tiles = tile1 - tile0;
-            if (!prefix) {
-                cvf_weights_kernel<<<tiles, CVF_THREADS, 0, stream>>>(m, lat, params, clip, pl, tile0, tiles, A, a0);
-                CVF_CK(cudaGetLastError());
-                wk.launches++;
-            }
-            /* tiles of the range by descending cost: the long ones start first */
-            if (analytic) {
-                cvf_lattice_order<<<(unsigned int)((tiles + tb - 1) / tb), tb, 0, stream>>>(
-                    TD, g0, g1, (int)(n_tiles / n_groups), pl.t_order_alt + tile0);
-                CVF_CK(cudaGetLastError());
-                pl.t_sorted = pl.t_order_alt + tile0;
-            } else {
-                cub::DoubleBuffer<int> dk(pl.t_key + tile0, pl.t_key_alt + tile0);
-                cub::DoubleBuffer<int> dv(pl.t_order + tile0, pl.t_order_alt + tile0);
-                size_t tb_ = tmp_bytes;
-                CVF_CK(cub::DeviceRadixSort::SortPairsDescending(tmp, tb_, dk, dv, tiles, 0, 32, stream));
-                pl.t_sorted = dv.Current();
-            }
-            if (wk.timed && i + 2 == cut.size())
-                CVF_CK(cudaEventRecord(wk.ev[2], stream));
-            int grid = tiles < 2 * n_sm ? tiles : 2 * n_sm;
-            if (prefix) {
-                const int per_sm = std::max(1, std::min(CVF_WARPS_SM / kp_nw, (int)((size_t)smem_max / (kp_smem + 1024))));
-                grid = tiles < per_sm * n_sm ? tiles : per_sm * n_sm;
-                kp<<<grid, 32 * kp_nw, kp_smem, stream>>>(m, lat, params, clip, pl, tile0, tiles, wk.W, w0, slot_mh,
-                                                           log_tab, nsteps, kp_slots, out_ll, wk.d_counters + 1,
-                                                           wk.d_scratch);
-            } else {
-                cvf_gemm_kernel<<<grid, CVF_THREADS, sizeof(CvfSmem), stream>>>(
-                    m, pl, tile0, tiles, wk.W, w0, A, a0, slot_mh, step_mask, log_tab, nsteps, out_ll,
-                    wk.d_counters + 1);
-            }
-            CVF_CK(cudaGetLastError());
-            wk.launches += 2;
-        }
-    }
+    for (size_t i = 0; i < ranges.size(); i++)
+        CVF_CK(cvf_launch_range(c, wk, P, ranges[i], k1, kp, A, i + 1 == ranges.size()));
     if (wk.timed)
         CVF_CK(cudaEventRecord(wk.ev[3], stream));
-    *used = prefix ? 2 : 1;
+    *ran = P.pl.prefix ? CvfRan::Prefix : CvfRan::Gemm;
     return cudaSuccess;
 }

@@ -40,13 +40,16 @@ struct CvfLatticeCache {
     cudaEvent_t uploaded = nullptr; /* the last upload has left the staging buffer */
 };
 
+/* The sizes of a batch's plan in the order of its header on the device: groups, tiles, profile items,
+ * profile doubles, K-chunks of copy weights, q-runs */
+struct CvfSizes { long long groups, tiles, items, w_doubles, a_chunks, runs; };
+
 struct CvFactorWork {
-    void *plan = nullptr; /* sort keys, indices, group tables, cub scratch */
+    unsigned char *plan = nullptr; /* sort keys, indices, group tables, cub scratch */
     size_t plan_cap = 0;
     double *W = nullptr;  /* profiles */
     size_t w_cap = 0;     /* doubles */
-    long long *h_header = nullptr; /* pinned host: n_groups, tiles, items, profile doubles */
-    std::size_t h_arrays_cap = 0;
+    CvfSizes *h_sizes = nullptr; /* pinned host: the sizes the general plan counted */
     unsigned long long *d_counters = nullptr; /* two device words */
     double *d_scratch = nullptr; /* prefix kernel: per CTA the per-(warp, point) partials of a batch */
     /* timing of the most recent evaluation (events recorded when `timed`) */
@@ -54,12 +57,10 @@ struct CvFactorWork {
     bool timed = false;
     /* facts about the most recent evaluation */
     long long n_groups = 0, n_tiles = 0, n_items = 0, w_doubles = 0, n_runs = 0;
-    int prefix = 0; /* 1: the prefix kernel ran, 0: the GEMM */
     int launches = 0;
     int analytic = 0; /* 1: the plan came from the lattice axes (no sort, no host synchronisation) */
     int poison = 0;   /* tests (COVEST_B200_POISON): byte W and d_scratch are filled with at each evaluation, 0 = off */
     CvfLatticeCache lattice;
-    double gemm_fma = 0.0; /* FMAs the tiles of K2 issue (128 rows x padded copies x padded slots) */
 };
 
 /* The slots of a profile row as the batch kernels (K1's stores, K2, K2p) see them.
@@ -127,22 +128,72 @@ static inline void cvf_build_slots(const std::vector<double> &slot_mult, const s
 /* Can this context use the factored path at all (repeats model, few enough error classes)? */
 bool cvf_supported(const CvModelDesc &m);
 
-/* Evaluates n points.  *used = 0 when the batch does not group well enough (nothing written to
- * out_ll; the caller runs the per-point kernel), 1 when K2 (the GEMM) ran, 2 when the prefix kernel
- * ran.  sl: the row layout (CvfSlots).  kernel_mode: 0 = prefix kernel when the batch has at least min_run points per q-run (points
- * of a group that also share q), else the GEMM; 1 = GEMM; 2 = prefix kernel.  `step_mask` of the row layout = per 32 slots,
- * bit 2 nt + c set when one of the slots 8 nt + 2 q + c, q < 4, has a count (cvf_step_masks);
- * `log_tab` = cv_log_table.  w_limit = largest profile workspace in
- * doubles; larger batches run in several group ranges. */
-/* lat_axes_host: the lattice axes in host memory (n_param pointers) when lat.enabled, else NULL */
-cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *const *lat_axes_host,
-                     const double *params, long long n,
-                     int clip, double *out_ll, const CvfSlots &sl,
-                     const double *log_tab, CvFactorWork &wk, int n_sm, int smem_max, size_t w_limit,
-                     double min_group, double min_run, int kernel_mode, cudaStream_t stream,
-                     int *used);
+/* What cvf_eval is asked to run: path mode 0, 2, 3 or 4 of cvb_set_path (Forced: the batched path
+ * however few points share a group, the kernel as in Auto) */
+enum class CvfRequest { Auto, Forced, Gemm, Prefix };
+/* What it ran.  None: the batch does not group well enough (nothing written to out_ll) */
+enum class CvfRan { None, Gemm, Prefix };
 
-/* host: the step masks of a slot_h table (length a multiple of 32) */
+/* Evaluates n points.  sl: the row layout (CvfSlots).  `log_tab` = cv_log_table.  w_limit = largest
+ * profile workspace in doubles; larger batches run in several group ranges.  lat_axes_host: the
+ * lattice axes in host memory (n_param pointers) when lat.enabled, else NULL. */
+cudaError_t cvf_eval(const CvModelDesc &m, const CvLattice &lat, const double *const *lat_axes_host,
+                     const double *params, long long n, int clip, double *out_ll, const CvfSlots &sl,
+                     const double *log_tab, CvFactorWork &wk, int n_sm, int smem_max, size_t w_limit,
+                     CvfRequest req, cudaStream_t stream, CvfRan *ran);
+
+/* host: the geometry of the prefix kernel (warps per CTA, slots per thread and pass) for rows of
+ * `half_lines` half-lines of 32 slots: one pass covers the row when 32 half-lines or fewer do it --
+ * the fewest warps, then the fewest slots (measured on the 9 half-lines of cfg3 with a mass: 3 warps
+ * x 3 slots 0.82 ms, 3 x 4 0.91 ms; on its 8 half-lines without one: 2 x 4 0.685 ms, 3 x 3
+ * 0.745 ms).  Longer rows take 8 x 4, in several passes beyond 32 half-lines.  Only these
+ * geometries are instantiated: 3 slots with 1, 2, 3 or 6 warps, 4 slots with 1, 2, 3, 4, 6 or 8. */
+struct CvfPrefixGeometry { int nw, sl; };
+static inline CvfPrefixGeometry cvf_prefix_geometry(int half_lines)
+{
+    if (half_lines > 24)
+        return {8, 4};
+    static const int nws[] = {1, 2, 3, 4, 6, 8};
+    int n3 = 8, n4 = 8;
+    for (int i = 5; i >= 0; i--) {
+        if (nws[i] * 3 >= half_lines && nws[i] != 4 && nws[i] != 8)
+            n3 = nws[i];
+        if (nws[i] * 4 >= half_lines)
+            n4 = nws[i];
+    }
+    if (n3 <= n4)
+        return {n3, 3};
+    return {n4, 4};
+}
+
+/* A range of consecutive groups whose profiles fit the workspace, with its bounds in the plan's
+ * prefix tables: tiles, profile items, profile doubles, K-chunks of copy weights */
+struct CvfRange {
+    int g0, g1, tile0, tile1, item0, item1; /* groups g0 .. g1 - 1 */
+    long long w0, w1, a0, a1;
+};
+
+/* host: groups 0 .. n - 1 cut into ranges whose profiles take at most w_limit doubles each, or one
+ * group alone when it takes more.  The tables are the exclusive prefix sums over the groups, n + 1
+ * entries each, as the plan holds them. */
+static inline std::vector<CvfRange> cvf_group_ranges(const std::vector<int> &tile, const std::vector<int> &item,
+                                                     const std::vector<int> &achunk, const std::vector<long long> &woff,
+                                                     size_t w_limit)
+{
+    std::vector<CvfRange> out;
+    const int n = (int)woff.size() - 1;
+    for (int g0 = 0; g0 < n;) {
+        int g1 = g0 + 1;
+        while (g1 < n && (size_t)(woff[g1 + 1] - woff[g0]) <= w_limit)
+            g1++;
+        out.push_back({g0, g1, tile[g0], tile[g1], item[g0], item[g1], woff[g0], woff[g1], achunk[g0], achunk[g1]});
+        g0 = g1;
+    }
+    return out;
+}
+
+/* host: the step masks of a slot_h table (length a multiple of 32): per 32 slots, bit 2 nt + c set
+ * when one of the slots 8 nt + 2 q + c, q < 4, has a count */
 static inline std::vector<int> cvf_step_masks(const std::vector<double> &slot_h)
 {
     std::vector<int> out(slot_h.size() / 32, 0);

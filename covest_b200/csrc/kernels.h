@@ -7,6 +7,24 @@
 
 #include "cvpoint.h"
 
+/* grows *buf (*cap elements of device memory, or of pinned host memory) to hold `want` elements; the
+ * contents are not kept */
+template <typename T>
+static cudaError_t cv_grow(T **buf, size_t *cap, size_t want, bool pinned = false)
+{
+    if (want <= *cap)
+        return cudaSuccess;
+    if (*buf)
+        pinned ? cudaFreeHost(*buf) : cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    const size_t bytes = want * sizeof(T);
+    cudaError_t e = pinned ? cudaMallocHost((void **)buf, bytes) : cudaMalloc((void **)buf, bytes);
+    if (e == cudaSuccess)
+        *cap = want;
+    return e;
+}
+
 /* A Cartesian lattice of parameter points generated on the device, decoded with the LAST axis
  * varying fastest (the order of itertools.product, which grid.py:33 uses for its candidate
  * grids).  A launch takes runs of `block` consecutive lattice indices: point i is the lattice

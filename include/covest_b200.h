@@ -168,17 +168,18 @@ CVB_API int cvb_last_kernel_ms(cvb_ctx *ctx, double *out_ms, int *out_launches);
  * points per distinct (c, e); prefix kernel at >= 4 points per q-run), 1 = per-point only,
  * 2 = factored whenever the model supports it, 3 = factored with the GEMM, 4 = factored with the
  * prefix kernel, 5 = every point term by term in the reference's order of operations (the kernel
- * that otherwise re-evaluates only points with subnormal bin probabilities; slow, a check).  The environment variable COVEST_B200_PATH=direct|factored|gemm|prefix|auto sets
- * the initial mode.  The factored path holds the repeats model with max_error <= 32 only: for the
- * basic model and for max_error > 32, modes 0 and 2-4 run the per-point kernel.  Per-bin
- * probabilities (cvb_probs_batch) always use the per-point kernel. */
+ * that otherwise re-evaluates only points with subnormal bin probabilities; slow, a check).  The
+ * environment variable COVEST_B200_PATH=auto|direct|factored|gemm|prefix|faithful sets the initial
+ * mode (0-5 in this order; any other value: 0).  The factored path holds the repeats model with
+ * max_error <= 32 only: for the basic model and for max_error > 32, modes 0 and 2-4 run the
+ * per-point kernel.  Per-bin probabilities (cvb_probs_batch) always use the per-point kernel. */
 CVB_API int cvb_set_path(cvb_ctx *ctx, int mode);
 
 /* Facts about the most recent evaluation: out[0] = path used (1 per-point, 2 factored with the
- * GEMM, 3 factored with the prefix kernel); for the factored path out[1] = distinct (c, e) groups,
- * out[2] = tiles, out[3] = profile items (16 copy numbers each), out[4] = doubles of profile
- * workspace, out[5..7] = device ms of the planning kernels, the profile kernel and the GEMM /
- * prefix kernel (after cvb_set_timing(ctx, 1)), out[8] = q-runs (0 when the GEMM ordering ran);
+ * GEMM, 3 factored with the prefix kernel, 4 term by term: mode 5); for the factored path
+ * out[1] = distinct (c, e) groups, out[2] = tiles, out[3] = profile items (16 copy numbers each),
+ * out[4] = doubles of profile workspace, out[5..7] = device ms of the planning kernels, the profile
+ * kernel and the GEMM / prefix kernel (after cvb_set_timing(ctx, 1)), out[8] = q-runs (0 when the GEMM ordering ran);
  * out[9] = points of the call that were re-evaluated term by term because a bin with a count had a
  * probability in the subnormal range, where the reference's per-term roundings decide the value
  * (reading it waits for the device); out[10] = 1 when the plan of the batch came from lattice axes
